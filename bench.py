@@ -1,10 +1,16 @@
 """Benchmark of the Real-BasicVSR x4 hot path (BASELINE.json: output frames/s, 720p out).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one `model(lr)` pass of the drop-in `vsrlab...RealBasicVSR` over `--clips`
 synthetic 30-frame 180x320 clips per GPU (cfg3 of BASELINE.json, experiment=basic 5/5 blocks
 unless --blocks is given), bf16 mode.  Prints ONE JSON line (rank 0).
+
+--dump-outputs DIR writes the `sr` and `lq` that the last timed step returned (rank 0's clips) as
+DIR/sr.npy and DIR/lq.npy, float32.  Inputs and weights are seeded, so two builds run with the same
+arguments can be compared output for output.  An output larger than DUMP_ELEMS elements is written
+as the 1-D sample at DUMP_ELEMS seeded flat indices (sorted, drawn with replacement), the same
+indices on every run with the same arguments.
 
 * value        frames/s, all ranks, inputs already resident in HBM (CUDA events, max over ranks)
 * e2e          same metric through the public nn.Module call with pinned HOST buffers: H2D of the
@@ -44,6 +50,7 @@ METRIC = "realbasicvsr_x4_output_frames_per_sec_720p"
 UNIT = "frames/s"
 T_FRAMES, LR_H, LR_W = 30, 180, 320
 CFG4_FWD_GFLOP = {5: 3824.66, 20: 9260.48}        # SURVEY.md §8d: forward conv FLOPs of one cfg4 micro-batch; training ~ 3x
+DUMP_ELEMS = 1 << 22                              # 16 MB of float32 per dumped array: sr + lq stay under 64 MB
 
 
 def peaks():
@@ -214,6 +221,18 @@ def workload_config(a, clips):
             "precision": "bf16 activations, fp32 accumulate", "cuda_graph": "whole forward captured once, replayed per step",
             "parallelism": f"clips sharded over {a.gpus} GPU(s), no collective",
             "l2": "per-step working set (GBs of activations) exceeds the 126 MB L2; no explicit flush"}
+
+
+def dump_outputs(path: str, outputs: dict) -> None:
+    """`outputs` name -> device tensor; see the module docstring for what is written."""
+    import numpy as np
+    out = Path(path)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, t in outputs.items():
+        if t.numel() > DUMP_ELEMS:
+            idx = torch.randint(t.numel(), (DUMP_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(out / f"{name}.npy", t.float().cpu().numpy())
 
 
 def emit(line: dict) -> None:
@@ -399,7 +418,13 @@ def main():
                     help="bf16 (headline) | fp32 = fp32-accurate split-bf16 on the tensor cores | fp32_ffma = FFMA kernel")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the reference CPU run and the parity record")
     ap.add_argument("--no-extras", action="store_true", help="skip the blocks20 / train_cfg4 / e2e_narrow legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the sr / lq of the last timed step to DIR/<name>.npy (float32, see the module docstring)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU path's outputs; it does not apply to --impl reference")
     a.warmup = max(a.warmup, 3) if a.impl != "reference" else a.warmup
     if a.impl == "reference":
         return run_reference(a)
@@ -459,14 +484,21 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     e0.record()
-    for _ in range(a.steps):
+    for _ in range(a.steps - 1):
         step()
+    out = step()
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     launches = ops.launch_count() - l0 + VF.replayed_launches() - r0      # direct launches + kernel nodes of graph replays
     sampler.stop_flag = True
     sampler.join(timeout=2)
+    if a.dump_outputs and rank == 0:
+        # dumped before anything else runs: `lq` is `work`, which the next step() overwrites in place
+        sr, lq = [torch.cat(o) for o in zip(*out)] if a.streams > 1 else out
+        dump_outputs(a.dump_outputs, {"sr": sr, "lq": lq})
+        del sr, lq
+    del out
 
     # ---- end to end: pinned host -> device -> model -> pinned host --------------------------
     # What a user of the drop-in does for a stream of clips: H2D of clip k+1 and D2H of clip k-1 run on a copy
