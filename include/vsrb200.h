@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define VSRB_VERSION 100
+#define VSRB_VERSION 101
 
 /* error codes */
 #define VSRB_OK            0
@@ -129,15 +129,6 @@ typedef struct vsrb_conv_args {
      * still be valid (launches the ring-walk kernel does not take use it).                                        */
     const void*  patch;
     int64_t      patch_img_stride, patch_group_stride;
-    /* Optional fused backward warp of the 64-channel segment (north_star part 2; basicvsr.py:52-58,66-73 =
-     * flow_warp -> cat -> stem conv): when `warp_flow` is given, in[] of the 64-channel segment is the UNWARPED feature
-     * map of the previous time step and the kernel samples it (bilinear, zeros padding, spynet.py:95-106) while it
-     * builds the conv's operand rows, so the warped tensor never exists in memory.  fp32 [.,h,w,2]; image li of group
-     * g: warp_flow + g * warp_flow_group_stride + li * warp_flow_img_stride (float2 elements);
-     * the feature map likewise through in_img_stride / in_group_stride (elements, 0 = dense).               */
-    const float* warp_flow;
-    int64_t      warp_flow_img_stride, warp_flow_group_stride;
-    int64_t      in_img_stride, in_group_stride;
 } vsrb_conv_args;
 
 /* ---- library ------------------------------------------------------------------------- */
@@ -155,8 +146,8 @@ int         vsrb_debug_status(void* stream);
 int         vsrb_debug_trace(uint64_t* out, int32_t n_ctas);
 
 /* debug aid: with VSRB_RING_DEBUG bit 64 set, CTA (0,0) of every ring-walk conv adds up clock cycles: out[0] MMA issuer waiting
- * for a free accumulator slot, [1] waiting for operand rows, [2] steps issued, [3] gather warp waiting for a free operand
- * slot, [4] gathering, [5] epilogue warp waiting for finished rows, [6] epilogue work                                  */
+ * for a free accumulator slot, [1] waiting for operand rows, [2] steps issued, [3] epilogue warp waiting for finished rows,
+ * [4] epilogue work                                                                                                    */
 int         vsrb_ring_debug_stats(uint64_t* out, int32_t reset);
 
 /* ---- convolution: replaces nn.Conv2d -> F.conv2d (+ the pointwise op that follows it) --
@@ -169,10 +160,6 @@ size_t vsrb_packed_weight_bytes(const vsrb_conv_geom* g);
 int    vsrb_pack_conv_weight(const vsrb_conv_geom* g, const float* w, int32_t cin_total,
                              const float* bias, void* packed, void* stream);
 int    vsrb_conv2d_fwd(const vsrb_conv_args* a, void* stream);
-/* 1 if this launch would run on the ring-walk kernel (conv_ring.cu) - the only one that implements `warp_flow` and
- * consumes `patch` - else 0.  A pure function of the arguments; lets a scheduler choose between the fused stem and
- * vsrb_flow_warp + vsrb_conv2d_fwd once per shape.                                                                */
-int    vsrb_conv2d_takes_ring(const vsrb_conv_args* a);
 /* How the library will tile this geometry (diagnostics / tests): info = {stacked, n_tile, n_blocks,
  * mma_n, k_chunk of segment 0, k_chunk of segment 1, pipeline stages per tile, weight KiB per block} */
 int    vsrb_conv_plan_info(const vsrb_conv_geom* g, int32_t info[8]);

@@ -32,7 +32,7 @@ def test_header_and_binding_agree(lib):
 
 def test_version_and_geometry_helpers_run_on_cpu(lib):
     from vsrlab_b200 import _lib
-    assert lib.vsrb_version() == 100
+    assert lib.vsrb_version() == 101
     g = _lib.ConvGeom()
     g.kh = g.kw = 3
     g.n_seg = 1

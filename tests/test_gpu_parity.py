@@ -724,89 +724,3 @@ def test_im2col3x3_patches(dev, shape):
     ops.im2col3x3(x, p, n, h, w)
     want = F.unfold(x, 3, padding=1).view(n, 3, 9, h, w).permute(0, 3, 4, 2, 1).reshape(n, h, w, 27).to(torch.bfloat16)
     assert torch.equal(p[..., :27], want) and (p[..., 27:] == 0).all()
-
-
-@pytest.mark.parametrize("case", [(2, 45, 64), (1, 180, 320), (3, 23, 61)], ids=lambda c: f"n{c[0]}_{c[1]}x{c[2]}")
-def test_fused_warp_stem_equals_warp_then_conv(dev, case, monkeypatch):
-    """North-star part 2 (basicvsr.py:52-58,66-73: flow_warp -> cat([lr_i, feat]) -> stem conv): the ring-walk stem that
-    samples the previous features through the flow while it builds its operand rows must give bit-identical results to
-    vsrb_flow_warp followed by the same stem on the warped tensor - flows of +-20 px incl. out-of-bounds, integer and
-    half-pixel positions, two weight groups reading different frames / flows through strides."""
-    from vsrlab_b200 import ops
-    from vsrlab_b200._lib import ACT_LRELU, BF16, PAD_ZEROS
-    n, h, w = case
-    monkeypatch.setenv("VSRB_RING_MIN_ROWS", "0")
-    monkeypatch.delenv("VSRB_TC_NO_RING", raising=False)
-    g = torch.Generator().manual_seed(n + h * 3 + w)
-    convs = []
-    for _ in range(2):
-        cv = torch.nn.Conv2d(67, 64, 3, 1, 1)
-        with torch.no_grad():
-            cv.weight.copy_(torch.randn(cv.weight.shape, generator=g) / (67 * 9) ** 0.5)
-            cv.bias.copy_(torch.randn(cv.bias.shape, generator=g) * 0.1)
-        convs.append(cv.to(dev))
-    pc = ops.PackedConv(convs, [(3, 64), (0, 3)], BF16)
-    B = 2 * n
-    # feature bank [2 groups][n clips][2 frames]: group 0 reads frame 1, group 1 frame 0; flows likewise from a [2][n][2] bank
-    bank = torch.randn(2, n, 2, h, w, 64, generator=g).to(dev).to(torch.bfloat16)
-    flows = ((torch.rand(2, n, 2, h, w, 2, generator=g) - 0.5) * 40).to(dev)
-    flows[0, 0, 1, 0, :4] = torch.tensor([[0.0, 0.0], [1.0, -1.0], [0.5, 0.5], [500.0, -500.0]], device=dev)
-    lr = torch.rand(B, 3, h, w, generator=g)
-    lr_t, _ = to_dev_nhwc(lr, BF16, dev)
-    patches = torch.empty(B, h, w, 32, dtype=torch.bfloat16, device=dev)
-    ops.im2col3x3(lr.to(dev).contiguous(), patches, B, h, w)
-    fe = h * w * 64
-    src0, src1 = bank[0, 0, 1], bank[1, 0, 0]
-    fl0, fl1 = flows[0, 0, 1], flows[1, 0, 0]
-    # reference path: two warps into a dense buffer, then the stem (ring kernel, TMA-fed)
-    warped = torch.empty(B, h, w, 64, dtype=torch.bfloat16, device=dev)
-    ops.flow_warp(src0.data_ptr(), fl0.data_ptr(), warped[:n], n, h, w, 64, BF16, PAD_ZEROS, x_img_stride=2 * fe, flow_img_stride=2 * h * w)
-    ops.flow_warp(src1.data_ptr(), fl1.data_ptr(), warped[n:], n, h, w, 64, BF16, PAD_ZEROS, x_img_stride=2 * fe, flow_img_stride=2 * h * w)
-    want = torch.empty(B, h, w, 64, dtype=torch.bfloat16, device=dev)
-    ops.conv2d_fwd(pc, [warped, lr_t], [64, 16], B, h, w, act=ACT_LRELU, slope=0.1, out=want, out_c=64, patch=patches)
-    got = torch.full((B, h, w, 64), 7.0, dtype=torch.bfloat16, device=dev)
-    kw = dict(warp_flow=fl0.data_ptr(), warp_flow_strides=(2 * h * w, (fl1.data_ptr() - fl0.data_ptr()) // 8),
-              in_strides=(2 * fe, (src1.data_ptr() - src0.data_ptr()) // 2))
-    assert ops.conv2d_fwd(pc, [src0.data_ptr(), lr_t], [64, 16], B, h, w, act=ACT_LRELU, out=got, out_c=64, patch=patches,
-                          query_ring=True, **kw)
-    ops.conv2d_fwd(pc, [src0.data_ptr(), lr_t], [64, 16], B, h, w, act=ACT_LRELU, slope=0.1, out=got, out_c=64, patch=patches, **kw)
-    torch.cuda.synchronize()
-    assert ops.debug_status() == 0
-    assert torch.equal(got, want)
-    # and against the oracle warp + fp32 conv on bf16-rounded operands
-    xs = torch.cat([O.flow_warp(bank[0, :, 1].float().cpu().permute(0, 3, 1, 2), flows[0, :, 1].cpu(), "zeros"),
-                    O.flow_warp(bank[1, :, 0].float().cpu().permute(0, 3, 1, 2), flows[1, :, 0].cpu(), "zeros")])
-    y = torch.cat([F.conv2d(torch.cat([bf16r(lr[i * n:(i + 1) * n]), bf16r(xs[i * n:(i + 1) * n])], 1), bf16r(convs[i].weight.detach().cpu()),
-                            convs[i].bias.detach().cpu(), padding=1) for i in range(2)])
-    y = O.lrelu(y)
-    assert (got.float().permute(0, 3, 1, 2).cpu() - y).abs().max().item() <= 2.0 ** -7 * max(y.abs().max().item(), 1.0)
-
-
-def test_model_with_fused_warp_equals_model_with_separate_warp(dev, monkeypatch):
-    """Whole model, bf16 mode: fusing flow_warp into the stem conv changes nothing in the output (bit for bit) and removes
-    every flow_warp launch of the propagation loop."""
-    from vsrlab_b200 import functional as VF, ops
-    monkeypatch.setenv("VSRB_RING_MIN_ROWS", "0")
-    net = build_state_dict("ragged").to(dev).eval()                   # SPyNet amplified: multi-pixel flows
-    x = torch.rand(2, 5, 3, 36, 52, generator=torch.Generator().manual_seed(3)).to(dev)
-    keep = (VF.FUSED_WARP, VF.GRAPHS)
-    outs, launches = [], []
-    try:
-        VF.GRAPHS = False
-        for fused in (True, False):
-            VF.FUSED_WARP = fused
-            VF.clear_caches()
-            ops.PROFILE = []
-            with torch.no_grad(), VF.precision("bf16"):
-                sr, lq = net(x.clone())
-            torch.cuda.synchronize()
-            launches.append(sum(1 for e in ops.PROFILE if e[0] == "flow_warp"))
-            ops.PROFILE = None
-            outs.append((sr.clone(), lq.clone()))
-    finally:
-        VF.FUSED_WARP, VF.GRAPHS = keep
-        ops.PROFILE = None
-        VF.clear_caches()
-    assert launches[0] == 0 and launches[1] == 4                     # one launch (both directions) per time step after the first
-    assert torch.equal(outs[0][0], outs[1][0]) and torch.equal(outs[0][1], outs[1][1])
-    assert ops.debug_status() == 0

@@ -1,5 +1,6 @@
-"""Propagation stem, fused vs separate: [flow_warp x2 + stem conv] against [stem conv that samples its input through the flow],
-two weight groups x `imgs` images, replayed from a CUDA graph between two ordinary resblock convs (so launch overlap is realistic).
+"""Propagation stem: [stem conv] alone and [flow_warp x2 + stem conv], two weight groups x `imgs` images, replayed from a CUDA
+graph between two ordinary resblock convs (so launch overlap is realistic).  With VSRB_RING_DEBUG=64 it prints the ring-walk
+kernel's cycle counters for the stem instead.
     python tools/stem_bench.py [--imgs 2]
 """
 import argparse
@@ -38,9 +39,6 @@ def main():
         ops.flow_warp(feat[:n], flow[:n], warped[:n], n, h, w, 64, BF16, PAD_ZEROS)
         ops.flow_warp(feat[n:], flow[n:], warped[n:], n, h, w, 64, BF16, PAD_ZEROS)
         ops.conv2d_fwd(stem, [warped, lr], [64, 16], B, h, w, act=ACT_LRELU, out=x1, out_c=64, patch=patches)
-
-    def fused():
-        ops.conv2d_fwd(stem, [feat, lr], [64, 16], B, h, w, act=ACT_LRELU, out=x1, out_c=64, patch=patches, warp_flow=flow)
 
     def stem_only():
         ops.conv2d_fwd(stem, [feat, lr], [64, 16], B, h, w, act=ACT_LRELU, out=x1, out_c=64, patch=patches)
@@ -82,18 +80,17 @@ def main():
         import ctypes as C
         from vsrlab_b200 import _lib as L
         buf = (C.c_uint64 * 8)()
-        for name, fn in (("stem only", stem_only), ("fused", fused)):
-            fn()
-            L.load().vsrb_ring_debug_stats(buf, 1)
-            for _ in range(20):
-                fn()
-            L.load().vsrb_ring_debug_stats(buf, 1)
-            v = [x / 20 for x in buf]
-            print(f"{name:10s}: per launch: issuer wait acc-slot {v[0]:.0f} cyc, wait rows {v[1]:.0f} cyc, steps {v[2]:.1f}; warp4: wait free slot "
-                  f"{v[3]:.0f}, gather {v[4]:.0f}, wait finished rows {v[5]:.0f}, epilogue {v[6]:.0f} cyc")
+        stem_only()
+        L.load().vsrb_ring_debug_stats(buf, 1)
+        for _ in range(20):
+            stem_only()
+        L.load().vsrb_ring_debug_stats(buf, 1)
+        v = [x / 20 for x in buf]
+        print(f"stem only: per launch: issuer wait acc-slot {v[0]:.0f} cyc, wait rows {v[1]:.0f} cyc, steps {v[2]:.1f}; warp4: "
+              f"wait finished rows {v[3]:.0f}, epilogue {v[4]:.0f} cyc")
         return
     base = run(body_only)
-    for name, fn in (("stem only (no warp)", stem_only), ("warp x2 + stem", separate), ("fused warp stem", fused)):
+    for name, fn in (("stem only (no warp)", stem_only), ("warp x2 + stem", separate)):
         t = run(fn)
         print(f"{name:22s}: {t - base:7.2f} us on top of the two body convs ({base:.2f} us)", flush=True)
 

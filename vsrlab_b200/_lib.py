@@ -63,9 +63,6 @@ class ConvArgs(C.Structure):
         ("split", C.c_int32),
         ("patch", C.c_void_p),
         ("patch_img_stride", C.c_int64), ("patch_group_stride", C.c_int64),
-        ("warp_flow", C.c_void_p),
-        ("warp_flow_img_stride", C.c_int64), ("warp_flow_group_stride", C.c_int64),
-        ("in_img_stride", C.c_int64), ("in_group_stride", C.c_int64),
     ]
 
 
@@ -83,7 +80,6 @@ SYMBOLS = {
     "vsrb_packed_weight_bytes": (C.c_size_t, [C.POINTER(ConvGeom)]),
     "vsrb_pack_conv_weight": (C.c_int, [C.POINTER(ConvGeom), C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "vsrb_conv2d_fwd": (C.c_int, [C.POINTER(ConvArgs), C.c_void_p]),
-    "vsrb_conv2d_takes_ring": (C.c_int, [C.POINTER(ConvArgs)]),
     "vsrb_conv_plan_info": (C.c_int, [C.POINTER(ConvGeom), C.POINTER(C.c_int32)]),
     "vsrb_conv2d_wgrad_multi": (C.c_int, [C.POINTER(ConvGeom), C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_int32),
                                           C.POINTER(C.c_void_p), C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,

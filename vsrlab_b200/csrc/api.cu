@@ -416,13 +416,6 @@ int vsrb_conv_plan_info(const vsrb_conv_geom* g, int32_t info[8]) {
     return VSRB_OK;
 }
 
-int vsrb_conv2d_takes_ring(const vsrb_conv_args* a) {
-    if (!a) return 0;
-    ConvPlan p;
-    if (make_plan(&a->geom, &p) != VSRB_OK || p.dtype != VSRB_BF16) return 0;
-    return ring_eligible(a, p) ? 1 : 0;
-}
-
 int vsrb_conv2d_fwd(const vsrb_conv_args* a, void* stream) {
     VSRB_CHECK_ARG(a, "null args");
     ConvPlan p;
@@ -467,8 +460,6 @@ int vsrb_conv2d_fwd(const vsrb_conv_args* a, void* stream) {
             VSRB_CHECK_ARG(false, "unknown epilogue %d", a->epilogue);
     }
     if (p.dtype == VSRB_BF16 && ring_eligible(a, p)) return launch_conv_ring(a, p, (cudaStream_t)stream);
-    VSRB_CHECK_ARG(!a->warp_flow, "the fused warp input exists on the ring-walk kernel only (bf16 3x3 64[+3] -> 64, launch large enough: "
-                                  "ask vsrb_conv2d_takes_ring first)");
     if (p.dtype == VSRB_BF16) return launch_conv_tc(a, p, (cudaStream_t)stream);
     return launch_conv_f32(a, p, (cudaStream_t)stream);
 }

@@ -22,6 +22,9 @@
 //   * CTA pairs (cta_group::2): the leader issues M = 256 MMAs for both CTAs' walks; each CTA holds half of the rows of
 //     every B tile (rank 0: [ky2 | ky1 lower half], rank 1: [ky1 upper half | ky0]).
 //
+// The propagation stem's flow_warp is not folded in here: epilogue warps that also sample the operand rows through the
+// flow were measured slower than the separate warp kernel plus this stem (DESIGN §4.1c).
+//
 // Work split: the rows of all column strips of a weight group are cut into 4 * gridDim.x ranges, either as one linear
 // index space (large launches: a range that starts mid-strip loads one halo row above and below, a range that crosses
 // into the next strip pays two zero rows - TMA out-of-bounds fill is the conv's zero padding) or, for small launches,
@@ -55,18 +58,10 @@ struct RingParams {
     CUtensorMap patch_map[2];   // per weight group: 3x3 im2col patches [32, W, H, imgs_per_group] box {32, 32, 1, 1} (SW64)
     int has_main, has_patch;    // operands: the 64-channel segment (N = 192 ring MMAs) / the 3-channel segment as K = 32 patches
     int num_slots, slot_bytes;
-    // fused backward warp (basicvsr.py:52-58,66-73): the main operand's rows are not loaded but SAMPLED from the previous
-    // time step's features with the flow field, by the epilogue warps, straight into the swizzled operand rows
-    int gather;
-    const __nv_bfloat16* feat;
-    long long feat_img_stride, feat_group_stride;      // elements
-    int feat_c;
-    const float2* flow;
-    long long flow_img_stride, flow_group_stride;      // float2 elements
     const uint8_t* w;      // ring image: [group][rank]{[kx][96 rows][128 B] | patch [32 rows][64 B]}
     const float* bias;     // [group][64]
     int has_res;
-    int H, W, strips, ipg;
+    int H, strips, ipg;
     int cols;              // ipg * strips column strips per weight group
     int rpc;               // ranges per column strip (aligned split), 0 = linear split of all rows
     uint32_t rows_g;       // cols * H
@@ -160,8 +155,7 @@ __device__ __forceinline__ void ring_fill_block(uint32_t taddr, const float* bia
 }
 
 // VSRB_RING_DEBUG bit 64: cycle counters of CTA (0,0): [0] issuer waiting for a free accumulator slot, [1] issuer waiting for
-// operand rows, [2] steps, [3] gather warp 4 waiting for a free operand slot, [4] its gather time, [5] its wait for finished
-// rows, [6] its epilogue time (vsrb_ring_debug_stats)
+// operand rows, [2] steps, [3] epilogue warp 4 waiting for finished rows, [4] its epilogue time (vsrb_ring_debug_stats)
 __device__ unsigned long long g_ring_stat[8];
 __device__ __forceinline__ long long ring_clock() { return clock64(); }
 
@@ -176,9 +170,9 @@ __global__ void __launch_bounds__(kRingThreads, 1) conv_ring_kernel(const __grid
     const int kSlots = P.num_slots;
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(base_ptr + 304);
     float* bias_s = reinterpret_cast<float*>(base_ptr + 512);
+    // then the weights, the operand slots (wres + VSRB_RING_W_BYTES) and one staging row per epilogue warp.  Each role
+    // computes the addresses it needs from wres: a slot base held from here on is spilled by ptxas.
     const uint32_t wres = base + kRingCtrl;
-    const uint32_t slots0 = wres + VSRB_RING_W_BYTES;
-    const uint32_t stg0 = slots0 + (uint32_t)P.num_slots * (uint32_t)P.slot_bytes;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int g = blockIdx.y;
@@ -196,16 +190,14 @@ __global__ void __launch_bounds__(kRingThreads, 1) conv_ring_kernel(const __grid
     }
 
     if (warp == 0 && lane == 0) {
-        if (P.has_main && !P.gather) prefetch_tensormap(&P.in_map);
+        if (P.has_main) prefetch_tensormap(&P.in_map);
         if (P.has_patch) prefetch_tensormap(&P.patch_map[g]);
         prefetch_tensormap(&P.out_map);
         if (P.has_res) prefetch_tensormap(&P.res_map);
     }
     if (warp == 1 && lane == 0) {
         for (int i = 0; i < kSlots; ++i) {
-            // a row is complete when its TMA bytes have landed (one expect_tx arrival of the leader's producer) and / or,
-            // with the fused warp, when the 4 + 4 gathering warps of the pair have written their quarters
-            mbar_init(full0 + 8 * i, (P.gather ? 8 : 0) + ((!P.gather || P.has_patch) ? 1 : 0));
+            mbar_init(full0 + 8 * i, 1);                          // the TMA bytes have landed (expect_tx of the leader's producer)
             mbar_init(empty0 + 8 * i, 1);
         }
         for (int i = 0; i < kRingAcc; ++i) {
@@ -257,9 +249,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) conv_ring_kernel(const __grid
             const uint32_t full_lead = mapa_rank(full0, 0);
             int slot = 0;
             uint32_t phase = 0;
-            const bool tma_main = P.has_main && !P.gather;
             for (int t = 0; t < S; ++t) {
-                if (!tma_main && !P.has_patch) break;              // fused warp without a patch operand: nothing to load
                 if ((P.debug & 1) && crank != 0) break;            // (timing experiment without loads: nothing paces this warp)
                 mbar_wait(empty0 + 8 * slot, phase ^ 1, P.dbg, 11, dead);
                 if (P.debug & 1) {
@@ -268,12 +258,12 @@ __global__ void __launch_bounds__(kRingThreads, 1) conv_ring_kernel(const __grid
                     int act = 0;
 #pragma unroll
                     for (int r = 0; r < 8; ++r) act += t < items[r] ? 1 : 0;
-                    mbar_expect_tx(full0 + 8 * slot, (uint32_t)act * ((tma_main ? 4096u : 0u) + (P.has_patch ? 2048u : 0u)));
+                    mbar_expect_tx(full0 + 8 * slot, (uint32_t)act * ((P.has_main ? 4096u : 0u) + (P.has_patch ? 2048u : 0u)));
                 }
                 if (lane < 4 && !wk.done && !(P.debug & 1)) {
                     const int li = wk.col / P.strips, strip = wk.col - li * P.strips;
-                    const uint32_t sa = slots0 + slot * P.slot_bytes;
-                    if (tma_main)
+                    const uint32_t sa = wres + VSRB_RING_W_BYTES + slot * P.slot_bytes;
+                    if (P.has_main)
                         tma_load_4d_pair(&P.in_map, full_lead + 8 * slot, sa + lane * 4096, 0, strip * kRingUW - 1, wk.y, g * P.ipg + li);
                     if (P.has_patch)      // the im2col row of this item's own pixels: no halo column, no kx shift
                         tma_load_4d_pair(&P.patch_map[g], full_lead + 8 * slot, sa + kRingSlotBytes + lane * 2048, 0, strip * kRingUW, wk.y, li);
@@ -316,7 +306,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) conv_ring_kernel(const __grid
                     }
                     tc_fence_after();
                     if (elect_one()) {
-                        const uint32_t sa = slots0 + slot * P.slot_bytes;
+                        const uint32_t sa = wres + VSRB_RING_W_BYTES + slot * P.slot_bytes;
                         const uint32_t a_lo = ((sa >> 4) & 0x3FFFu) | (1u << 16);
                         const uint32_t d0 = tmem_base + (uint32_t)b0 * 64u;
                         if (P.has_patch && !(P.debug & 4)) {
@@ -373,121 +363,16 @@ __global__ void __launch_bounds__(kRingThreads, 1) conv_ring_kernel(const __grid
             ring_range(P.rows_g, P.H, P.cols, P.rpc, n_ranges, pair0 + (int)crank * 4 + q, lo, hi);
             wk.init(lo, hi, P.H);
         }
-        const uint32_t stg = stg0 + (uint32_t)(eh * 4 + q) * 4096u;       // this warp's staging row
-        // ---- fused warp: this warp also PRODUCES the operand row of its quarter for the steps t with (t & 1) == eh -------
-        // Measured (tools/stem_bench.py, VSRB_RING_DEBUG=64, ncu source view profiles/r2_fused_stem_hot_sass.txt): a row costs
-        // its warp ~7 000 cycles - flow load -> taps -> two batches of tap loads are three dependent L2 round trips, plus
-        // ~600 instructions issued by one warp - against a budget of ~1 800 (two MMA steps minus the epilogue of a row).  The
-        // stand-alone flow_warp kernel hides the same latency with 64 warps per SM.  Splitting a row between the two warps of
-        // a quarter made it worse (each half still pays the fixed chain); shared-memory tap exchange instead of shuffles and
-        // leaving L1 more room changed nothing.
-        RingWalk fwk = wk;                        // cursor over the same items, kGatherAhead steps ahead of the epilogue
-        int fslot = 0;
-        uint32_t fphase = 0;
-        const uint32_t full_lead = mapa_rank(full0, 0);
-        constexpr int kGatherAhead = 4;           // even: a warp alternates between producing a row and finishing a row
-        auto fill_row = [&](bool mine) {
-            if (mine) {
-                const bool stat = (P.debug & 64) && blockIdx.x == 0 && blockIdx.y == 0 && warp == 4 && lane == 0;
-                const long long c0 = stat ? ring_clock() : 0;
-                mbar_wait(empty0 + 8 * fslot, fphase ^ 1, P.dbg, 19, dead);
-                const long long c1 = stat ? ring_clock() : 0;
-                if (stat) atomicAdd(&g_ring_stat[3], (unsigned long long)(c1 - c0));
-                if (!fwk.done) {
-                    const int li = fwk.col / P.strips, strip = fwk.col - li * P.strips;
-                    const int x = strip * kRingUW - 1 + lane, y = fwk.y;
-                    // lane = pixel for the sampling positions ...
-                    TapSet tp;
-                    const bool inside = y >= 0 && y < P.H && x >= 0 && x < P.W;        // outside: the conv's zero padding
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) { tp.off[k] = -1; tp.wgt[k] = 0.f; }
-                    if (inside) {
-                        const float2 f = (P.debug & 32) ? make_float2(0.25f, 0.25f)
-                                                        : __ldg(P.flow + (long long)g * P.flow_group_stride + (long long)li * P.flow_img_stride +
-                                                                (long long)y * P.W + x);
-                        float ix, iy;
-                        sample_pos((float)x + f.x, (float)y + f.y, P.W, P.H, ix, iy);
-                        make_taps(ix, iy, P.W, P.H, 0, tp);
-                    }
-                    const __nv_bfloat16* fb = P.feat + (long long)g * P.feat_group_stride + (long long)li * P.feat_img_stride;
-                    // ... and 8 lanes per pixel for the gathers: one load instruction reads four whole 128-byte pixel rows.
-                    // The tap tables change hands through this warp's (idle) staging row rather than 64 shuffles per row (measured
-                    // neutral: ncu's source view puts the row's stalls on the first uses of the flow and tap loads - three
-                    // dependent L2 round trips per row - not on instruction issue).
-                    if (lane == 0) bulk_wait_read<0>();            // a previous output row may still be read from there by the TMA
-                    __syncwarp();
-                    st_shared_v4(stg + (uint32_t)lane * 32u, (uint32_t)tp.off[0], (uint32_t)tp.off[1], (uint32_t)tp.off[2], (uint32_t)tp.off[3]);
-                    st_shared_v4(stg + (uint32_t)lane * 32u + 16u, __float_as_uint(tp.wgt[0]), __float_as_uint(tp.wgt[1]),
-                                 __float_as_uint(tp.wgt[2]), __float_as_uint(tp.wgt[3]));
-                    __syncwarp();
-                    const int j = lane & 7;
-                    // two batches of four pixel groups: all sixteen 16-byte loads of a batch are issued before the first result is
-                    // used (the shared-memory stores below are compiler barriers: without the explicit batching every group paid
-                    // its own L2 round trip, 8 in a row)
-#pragma unroll
-                    for (int half = 0; half < 2; ++half) {
-                        int o[4][4];
-                        float wt[4][4];
-                        uint4 u[4][4];
-#pragma unroll
-                        for (int gi = 0; gi < 4; ++gi) {
-                            const int src = (half * 4 + gi) * 4 + (lane >> 3);
-                            const uint4 to = ld_shared_v4(stg + (uint32_t)src * 32u), tw = ld_shared_v4(stg + (uint32_t)src * 32u + 16u);
-                            o[gi][0] = (int)to.x; o[gi][1] = (int)to.y; o[gi][2] = (int)to.z; o[gi][3] = (int)to.w;
-                            wt[gi][0] = __uint_as_float(tw.x); wt[gi][1] = __uint_as_float(tw.y);
-                            wt[gi][2] = __uint_as_float(tw.z); wt[gi][3] = __uint_as_float(tw.w);
-                        }
-#pragma unroll
-                        for (int gi = 0; gi < 4; ++gi)
-#pragma unroll
-                            for (int k = 0; k < 4; ++k)
-                                u[gi][k] = (o[gi][k] >= 0 && !(P.debug & 16)) ? __ldg(reinterpret_cast<const uint4*>(fb + (long long)o[gi][k] * P.feat_c + j * 8))
-                                                                             : make_uint4(0u, 0u, 0u, 0u);
-#pragma unroll
-                        for (int gi = 0; gi < 4; ++gi) {
-                            const int src = (half * 4 + gi) * 4 + (lane >> 3);
-                            float acc[8];
-#pragma unroll
-                            for (int e = 0; e < 8; ++e) acc[e] = 0.f;
-#pragma unroll
-                            for (int k = 0; k < 4; ++k) {
-                                if (o[gi][k] >= 0) {            // same order and arithmetic as flow_warp_kernel (warp.cu)
-                                    const uint32_t uu[4] = {u[gi][k].x, u[gi][k].y, u[gi][k].z, u[gi][k].w};
-#pragma unroll
-                                    for (int e = 0; e < 4; ++e) {
-                                        const float2 v2 = unpack_bf16(uu[e]);
-                                        acc[2 * e] = fmaf(v2.x, wt[gi][k], acc[2 * e]);
-                                        acc[2 * e + 1] = fmaf(v2.y, wt[gi][k], acc[2 * e + 1]);
-                                    }
-                                }
-                            }
-                            const uint32_t prow = slots0 + (uint32_t)fslot * (uint32_t)P.slot_bytes + (uint32_t)q * 4096u + (uint32_t)src * 128u;
-                            st_shared_v4(prow + (((uint32_t)j ^ ((uint32_t)src & 7u)) << 4), pack_bf16(acc[0], acc[1]), pack_bf16(acc[2], acc[3]),
-                                         pack_bf16(acc[4], acc[5]), pack_bf16(acc[6], acc[7]));
-                        }
-                    }
-                    fence_proxy_async();
-                }
-                __syncwarp();
-                // plain arrive, like every other cross-CTA handshake here: the rows are in THIS CTA's shared memory, published
-                // to the async proxy by the fence above; a .release.cluster arrive costs a cluster-wide fence per row (4x the kernel)
-                if (lane == 0) mbar_arrive_cluster(full_lead + 8 * fslot);
-                if (stat) atomicAdd(&g_ring_stat[4], (unsigned long long)(ring_clock() - c1));
-            }
-            fwk.next();
-            if (++fslot == kSlots) { fslot = 0; fphase ^= 1; }
-        };
+        // this warp's staging row
+        const uint32_t stg = wres + VSRB_RING_W_BYTES + (uint32_t)P.num_slots * (uint32_t)P.slot_bytes + (uint32_t)(eh * 4 + q) * 4096u;
         const float act_k = P.act_k;
         const uint32_t rbar = rbar0 + 8 * (eh * 4 + q);
         uint32_t rphase = 0;
         griddep_wait();        // this role reads / writes global memory other kernels on the stream own
-        if (P.gather)
-            for (int t = 0; t < kGatherAhead && t < S; ++t) fill_row((t & 1) == eh);
         // output row p (p = -1 is the ring's dummy first tenant) is complete after step p + 1; slot = (p + 1) mod 6
         int slot = 0;
         uint32_t sphase = 0;                      // ((p + 1) / 6) & 1
         for (int p = -1; p <= S - 2; ++p) {
-            if (P.gather && p + 1 + kGatherAhead < S) fill_row(((p + 1 + kGatherAhead) & 1) == eh);
             const bool mine = (p & 1) == eh;
             const bool valid = mine && p >= 0 && wk.valid();
             int li = 0, x0 = 0, y = 0;
@@ -516,7 +401,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) conv_ring_kernel(const __grid
             const long long e0 = estat ? ring_clock() : 0;
             mbar_wait(tfull0 + 8 * s, sp, P.dbg, 17, dead);
             const long long e1 = estat ? ring_clock() : 0;
-            if (estat) atomicAdd(&g_ring_stat[5], (unsigned long long)(e1 - e0));
+            if (estat) atomicAdd(&g_ring_stat[3], (unsigned long long)(e1 - e0));
             tc_fence_after();
             float v[64];
             if (valid) {
@@ -573,7 +458,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) conv_ring_kernel(const __grid
                     bulk_commit();
                 }
             }
-            if (estat) atomicAdd(&g_ring_stat[6], (unsigned long long)(ring_clock() - e1));
+            if (estat) atomicAdd(&g_ring_stat[4], (unsigned long long)(ring_clock() - e1));
         }
         if (lane == 0) bulk_wait_all();                            // staged rows must be read out before shared memory goes away
         tc_fence_before();
@@ -610,9 +495,6 @@ bool ring_eligible(const vsrb_conv_args* a, const ConvPlan& p) {
     if (p.ring & 1) {
         const int ms = p.ring_main_seg;
         if (a->in_c[ms] % 8 != 0 || (reinterpret_cast<uintptr_t>(a->in[ms]) & 15) != 0) return false;
-        if (a->warp_flow && (a->in_img_stride % 8 != 0 || a->in_group_stride % 8 != 0)) return false;
-    } else if (a->warp_flow) {
-        return false;
     }
     if (a->out_c % 8 != 0 || (reinterpret_cast<uintptr_t>(a->out) & 15) != 0) return false;
     if (a->out_img_stride % 8 != 0 || a->out_group_stride % 8 != 0 || a->out_img_stride < 0 || a->out_group_stride < 0) return false;
@@ -663,21 +545,9 @@ int launch_conv_ring(const vsrb_conv_args* a, const ConvPlan& p, cudaStream_t st
     P.has_res = a->residual != nullptr;
     P.has_main = (p.ring & 1) ? 1 : 0;
     P.has_patch = (p.ring & 2) ? 1 : 0;
-    P.gather = (a->warp_flow && P.has_main) ? 1 : 0;
-    if (P.gather) {
-        const int ms = p.ring_main_seg;
-        P.feat = reinterpret_cast<const __nv_bfloat16*>(a->in[ms]);
-        P.feat_c = a->in_c[ms];
-        P.feat_img_stride = a->in_img_stride ? a->in_img_stride : (long long)a->h * a->w * a->in_c[ms];
-        P.feat_group_stride = (a->in_img_stride || a->in_group_stride) ? a->in_group_stride : P.feat_img_stride * a->imgs_per_group;
-        P.flow = reinterpret_cast<const float2*>(a->warp_flow);
-        P.flow_img_stride = a->warp_flow_img_stride ? a->warp_flow_img_stride : (long long)a->h * a->w;
-        P.flow_group_stride = (a->warp_flow_img_stride || a->warp_flow_group_stride) ? a->warp_flow_group_stride
-                                                                                      : P.flow_img_stride * a->imgs_per_group;
-    }
     P.num_slots = P.has_patch ? kRingSlotsPatch : kRingSlots;
     P.slot_bytes = kRingSlotBytes + (P.has_patch ? kRingPatchBytes : 0);
-    P.H = a->h; P.W = a->w; P.strips = ceil_div(a->w, kRingUW); P.ipg = a->imgs_per_group;
+    P.H = a->h; P.strips = ceil_div(a->w, kRingUW); P.ipg = a->imgs_per_group;
     P.cols = P.ipg * P.strips;
     P.rows_g = (uint32_t)P.cols * (uint32_t)P.H;
     P.act_k = e.act_k;
@@ -687,7 +557,7 @@ int launch_conv_ring(const vsrb_conv_args* a, const ConvPlan& p, cudaStream_t st
         P.debug = dbg_env ? atoi(dbg_env) : 0;
     }
     cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    if (P.has_main && !P.gather) {
+    if (P.has_main) {
         const int ms = p.ring_main_seg;
         cuuint64_t dims[4] = {(cuuint64_t)a->in_c[ms], (cuuint64_t)a->w, (cuuint64_t)a->h, (cuuint64_t)a->batch};
         cuuint64_t strides[3] = {(cuuint64_t)a->in_c[ms] * 2, (cuuint64_t)a->w * a->in_c[ms] * 2, (cuuint64_t)a->h * a->w * a->in_c[ms] * 2};

@@ -14,6 +14,39 @@ namespace vsrb {
 // contiguous C*sizeof(T) run per tap), blend in fp32 and store one 16-byte vector.
 // Algorithmic traffic: C*sizeof(T) read + 8 B flow + C*sizeof(T) written per pixel.
 // ---------------------------------------------------------------------------------------
+struct TapSet {
+    int off[4];     // pixel index of the tap inside the image, or -1 when it contributes zero
+    float wgt[4];
+};
+
+__device__ __forceinline__ void sample_pos(float px, float py, int w, int h, float& ix, float& iy) {
+    // the reference normalises to [-1,1] and grid_sample(align_corners=True) maps back
+    float nx = 2.0f * px / (float)max(w - 1, 1) - 1.0f;
+    float ny = 2.0f * py / (float)max(h - 1, 1) - 1.0f;
+    ix = (nx + 1.0f) / 2.0f * (float)(w - 1);
+    iy = (ny + 1.0f) / 2.0f * (float)(h - 1);
+}
+
+__device__ __forceinline__ void make_taps(float ix, float iy, int w, int h, int border, TapSet& t) {
+    if (border) {
+        ix = fminf(fmaxf(ix, 0.f), (float)(w - 1));
+        iy = fminf(fmaxf(iy, 0.f), (float)(h - 1));
+    }
+    float fx = floorf(ix), fy = floorf(iy);
+    float wx1 = ix - fx, wy1 = iy - fy, wx0 = 1.f - wx1, wy0 = 1.f - wy1;
+    // guard the float->int conversion for wild flows
+    fx = fminf(fmaxf(fx, -2.f), (float)w);
+    fy = fminf(fmaxf(fy, -2.f), (float)h);
+    int x0 = (int)fx, y0 = (int)fy;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        int xi = x0 + (k & 1), yi = y0 + (k >> 1);
+        bool ok = xi >= 0 && xi < w && yi >= 0 && yi < h;
+        t.off[k] = ok ? yi * w + xi : -1;
+        t.wgt[k] = ((k & 1) ? wx1 : wx0) * ((k >> 1) ? wy1 : wy0);
+    }
+}
+
 template <typename T> struct Vec16;
 template <> struct Vec16<__nv_bfloat16> {
     static constexpr int N = 8;

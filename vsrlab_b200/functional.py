@@ -36,10 +36,6 @@ CLEAN_CHUNK = int(os.environ.get("VSRB_CLEAN_CHUNK", "60"))
 TAIL_CHUNK = int(os.environ.get("VSRB_TAIL_CHUNK", "15"))
 # the image stems (3 -> 64, 64+3 -> 64) read the frame as 3x3 im2col patches (K = 32 on the ring-walk kernel); 0 = nine K = 16 chunks
 STEM_PATCHES = os.environ.get("VSRB_STEM_PATCHES", "1") == "1"
-# flow_warp of the propagated features fused into the stem conv (basicvsr.py:52-58,66-73): the warped tensor never exists.
-# Opt-in: bit-identical results and no flow_warp launches, but measured slightly slower than the two separate kernels
-# (stem 49 us vs 19 + 2 x 12 us at the cfg3 shape: DESIGN.md) - the separate path is the default.
-FUSED_WARP = os.environ.get("VSRB_FUSED_WARP", "0") == "1"
 
 
 # Opt-in narrow `sr` output (default None = fp32, the reference's dtype).  "fp16" halves and "uint8" quarters the bytes a
@@ -267,7 +263,7 @@ def conv_chain(x: torch.Tensor, convs: Sequence[torch.nn.Conv2d], act: str = "re
 
 
 def _run_resblocks(cur, ca, stem_pc, block_pcs, n, h, w, mid_c, dt, device, tag, final_out=None, final_strides=(0, 0),
-                   extra_in=None, extra_c=0, groups=1, stem_patch=None, stem_patch_strides=(0, 0), stem_warp=None):
+                   extra_in=None, extra_c=0, groups=1, stem_patch=None, stem_patch_strides=(0, 0)):
     """stem (+LeakyReLU) then residual blocks on NHWC buffers; returns (tensor, channels).
     If `final_out` is given the last conv of the chain writes there (raw address allowed)."""
     tdt = ops.TORCH_DT[dt]
@@ -286,10 +282,9 @@ def _run_resblocks(cur, ca, stem_pc, block_pcs, n, h, w, mid_c, dt, device, tag,
     if stem_pc is not None:
         o, st = target(free[0])
         ins, cs = ([cur, extra_in], [ca, extra_c]) if extra_in is not None else ([cur], [ca])
-        wkw = {} if stem_warp is None else dict(warp_flow=stem_warp[0], warp_flow_strides=stem_warp[1], in_strides=stem_warp[2])
         ops.conv2d_fwd(stem_pc, ins, cs, n, h, w, act=ACT_LRELU, slope=0.1, out=o, out_c=mid_c,
                        out_img_stride=st[0], out_group_stride=st[1], patch=stem_patch, patch_img_stride=stem_patch_strides[0],
-                       patch_group_stride=stem_patch_strides[1], **wkw)
+                       patch_group_stride=stem_patch_strides[1])
         cur, ca, cur_i = o, mid_c, free[0]
     else:
         cur_i = -1
@@ -577,17 +572,9 @@ def _basicvsr_run(bv, lrs: torch.Tensor, dt: int, x_nhwc: Optional[torch.Tensor]
         lr_patch = ws("lr_patch", (n * t, h, w, 32), torch.bfloat16, dev)
         ops.im2col3x3(x_flat, lr_patch, n * t, h, w)
     pf = h * w * 32                                                      # elements of one frame of patches
-    fused = False
-    if FUSED_WARP and lr_patch is not None and t > 1:
-        # would the stem of a time step run on the ring-walk kernel (the one that can sample its input through the flow)?
-        fused = ops.conv2d_fwd(stem, [fbk.data_ptr(), pairs[0]], [mid_c, clr], 2 * n, h, w, act=ACT_LRELU, out=warped, out_c=mid_c,
-                               patch=lr_patch, patch_img_stride=t * pf, patch_group_stride=pf, warp_flow=flows_b,
-                               warp_flow_strides=((t - 1) * h * w, h * w), in_strides=(t * frame_el, frame_el), query_ring=True)
     for s in range(t):
         if s == 0:
             warped.zero_()
-        elif fused:
-            pass
         elif dt == BF16:
             # both directions in one launch: backward chain = bank frame t-s warped by flows_b[t-1-s], forward chain = bank
             # frame s-1 warped by flows_f[s-1] (basicvsr.py:52-54, 66-69)
@@ -603,20 +590,10 @@ def _basicvsr_run(bv, lrs: torch.Tensor, dt: int, x_nhwc: Optional[torch.Tensor]
         o_b = fbk.data_ptr() + (t - 1 - s) * frame_el * es
         o_f = ffw.data_ptr() + s * frame_el * es
         # group 0 (backward chain) reads frame t-1-s of every clip, group 1 (forward chain) frame s
-        src, stem_warp = warped, None
-        if fused and s > 0:
-            # the stem samples the previous step's features itself: backward chain = bank frame t-s warped by flows_b[t-1-s],
-            # forward chain = bank frame s-1 warped by flows_f[s-1]; strides between clips / between the two chains
-            src_b = fbk.data_ptr() + (t - s) * frame_el * es
-            src_f = ffw.data_ptr() + (s - 1) * frame_el * es
-            fl_b = flows_b.data_ptr() + (t - 1 - s) * h * w * 8
-            fl_f = flows_f.data_ptr() + (s - 1) * h * w * 8
-            src = src_b
-            stem_warp = (fl_b, ((t - 1) * h * w, (fl_f - fl_b) // 8), (t * frame_el, (src_f - src_b) // es))
-        _run_resblocks(src, mid_c, stem, blocks, 2 * n, h, w, mid_c, dt, dev, "pp", final_out=o_b,
+        _run_resblocks(warped, mid_c, stem, blocks, 2 * n, h, w, mid_c, dt, dev, "pp", final_out=o_b,
                        final_strides=(t * frame_el, (o_f - o_b) // es), extra_in=pairs[s], extra_c=clr, groups=2,
                        stem_patch=None if lr_patch is None else lr_patch.data_ptr() + (t - 1 - s) * pf * 2,
-                       stem_patch_strides=(t * pf, (2 * s - (t - 1)) * pf), stem_warp=stem_warp)
+                       stem_patch_strides=(t * pf, (2 * s - (t - 1)) * pf))
 
     # ---- fusion + upsampling + reconstruction, batched over frames (basicvsr.py:75-83) --
     ops.TAG = "tail"

@@ -143,13 +143,9 @@ def conv2d_fwd(pc: PackedConv, ins: Sequence, in_c: Sequence[int], batch: int, h
                imgs_per_group: Optional[int] = None, act: int = ACT_NONE, slope: float = 0.1, epilogue: int = EPI_NHWC,
                out=None, out_c: int = 0, out_img_stride: int = 0, out_group_stride: int = 0, residual=None, res_c: int = 0,
                f32_io=None, f32_in=None, aux_hw: Tuple[int, int] = (0, 0), max_ctas: int = 0, extra_flags: int = 0,
-               patch=None, patch_img_stride: int = 0, patch_group_stride: int = 0,
-               warp_flow=None, warp_flow_strides: Tuple[int, int] = (0, 0), in_strides: Tuple[int, int] = (0, 0),
-               query_ring: bool = False):
+               patch=None, patch_img_stride: int = 0, patch_group_stride: int = 0):
     """Enqueue one fused convolution.  `ins`, `out`, `residual`, `f32_io`, `f32_in` are tensors
-    (or raw int device addresses) that the caller keeps alive.  `warp_flow`: fused backward warp of the 64-channel
-    input (see vsrb_conv_args.warp_flow).  `query_ring=True` launches nothing and returns whether this launch
-    would run on the ring-walk kernel."""
+    (or raw int device addresses) that the caller keeps alive."""
     a = L.ConvArgs()
     a.geom = pc.geom
     if pc.split:
@@ -183,12 +179,6 @@ def conv2d_fwd(pc: PackedConv, ins: Sequence, in_c: Sequence[int], batch: int, h
     if patch is not None:
         a.patch = _p(patch)
         a.patch_img_stride, a.patch_group_stride = patch_img_stride, patch_group_stride
-    if warp_flow is not None:
-        a.warp_flow = _p(warp_flow)
-        a.warp_flow_img_stride, a.warp_flow_group_stride = warp_flow_strides
-        a.in_img_stride, a.in_group_stride = in_strides
-    if query_ring:
-        return bool(L.load().vsrb_conv2d_takes_ring(C.byref(a)))
     a.flags = (L.CONV_PDL if (pc.uses > 0 and PDL) else 0) | extra_flags
     pc.uses += 1
     if PROFILE is None:                            # the common case: no per-launch bookkeeping
