@@ -49,9 +49,15 @@ extern "C" {
 #define VSRB_ACT_RELU  1       /* reference conv.py:19,87 ; spynet.py:16-18        */
 #define VSRB_ACT_LRELU 2       /* LeakyReLU(slope); reference conv.py:98           */
 
-/* padding modes of the backward warp (reference spynet.py:95) */
-#define VSRB_PAD_ZEROS  0
-#define VSRB_PAD_BORDER 1
+/* padding modes of the backward warp (reference spynet.py:95; F.grid_sample padding_mode) */
+#define VSRB_PAD_ZEROS      0
+#define VSRB_PAD_BORDER     1
+#define VSRB_PAD_REFLECTION 2   /* vsrb_flow_warp_ex / _ex_bwd only */
+
+/* interpolation modes of vsrb_flow_warp_ex (F.grid_sample mode) */
+#define VSRB_INTERP_BILINEAR 0
+#define VSRB_INTERP_NEAREST  1
+#define VSRB_INTERP_BICUBIC  2
 
 /* conv epilogues (what happens to acc + bias) */
 #define VSRB_EPI_NHWC   0  /* act(acc+bias) [+ residual] -> NHWC `out`; with geom.pixshuf=2 the store
@@ -200,6 +206,20 @@ int vsrb_flow_warp(const void* x, int64_t x_img_stride /* elements, 0 = dense */
 int vsrb_flow_warp_groups(const void* x, int64_t x_img_stride, int64_t x_group_stride, const float* flow,
                           int64_t flow_img_stride, int64_t flow_group_stride, void* out, int32_t imgs_per_group,
                           int32_t groups, int32_t h, int32_t w, int32_t c, int32_t dtype, int32_t padding_mode, void* stream);
+
+/* vsrb_flow_warp with every F.grid_sample mode the reference flow_warp accepts (spynet.py:95-106 passes them through):
+ * interp VSRB_INTERP_*, padding_mode VSRB_PAD_* (reflection included), align_corners 0 / 1.  The pixel position
+ * (x + fx, y + fy) is normalised with max(size-1, 1) whatever align_corners is, as the reference does, and
+ * grid_sample's un-normalisation is applied to that.  dtype VSRB_BF16 (c % 8 == 0) or VSRB_F32 (c % 4 == 0);
+ * (bilinear, zeros | border, align_corners = 1) runs vsrb_flow_warp itself, and then VSRB_BF16X2 is accepted too.   */
+int vsrb_flow_warp_ex(const void* x, int64_t x_img_stride, const float* flow, int64_t flow_img_stride, void* out,
+                      int32_t n, int32_t h, int32_t w, int32_t c, int32_t dtype, int32_t interp,
+                      int32_t padding_mode, int32_t align_corners, void* stream);
+/* backward of vsrb_flow_warp_ex; the contract of vsrb_flow_warp_bwd (dx accumulated, dflow overwritten).  nearest:
+ * dflow = 0, as grid_sample's.  (bilinear, zeros | border, align_corners = 1) runs vsrb_flow_warp_bwd itself.      */
+int vsrb_flow_warp_ex_bwd(const void* x, const float* flow, const void* dout, float* dx, float* dflow,
+                          int32_t n, int32_t h, int32_t w, int32_t c, int32_t dtype, int32_t interp,
+                          int32_t padding_mode, int32_t align_corners, void* stream);
 
 /* ---- layout: module-boundary NCHW fp32 <-> internal NHWC ------------------------------
  * (the reference keeps NCHW throughout; these sit at the nn.Module boundary)            */

@@ -44,7 +44,6 @@ class Spynet(nn.Module):
 
 
 def flow_warp(x, flow, interpolation="bilinear", padding_mode="zeros", align_corners=True):
-    """Bilinear backward warp; `flow` is channels-last [T,h,w,2] (spynet.py:95-106)."""
-    if interpolation != "bilinear" or not align_corners:
-        raise NotImplementedError("the hot path only uses bilinear / align_corners=True (reference spynet.py:95)")
-    return VF.flow_warp(x, flow, padding_mode)
+    """Backward warp; `flow` is channels-last [T,h,w,2] (spynet.py:95-106).  Every F.grid_sample mode: interpolation
+    bilinear / nearest / bicubic, padding_mode zeros / border / reflection, align_corners True / False."""
+    return VF.flow_warp(x, flow, padding_mode, interpolation, align_corners)

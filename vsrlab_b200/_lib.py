@@ -15,7 +15,8 @@ LIB_PATH = HERE / "csrc" / "libvsrb200.so"
 
 BF16, F32, BF16X2 = 0, 1, 2
 ACT_NONE, ACT_RELU, ACT_LRELU = 0, 1, 2
-PAD_ZEROS, PAD_BORDER = 0, 1
+PAD_ZEROS, PAD_BORDER, PAD_REFLECTION = 0, 1, 2
+INTERP_BILINEAR, INTERP_NEAREST, INTERP_BICUBIC = 0, 1, 2
 EPI_NHWC, EPI_CLEAN, EPI_FLOW, EPI_SR = 0, 1, 2, 3
 CONV_PDL = 1
 CONV_SR_U8, CONV_SR_F16 = 2, 4
@@ -91,6 +92,8 @@ SYMBOLS = {
                                  C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "vsrb_flow_warp_groups": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p] + [C.c_int32] * 7 +
                               [C.c_void_p]),
+    "vsrb_flow_warp_ex": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p] + [C.c_int32] * 8 + [C.c_void_p]),
+    "vsrb_flow_warp_ex_bwd": (C.c_int, [C.c_void_p] * 5 + [C.c_int32] * 8 + [C.c_void_p]),
     "vsrb_nchw_to_nhwc": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int32] * 6 + [C.c_void_p]),
     "vsrb_nhwc_to_nchw": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int32] * 6 + [C.c_void_p]),
     "vsrb_spynet_pyramid_base": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int32] * 5 +

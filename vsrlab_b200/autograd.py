@@ -289,6 +289,33 @@ class WarpFn(torch.autograd.Function):
         return dx, dflow, None
 
 
+class WarpExFn(torch.autograd.Function):
+    """WarpFn with any grid_sample mode: interp INTERP_*, padding PAD_* (reflection included), align_corners."""
+
+    @staticmethod
+    def forward(ctx, x, flow, interp, padding, align_corners):
+        x = _cl(x)
+        flow = flow.contiguous()
+        b, c, h, w = x.shape
+        dt = BF16 if x.dtype == torch.bfloat16 else F32
+        out = torch.empty_like(x, memory_format=CL)
+        ops.flow_warp_ex(x, flow, out, b, h, w, c, dt, interp, padding, align_corners)
+        ctx.mode, ctx.dt = (interp, padding, align_corners), dt
+        ctx.save_for_backward(x, flow)
+        return out
+
+    @staticmethod
+    def backward(ctx, dout):
+        x, flow = ctx.saved_tensors
+        dout = _cl(dout)
+        b, c, h, w = x.shape
+        dx32 = torch.zeros((b, h, w, c), dtype=torch.float32, device=x.device) if ctx.needs_input_grad[0] else None
+        dflow = torch.empty_like(flow) if ctx.needs_input_grad[1] else None
+        ops.flow_warp_ex_bwd(x, flow, dout, dx32, dflow, b, h, w, c, ctx.dt, *ctx.mode)
+        dx = dx32.to(x.dtype).permute(0, 3, 1, 2) if dx32 is not None else None
+        return dx, dflow, None, None, None
+
+
 # --------------------------------------------------------------------------------------
 # the modules, differentiable
 # --------------------------------------------------------------------------------------

@@ -19,7 +19,7 @@ def needs_build() -> bool:
     if not OUT.exists():
         return True
     t = OUT.stat().st_mtime
-    deps = [CSRC / s for s in SOURCES] + [CSRC / "common.cuh", CSRC / "tc_ptx.cuh", HERE.parent / "include" / "vsrb200.h"]
+    deps = [CSRC / s for s in SOURCES] + [CSRC / "common.cuh", CSRC / "tc_ptx.cuh", CSRC / "warp_modes.cuh", HERE.parent / "include" / "vsrb200.h"]
     return any(d.stat().st_mtime > t for d in deps)
 
 

@@ -10,6 +10,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "warp_modes.cuh"
 
 namespace vsrb {
 
@@ -450,6 +451,173 @@ static int launch_warp_bwd(const T* x, const float2* flow, const T* dout, float*
     return VSRB_OK;
 }
 
+// ---------------------------------------------------------------------------------------
+// flow_warp_ex backward (nearest / bicubic, reflection, align_corners=False): flow_warp_bwd_kernel's work split, taps
+// from warp_modes.cuh.  dx: the output gradient scattered through the taps (fp32 atomics; reflected / clipped taps may
+// coincide).  dflow: sum over taps and channels of dout * x * d weight / d coordinate, times the derivative of the
+// coordinate wrt the flow (un-normalisation, and for nearest / bilinear the padding).  nearest: 0.
+// ---------------------------------------------------------------------------------------
+template <typename T>
+__device__ __forceinline__ void ld_vec(const T* p, float (&v)[16 / sizeof(T)]) {
+    if constexpr (sizeof(T) == 2) {
+        Ld8<T>::load(p, v);
+    } else {
+        const float4 q = __ldg(reinterpret_cast<const float4*>(p));
+        v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+    }
+}
+
+template <typename T, int TPP, int kInterp>
+__global__ void __launch_bounds__(256) flow_warp_ex_bwd_kernel(const T* __restrict__ x, const float2* __restrict__ flow,
+                                                               const T* __restrict__ dout, float* __restrict__ dx,
+                                                               float2* __restrict__ dflow, int n, int h, int w, int pad, int align,
+                                                               int tpp_rt) {
+    constexpr int VEC = 16 / sizeof(T);
+    const int tpp = TPP > 0 ? TPP : tpp_rt;            // TPP == 0: any channel count; dflow must then be zeroed (atomics)
+    const int C = tpp * VEC;
+    const int hw = h * w;
+    const long long total = (long long)n * hw * tpp;
+    const long long total_up = (total + 31) / 32 * 32;          // whole warps iterate together (shuffles below)
+    for (long long i0 = (long long)blockIdx.x * 256 + threadIdx.x; i0 < total_up; i0 += (long long)gridDim.x * 256) {
+        const bool live = i0 < total;
+        const long long i = live ? i0 : total - 1;              // dead lanes shadow the last item, write nothing
+        const int part = (int)(i % tpp);
+        const long long pix = i / tpp;
+        const int img = (int)(pix / hw), r = (int)(pix - (long long)img * hw);
+        const int yy = r / w, xx = r - yy * w;
+        const float2 f = __ldg(flow + pix);
+        float ix = ex_unnormalize((float)xx + f.x, w, align), iy = ex_unnormalize((float)yy + f.y, h, align);
+        float gmx = ex_unnormalize_grad(w, align), gmy = ex_unnormalize_grad(h, align);
+        const T* xb = x + (long long)img * hw * C + part * VEC;
+        float* dxb = dx + (long long)img * hw * C + part * VEC;
+        float go[VEC];
+        ld_vec<T>(dout + pix * C + part * VEC, go);
+        float gx = 0.f, gy = 0.f;
+        if constexpr (kInterp == VSRB_INTERP_NEAREST) {
+            float g;
+            const int xi = ex_index(nearbyintf(ex_pad_coord(ix, w, pad, align, g)), w);
+            const int yi = ex_index(nearbyintf(ex_pad_coord(iy, h, pad, align, g)), h);
+            if (dx && live && xi >= 0 && yi >= 0) {
+#pragma unroll
+                for (int j = 0; j < VEC; ++j) atomicAdd(dxb + ((long long)yi * w + xi) * C + j, go[j]);
+            }
+            gmx = gmy = 0.f;                           // piecewise constant in the flow
+        } else if constexpr (kInterp == VSRB_INTERP_BILINEAR) {
+            float px, py;
+            ix = ex_pad_coord(ix, w, pad, align, px);
+            iy = ex_pad_coord(iy, h, pad, align, py);
+            gmx *= px;
+            gmy *= py;
+            float fx = floorf(ix), fy = floorf(iy);
+            const float wx1 = ix - fx, wy1 = iy - fy, wx0 = 1.f - wx1, wy0 = 1.f - wy1;
+            fx = fminf(fmaxf(fx, -2.f), (float)w);
+            fy = fminf(fmaxf(fy, -2.f), (float)h);
+            const int x0 = (int)fx, y0 = (int)fy;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const int xi = x0 + (k & 1), yi = y0 + (k >> 1);
+                if (xi < 0 || xi >= w || yi < 0 || yi >= h) continue;
+                const long long tp = ((long long)yi * w + xi) * C;
+                if (dx && live) {
+                    const float wgt = ((k & 1) ? wx1 : wx0) * ((k >> 1) ? wy1 : wy0);
+#pragma unroll
+                    for (int j = 0; j < VEC; ++j) atomicAdd(dxb + tp + j, go[j] * wgt);
+                }
+                if (dflow) {
+                    float xv[VEC];
+                    ld_vec<T>(xb + tp, xv);
+                    float dot = 0.f;
+#pragma unroll
+                    for (int j = 0; j < VEC; ++j) dot = fmaf(go[j], xv[j], dot);
+                    gx = fmaf(dot, ((k & 1) ? 1.f : -1.f) * ((k >> 1) ? wy1 : wy0), gx);
+                    gy = fmaf(dot, ((k >> 1) ? 1.f : -1.f) * ((k & 1) ? wx1 : wx0), gy);
+                }
+            }
+        } else {
+            const float fx = floorf(ix), fy = floorf(iy);
+            float wx[4], wy[4], dwx[4], dwy[4];
+            cubic_weights(ix - fx, wx);
+            cubic_weights(iy - fy, wy);
+            cubic_weights_grad(ix - fx, dwx);
+            cubic_weights_grad(iy - fy, dwy);
+            int xo[4];
+#pragma unroll
+            for (int q = 0; q < 4; ++q) xo[q] = ex_bicubic_tap(fx + (float)(q - 1), w, pad, align);
+#pragma unroll
+            for (int rr = 0; rr < 4; ++rr) {
+                const int yi = ex_bicubic_tap(fy + (float)(rr - 1), h, pad, align);
+                if (yi < 0) continue;
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    if (xo[q] < 0) continue;
+                    const long long tp = ((long long)yi * w + xo[q]) * C;
+                    if (dx && live) {
+                        const float wgt = wx[q] * wy[rr];
+#pragma unroll
+                        for (int j = 0; j < VEC; ++j) atomicAdd(dxb + tp + j, go[j] * wgt);
+                    }
+                    if (dflow) {
+                        float xv[VEC];
+                        ld_vec<T>(xb + tp, xv);
+                        float dot = 0.f;
+#pragma unroll
+                        for (int j = 0; j < VEC; ++j) dot = fmaf(go[j], xv[j], dot);
+                        gx = fmaf(dot, dwx[q] * wy[rr], gx);
+                        gy = fmaf(dot, wx[q] * dwy[rr], gy);
+                    }
+                }
+            }
+        }
+        if (dflow) {
+            if (TPP > 0) {
+#pragma unroll
+                for (int o = TPP / 2; o > 0; o >>= 1) {
+                    gx += __shfl_xor_sync(0xffffffffu, gx, o);
+                    gy += __shfl_xor_sync(0xffffffffu, gy, o);
+                }
+                if (part == 0 && live) dflow[pix] = make_float2(gx * gmx, gy * gmy);
+            } else if (live && kInterp != VSRB_INTERP_NEAREST) {
+                atomicAdd(&dflow[pix].x, gx * gmx);
+                atomicAdd(&dflow[pix].y, gy * gmy);
+            }
+        }
+    }
+}
+
+template <typename T, int kInterp>
+static void launch_warp_ex_bwd_t(const T* x, const float2* flow, const T* dout, float* dx, float2* dflow, int n, int h, int w,
+                                 int c, int pad, int align, cudaStream_t s) {
+    constexpr int VEC = 16 / sizeof(T);
+    const int tpp = c / VEC;
+    const long long total = (long long)n * h * w * tpp;
+    long long b = (total + 255) / 256;
+    if (b > 148 * 16) b = 148 * 16;                    // grid-stride: a pixel's lanes stay in one warp (see launch_warp_bwd)
+    const int blocks = (int)b;
+#define VSRB_WARP_EX_BWD(TPP) \
+    flow_warp_ex_bwd_kernel<T, TPP, kInterp><<<blocks, 256, 0, s>>>(x, flow, dout, dx, dflow, n, h, w, pad, align, tpp)
+    switch (tpp) {
+        case 1: VSRB_WARP_EX_BWD(1); break;
+        case 2: VSRB_WARP_EX_BWD(2); break;
+        case 4: VSRB_WARP_EX_BWD(4); break;
+        case 8: VSRB_WARP_EX_BWD(8); break;
+        case 16: VSRB_WARP_EX_BWD(16); break;
+        case 32: VSRB_WARP_EX_BWD(32); break;
+        default:
+            if (dflow) cudaMemsetAsync(dflow, 0, sizeof(float2) * (size_t)n * h * w, s);
+            VSRB_WARP_EX_BWD(0);
+            break;
+    }
+#undef VSRB_WARP_EX_BWD
+}
+
+template <typename T>
+static void launch_warp_ex_bwd(const T* x, const float2* flow, const T* dout, float* dx, float2* dflow, int n, int h, int w, int c,
+                               int interp, int pad, int align, cudaStream_t s) {
+    if (interp == VSRB_INTERP_NEAREST) launch_warp_ex_bwd_t<T, VSRB_INTERP_NEAREST>(x, flow, dout, dx, dflow, n, h, w, c, pad, align, s);
+    else if (interp == VSRB_INTERP_BICUBIC) launch_warp_ex_bwd_t<T, VSRB_INTERP_BICUBIC>(x, flow, dout, dx, dflow, n, h, w, c, pad, align, s);
+    else launch_warp_ex_bwd_t<T, VSRB_INTERP_BILINEAR>(x, flow, dout, dx, dflow, n, h, w, c, pad, align, s);
+}
+
 int launch_wgrad_tc(const void* x, int x_c, int c0, int ci_off, const void* dz, int dz_c, int batch, int h, int w, int cout,
                     int cin_total, float* dw, cudaStream_t stream, float* db = nullptr);
 int launch_bias_grad(const void* dz, int dz_c, long long pixels, int cout, int dtype, float* db, cudaStream_t s);
@@ -651,6 +819,36 @@ int vsrb_flow_warp_bwd(const void* x, const float* flow, const void* dout, float
                                     padding_mode, s);
     }
     if (rc != VSRB_OK) return rc;
+    VSRB_LAUNCH_CHECK();
+    return VSRB_OK;
+}
+
+int vsrb_flow_warp_ex_bwd(const void* x, const float* flow, const void* dout, float* dx, float* dflow, int32_t n, int32_t h,
+                          int32_t w, int32_t c, int32_t dtype, int32_t interp, int32_t padding_mode, int32_t align_corners,
+                          void* stream) {
+    VSRB_CHECK_ARG(flow && dout && (dx || dflow) && n >= 1 && h >= 1 && w >= 1, "flow_warp_ex_bwd: bad arguments");
+    VSRB_CHECK_ARG(!dflow || x, "flow_warp_ex_bwd: the flow gradient needs the forward input x");
+    VSRB_CHECK_ARG(interp == VSRB_INTERP_BILINEAR || interp == VSRB_INTERP_NEAREST || interp == VSRB_INTERP_BICUBIC,
+                   "flow_warp_ex_bwd: bad interpolation mode %d (bilinear 0, nearest 1, bicubic 2)", interp);
+    VSRB_CHECK_ARG(padding_mode == VSRB_PAD_ZEROS || padding_mode == VSRB_PAD_BORDER || padding_mode == VSRB_PAD_REFLECTION,
+                   "flow_warp_ex_bwd: bad padding mode %d (zeros 0, border 1, reflection 2)", padding_mode);
+    VSRB_CHECK_ARG(align_corners == 0 || align_corners == 1, "flow_warp_ex_bwd: align_corners must be 0 or 1 (got %d)", align_corners);
+    VSRB_CHECK_ARG(dtype == VSRB_BF16 || dtype == VSRB_F32, "flow_warp_ex_bwd: dtype must be bf16 or fp32 (got %d)", dtype);
+    if (interp == VSRB_INTERP_BILINEAR && align_corners && padding_mode != VSRB_PAD_REFLECTION)
+        return vsrb_flow_warp_bwd(x, flow, dout, dx, dflow, n, h, w, c, dtype, padding_mode, stream);
+    VSRB_CHECK_ARG((long long)h * w < (1LL << 31) && (long long)n * h * w * c < (1LL << 40), "flow_warp_ex_bwd: tensor too large");
+    cudaStream_t s = (cudaStream_t)stream;
+    if (dtype == VSRB_BF16) {
+        VSRB_CHECK_ARG(c >= 8 && c % 8 == 0, "flow_warp_ex_bwd: bf16 needs c %% 8 == 0 (got %d)", c);
+        launch_warp_ex_bwd<__nv_bfloat16>(reinterpret_cast<const __nv_bfloat16*>(x), reinterpret_cast<const float2*>(flow),
+                                          reinterpret_cast<const __nv_bfloat16*>(dout), dx, reinterpret_cast<float2*>(dflow), n, h, w,
+                                          c, interp, padding_mode, align_corners, s);
+    } else {
+        VSRB_CHECK_ARG(c >= 4 && c % 4 == 0, "flow_warp_ex_bwd: fp32 needs c %% 4 == 0 (got %d)", c);
+        launch_warp_ex_bwd<float>(reinterpret_cast<const float*>(x), reinterpret_cast<const float2*>(flow),
+                                  reinterpret_cast<const float*>(dout), dx, reinterpret_cast<float2*>(dflow), n, h, w, c, interp,
+                                  padding_mode, align_corners, s);
+    }
     VSRB_LAUNCH_CHECK();
     return VSRB_OK;
 }

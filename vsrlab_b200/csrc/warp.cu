@@ -1,6 +1,7 @@
 // Memory-bound resampling kernels: backward warp (flow_warp), layout changes, SPyNet glue.
 // All activations NHWC; every gather is a 16-byte vector of consecutive channels.
 #include "common.cuh"
+#include "warp_modes.cuh"
 
 namespace vsrb {
 
@@ -168,6 +169,152 @@ static int launch_flow_warp(const T* x, long long xs, const float2* flow, long l
         default: flow_warp_kernel<T, 0><<<blocks, 256, 0, s>>>(x, xs, flow, fs, out, n, h, w, border, tpp, ipg, xg, fg); break;
     }
     return VSRB_OK;
+}
+
+// ---------------------------------------------------------------------------------------
+// flow_warp_ex: the other F.grid_sample modes (nearest / bicubic, reflection padding, align_corners=False).
+// The structure of flow_warp_kernel: taps built once per pixel into shared memory, then C/VEC threads per pixel gather
+// 16-byte channel vectors and blend in fp32.  nearest keeps one tap, bilinear four (a TapSet), bicubic a separable
+// 4 + 4 table (column indices, row offsets, weights; -1 = reads zero) instead of 16 offsets.
+// ---------------------------------------------------------------------------------------
+struct NearestTap {
+    int off;        // pixel index of the tap, or -1
+};
+struct BicubicTaps {
+    int xo[4];      // column of tap floor(ix) - 1 + i after padding, or -1
+    int yo[4];      // row offset (row * w) of tap floor(iy) - 1 + j after padding, or -1
+    float wx[4], wy[4];
+};
+template <int kInterp> struct ExTapsOf { using type = TapSet; };
+template <> struct ExTapsOf<VSRB_INTERP_NEAREST> { using type = NearestTap; };
+template <> struct ExTapsOf<VSRB_INTERP_BICUBIC> { using type = BicubicTaps; };
+
+__device__ __forceinline__ void make_taps_ex(float ix, float iy, int w, int h, int pad, int align, NearestTap& t) {
+    float g;
+    const int xi = ex_index(nearbyintf(ex_pad_coord(ix, w, pad, align, g)), w);     // round half to even
+    const int yi = ex_index(nearbyintf(ex_pad_coord(iy, h, pad, align, g)), h);
+    t.off = (xi >= 0 && yi >= 0) ? yi * w + xi : -1;
+}
+__device__ __forceinline__ void make_taps_ex(float ix, float iy, int w, int h, int pad, int align, TapSet& t) {
+    float g;
+    make_taps(ex_pad_coord(ix, w, pad, align, g), ex_pad_coord(iy, h, pad, align, g), w, h, 0, t);
+}
+__device__ __forceinline__ void make_taps_ex(float ix, float iy, int w, int h, int pad, int align, BicubicTaps& t) {
+    const float fx = floorf(ix), fy = floorf(iy);
+    cubic_weights(ix - fx, t.wx);
+    cubic_weights(iy - fy, t.wy);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        t.xo[i] = ex_bicubic_tap(fx + (float)(i - 1), w, pad, align);
+        const int yi = ex_bicubic_tap(fy + (float)(i - 1), h, pad, align);
+        t.yo[i] = yi >= 0 ? yi * w : -1;
+    }
+}
+
+template <typename T, int VEC>
+__device__ __forceinline__ void gather_ex(const T* img, int C, const NearestTap& t, float (&acc)[VEC]) {
+    if (t.off >= 0) Vec16<T>::load(img + (long long)t.off * C, acc);
+}
+template <typename T, int VEC>
+__device__ __forceinline__ void gather_ex(const T* img, int C, const TapSet& t, float (&acc)[VEC]) {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        if (t.off[k] >= 0) {
+            float v[VEC];
+            Vec16<T>::load(img + (long long)t.off[k] * C, v);
+#pragma unroll
+            for (int j = 0; j < VEC; ++j) acc[j] = fmaf(v[j], t.wgt[k], acc[j]);
+        }
+    }
+}
+template <typename T, int VEC>
+__device__ __forceinline__ void gather_ex(const T* img, int C, const BicubicTaps& t, float (&acc)[VEC]) {
+    // along x within each row, then across the rows (ATen's cubic_interp1d order)
+#pragma unroll
+    for (int r = 0; r < 4; ++r) {
+        if (t.yo[r] < 0) continue;
+        float row[VEC];
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) row[j] = 0.f;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            if (t.xo[q] < 0) continue;
+            float v[VEC];
+            Vec16<T>::load(img + (long long)(t.yo[r] + t.xo[q]) * C, v);
+#pragma unroll
+            for (int j = 0; j < VEC; ++j) row[j] = fmaf(v[j], t.wx[q], row[j]);
+        }
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) acc[j] = fmaf(row[j], t.wy[r], acc[j]);
+    }
+}
+
+// (256, 1): under the plain (256) bound ptxas held the bf16 bicubic variants to 40 - 48 registers and spilled
+template <typename T, int TPP, int kInterp>
+__global__ void __launch_bounds__(256, 1) flow_warp_ex_kernel(const T* __restrict__ x, long long x_stride,
+                                                           const float2* __restrict__ flow, long long f_stride,
+                                                           T* __restrict__ out, int n, int h, int w, int pad, int align,
+                                                           int tpp_rt) {
+    using Taps = typename ExTapsOf<kInterp>::type;
+    __shared__ Taps taps[kWarpPix];
+    __shared__ long long bases[kWarpPix];
+    constexpr int VEC = Vec16<T>::N;
+    const int tpp = TPP > 0 ? TPP : tpp_rt;            // TPP == 0: any channel count (runtime divisions)
+    const int C = tpp * VEC;
+    const int hw = h * w;
+    const int total = n * hw;                          // launcher guarantees < 2^31
+    const int pix0 = blockIdx.x * kWarpPix;
+    {
+        const int pix = pix0 + threadIdx.x;
+        if (pix < total) {
+            const int img = pix / hw, r = pix - img * hw;
+            const int yy = r / w, xx = r - yy * w;
+            const float2 f = __ldg(flow + (long long)img * f_stride + r);
+            make_taps_ex(ex_unnormalize((float)xx + f.x, w, align), ex_unnormalize((float)yy + f.y, h, align), w, h, pad, align,
+                         taps[threadIdx.x]);
+            bases[threadIdx.x] = (long long)img * x_stride;
+        }
+    }
+    __syncthreads();
+    const int npix = min(kWarpPix, total - pix0);
+    const int work = npix * tpp;
+    constexpr int kUnroll = kInterp == VSRB_INTERP_BICUBIC ? 1 : 4;     // bicubic: 16 loads in flight per item already
+#pragma unroll kUnroll
+    for (int i = threadIdx.x; i < work; i += 256) {
+        const int lp = i / tpp, part = i % tpp;          // compile-time power of two: shift / mask
+        float acc[VEC];
+#pragma unroll
+        for (int j = 0; j < VEC; ++j) acc[j] = 0.f;
+        gather_ex<T, VEC>(x + bases[lp] + part * VEC, C, taps[lp], acc);       // the table is read from shared memory
+        Vec16<T>::store(out + (long long)(pix0 + lp) * C + part * VEC, acc);
+    }
+}
+
+template <typename T, int kInterp>
+static void launch_flow_warp_ex_t(const T* x, long long xs, const float2* flow, long long fs, T* out, int n, int h, int w, int c,
+                                  int pad, int align, cudaStream_t s) {
+    constexpr int VEC = Vec16<T>::N;
+    const int tpp = c / VEC;
+    const int blocks = (int)(((long long)n * h * w + kWarpPix - 1) / kWarpPix);
+#define VSRB_WARP_EX(TPP) flow_warp_ex_kernel<T, TPP, kInterp><<<blocks, 256, 0, s>>>(x, xs, flow, fs, out, n, h, w, pad, align, tpp)
+    switch (tpp) {
+        case 1: VSRB_WARP_EX(1); break;
+        case 2: VSRB_WARP_EX(2); break;
+        case 4: VSRB_WARP_EX(4); break;
+        case 8: VSRB_WARP_EX(8); break;
+        case 16: VSRB_WARP_EX(16); break;
+        case 32: VSRB_WARP_EX(32); break;
+        default: VSRB_WARP_EX(0); break;
+    }
+#undef VSRB_WARP_EX
+}
+
+template <typename T>
+static void launch_flow_warp_ex(const T* x, long long xs, const float2* flow, long long fs, T* out, int n, int h, int w, int c,
+                                int interp, int pad, int align, cudaStream_t s) {
+    if (interp == VSRB_INTERP_NEAREST) launch_flow_warp_ex_t<T, VSRB_INTERP_NEAREST>(x, xs, flow, fs, out, n, h, w, c, pad, align, s);
+    else if (interp == VSRB_INTERP_BICUBIC) launch_flow_warp_ex_t<T, VSRB_INTERP_BICUBIC>(x, xs, flow, fs, out, n, h, w, c, pad, align, s);
+    else launch_flow_warp_ex_t<T, VSRB_INTERP_BILINEAR>(x, xs, flow, fs, out, n, h, w, c, pad, align, s);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -556,6 +703,37 @@ int vsrb_flow_warp_groups(const void* x, int64_t x_img_stride, int64_t x_group_s
                                              reinterpret_cast<__nv_bfloat16*>(out), imgs_per_group * groups, h, w, c, padding_mode,
                                              (cudaStream_t)stream, imgs_per_group, x_group_stride, flow_group_stride);
     if (rc != VSRB_OK) return rc;
+    VSRB_LAUNCH_CHECK();
+    return VSRB_OK;
+}
+
+int vsrb_flow_warp_ex(const void* x, int64_t x_img_stride, const float* flow, int64_t flow_img_stride, void* out, int32_t n,
+                      int32_t h, int32_t w, int32_t c, int32_t dtype, int32_t interp, int32_t padding_mode, int32_t align_corners,
+                      void* stream) {
+    VSRB_CHECK_ARG(x && flow && out && n >= 1 && h >= 1 && w >= 1, "flow_warp_ex: bad arguments");
+    VSRB_CHECK_ARG(interp == VSRB_INTERP_BILINEAR || interp == VSRB_INTERP_NEAREST || interp == VSRB_INTERP_BICUBIC,
+                   "flow_warp_ex: bad interpolation mode %d (bilinear 0, nearest 1, bicubic 2)", interp);
+    VSRB_CHECK_ARG(padding_mode == VSRB_PAD_ZEROS || padding_mode == VSRB_PAD_BORDER || padding_mode == VSRB_PAD_REFLECTION,
+                   "flow_warp_ex: bad padding mode %d (zeros 0, border 1, reflection 2)", padding_mode);
+    VSRB_CHECK_ARG(align_corners == 0 || align_corners == 1, "flow_warp_ex: align_corners must be 0 or 1 (got %d)", align_corners);
+    // the propagation warp's mode: the existing kernel, so these results are the ones vsrb_flow_warp gives
+    if (interp == VSRB_INTERP_BILINEAR && align_corners && padding_mode != VSRB_PAD_REFLECTION)
+        return vsrb_flow_warp(x, x_img_stride, flow, flow_img_stride, out, n, h, w, c, dtype, padding_mode, stream);
+    VSRB_CHECK_ARG((long long)n * h * w < (1LL << 31), "flow_warp_ex: more than 2^31 pixels in one call");
+    const long long xs = x_img_stride ? x_img_stride : (long long)h * w * c;
+    const long long fs = flow_img_stride ? flow_img_stride : (long long)h * w;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (dtype == VSRB_BF16) {
+        VSRB_CHECK_ARG(c >= 8 && c % 8 == 0, "flow_warp_ex: bf16 needs c %% 8 == 0 (got %d)", c);
+        launch_flow_warp_ex<__nv_bfloat16>(reinterpret_cast<const __nv_bfloat16*>(x), xs, reinterpret_cast<const float2*>(flow), fs,
+                                           reinterpret_cast<__nv_bfloat16*>(out), n, h, w, c, interp, padding_mode, align_corners, s);
+    } else if (dtype == VSRB_F32) {
+        VSRB_CHECK_ARG(c >= 4 && c % 4 == 0, "flow_warp_ex: fp32 needs c %% 4 == 0 (got %d)", c);
+        launch_flow_warp_ex<float>(reinterpret_cast<const float*>(x), xs, reinterpret_cast<const float2*>(flow), fs,
+                                   reinterpret_cast<float*>(out), n, h, w, c, interp, padding_mode, align_corners, s);
+    } else {
+        VSRB_CHECK_ARG(false, "flow_warp_ex: this mode needs dtype bf16 or fp32 (got %d)", dtype);
+    }
     VSRB_LAUNCH_CHECK();
     return VSRB_OK;
 }

@@ -21,8 +21,8 @@ from typing import Dict, List, Optional, Sequence, Tuple
 import torch
 
 from . import ops
-from ._lib import (ACT_LRELU, ACT_NONE, ACT_RELU, BF16, BF16X2, EPI_CLEAN, EPI_FLOW, EPI_NHWC, EPI_SR, F32, PAD_BORDER,
-                   PAD_ZEROS, VsrbError)
+from ._lib import (ACT_LRELU, ACT_NONE, ACT_RELU, BF16, BF16X2, EPI_CLEAN, EPI_FLOW, EPI_NHWC, EPI_SR, F32, INTERP_BICUBIC,
+                   INTERP_BILINEAR, INTERP_NEAREST, PAD_BORDER, PAD_REFLECTION, PAD_ZEROS, VsrbError)
 
 _forced: Optional[int] = None
 # "fp32" = fp32-accurate mode.  Default implementation: split-bf16 (x = hi + lo) on the tensor cores, three MMA passes
@@ -345,8 +345,22 @@ def unet_discriminator_forward(D, img: torch.Tensor) -> torch.Tensor:
         return A.unet_discriminator(D, img)
 
 
-def flow_warp(x: torch.Tensor, flow: torch.Tensor, padding_mode: str = "zeros") -> torch.Tensor:
-    """flow_warp(x [T,c,h,w], flow [T,h,w,2]) (spynet.py:95-106)."""
+_WARP_PADS = {"zeros": PAD_ZEROS, "border": PAD_BORDER, "reflection": PAD_REFLECTION}
+_WARP_INTERPS = {"bilinear": INTERP_BILINEAR, "nearest": INTERP_NEAREST, "bicubic": INTERP_BICUBIC}
+
+
+def flow_warp(x: torch.Tensor, flow: torch.Tensor, padding_mode: str = "zeros", interpolation: str = "bilinear",
+              align_corners: bool = True) -> torch.Tensor:
+    """flow_warp(x [T,c,h,w], flow [T,h,w,2]) (spynet.py:95-106) with any mode F.grid_sample accepts.  The propagation
+    warp's mode (bilinear, zeros / border, align_corners) runs the propagation kernel; the others run flow_warp_ex (fp32
+    NHWC in fp32 mode, bf16 in bf16 mode)."""
+    if padding_mode not in _WARP_PADS:
+        raise ValueError(f"flow_warp: padding_mode must be 'zeros', 'border' or 'reflection', got {padding_mode!r}")
+    if interpolation not in _WARP_INTERPS:
+        raise ValueError(f"flow_warp: interpolation must be 'bilinear', 'nearest' or 'bicubic', got {interpolation!r}")
+    align_corners = bool(align_corners)
+    if interpolation != "bilinear" or padding_mode == "reflection" or not align_corners:
+        return _flow_warp_ex(x, flow, _WARP_INTERPS[interpolation], _WARP_PADS[padding_mode], align_corners)
     x = _check_input(x, "input")
     flow = _check_input(flow, "flow").contiguous()
     n, c, h, w = x.shape
@@ -370,6 +384,30 @@ def flow_warp(x: torch.Tensor, flow: torch.Tensor, padding_mode: str = "zeros") 
     xin, _ = _to_nhwc(x, dt, "m_in", ca)
     out = ws("m_out", (n, h, w, ca), ops.TORCH_DT[dt], x.device)
     ops.flow_warp(xin, flow, out, n, h, w, ca, dt, PAD_BORDER if padding_mode == "border" else PAD_ZEROS)
+    return _to_nchw(out, n, c, h, w, ca, dt)
+
+
+def _flow_warp_ex(x: torch.Tensor, flow: torch.Tensor, interp: int, pad: int, align_corners: bool) -> torch.Tensor:
+    x = _check_input(x, "input")
+    flow = _check_input(flow, "flow").contiguous()
+    n, c, h, w = x.shape
+    nv = 1
+    if _wants_grad(None, x, flow):
+        AG = _autograd()
+        while nv * 4 < c:
+            nv *= 2
+        xp = torch.nn.functional.pad(x, (0, 0, 0, 0, 0, nv * 4 - c)).contiguous(memory_format=torch.channels_last)
+        return AG.WarpExFn.apply(xp, flow, interp, pad, align_corners)[:, :c].contiguous()
+    # fp32 mode (split-bf16 or FFMA) runs the fp32 NHWC kernel: a memory-bound gather that moves as many bytes as the
+    # split-bf16 [hi | lo] layout would, and is exact
+    dt = BF16 if current_dtype() == BF16 else F32
+    vec = 8 if dt == BF16 else 4
+    while nv * vec < c:                    # a power-of-two number of 16-byte vectors per pixel
+        nv *= 2
+    ca = nv * vec
+    xin, _ = _to_nhwc(x, dt, "m_in", ca)
+    out = ws("m_out", (n, h, w, ca), ops.TORCH_DT[dt], x.device)
+    ops.flow_warp_ex(xin, flow, out, n, h, w, ca, dt, interp, pad, align_corners)
     return _to_nchw(out, n, c, h, w, ca, dt)
 
 

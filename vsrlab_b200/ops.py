@@ -10,8 +10,8 @@ from typing import Optional, Sequence, Tuple
 import torch
 
 from . import _lib as L
-from ._lib import (ACT_LRELU, ACT_NONE, ACT_RELU, BF16, BF16X2, EPI_CLEAN, EPI_FLOW, EPI_NHWC, EPI_SR, F32, PAD_BORDER,
-                   PAD_ZEROS)
+from ._lib import (ACT_LRELU, ACT_NONE, ACT_RELU, BF16, BF16X2, EPI_CLEAN, EPI_FLOW, EPI_NHWC, EPI_SR, F32, INTERP_BILINEAR,
+                   PAD_BORDER, PAD_ZEROS)
 
 # BF16X2 = split-bf16 (fp32-accurate tensor-core mode): per pixel [hi C | lo C] bf16, value = hi + lo
 TORCH_DT = {BF16: torch.bfloat16, F32: torch.float32, BF16X2: torch.bfloat16}
@@ -201,6 +201,14 @@ def flow_warp(x, flow, out, n: int, h: int, w: int, c: int, dtype: int, padding:
                                         _stream()), "vsrb_flow_warp")
 
 
+def flow_warp_ex(x, flow, out, n: int, h: int, w: int, c: int, dtype: int, interp: int = INTERP_BILINEAR, padding: int = PAD_ZEROS,
+                 align_corners: bool = True, x_img_stride: int = 0, flow_img_stride: int = 0) -> None:
+    """flow_warp with any grid_sample mode (INTERP_*, PAD_* incl. reflection, align_corners)."""
+    with _Timed("flow_warp_ex", float(n) * h * w * (2 * c * ESIZE[dtype] + 8)):
+        L.check(L.load().vsrb_flow_warp_ex(_p(x), x_img_stride, _p(flow), flow_img_stride, _p(out), n, h, w, c, dtype, interp, padding,
+                                           int(bool(align_corners)), _stream()), "vsrb_flow_warp_ex")
+
+
 def flow_warp_groups(x, x_strides: Tuple[int, int], flow, flow_strides: Tuple[int, int], out, imgs_per_group: int, groups: int, h: int,
                      w: int, c: int, dtype: int, padding: int = PAD_ZEROS) -> None:
     """One launch for `groups` sets of images that read different bases (x / flow: raw addresses + (image, group) strides)."""
@@ -328,3 +336,10 @@ def flow_warp_bwd(x, flow, dout, dx, dflow, n: int, h: int, w: int, c: int, dtyp
     with _Timed("flow_warp_bwd", float(n) * h * w * (3 * c * ESIZE[dtype] + 4 * c * 4)):
         L.check(L.load().vsrb_flow_warp_bwd(_p(x), _p(flow), _p(dout), _p(dx), _p(dflow), n, h, w, c, dtype, padding, _stream()),
                 "vsrb_flow_warp_bwd")
+
+
+def flow_warp_ex_bwd(x, flow, dout, dx, dflow, n: int, h: int, w: int, c: int, dtype: int, interp: int = INTERP_BILINEAR,
+                     padding: int = PAD_ZEROS, align_corners: bool = True) -> None:
+    with _Timed("flow_warp_ex_bwd", float(n) * h * w * (3 * c * ESIZE[dtype] + 4 * c * 4)):
+        L.check(L.load().vsrb_flow_warp_ex_bwd(_p(x), _p(flow), _p(dout), _p(dx), _p(dflow), n, h, w, c, dtype, interp, padding,
+                                               int(bool(align_corners)), _stream()), "vsrb_flow_warp_ex_bwd")
