@@ -111,7 +111,9 @@ typedef struct vsrb_conv_args {
     float        slope;       /* LeakyReLU slope                                                 */
     int32_t      epilogue;    /* VSRB_EPI_*                                                      */
     void*        out;         /* EPI_NHWC: NHWC output (dtype); EPI_CLEAN: NHWC refreshed frame  */
-    int32_t      out_c;       /* channels allocated per pixel in `out`                           */
+    int32_t      out_c;       /* channels allocated per pixel in `out`.  EPI_NHWC: a multiple of 8
+                                 (of 16 with `split`).  EPI_CLEAN: 3..16, or exactly 32 with
+                                 `split`; `out` must be 16-byte aligned when out_c == 16 or split */
     int64_t      out_img_stride;   /* EPI_NHWC: elements between consecutive images of a group in
                                       `out` (0 = dense); lets a step write straight into frame t
                                       of a [N,T,h,w,C] feature bank                               */
@@ -125,7 +127,10 @@ typedef struct vsrb_conv_args {
     int32_t      max_ctas;    /* 0 = one persistent CTA per SM                                   */
     int32_t      flags;       /* VSRB_CONV_* bits                                                */
     int32_t      split;       /* 1: `out`, `residual` (and the EPI_CLEAN frame) are split-bf16: per pixel
-                                 [hi C | lo C] with C = out_c/2, value = hi + lo                  */
+                                 [hi C | lo C] with C = out_c/2, value = hi + lo.  The stores move
+                                 16 channels at a time, so out_c and res_c must be multiples of 16;
+                                 the EPI_CLEAN frame is [hi 16 | lo 16] (out_c = 32).  Anything
+                                 else returns VSRB_E_ARG                                          */
     /* Optional fast operand for a 3-channel 3x3 segment (the image stems 3 -> 64 and 64+3 -> 64: conv.py:97-98 behind
      * realbasicvsr.py:21 and basicvsr.py:56,71): the frames as 3x3 im2col patches, bf16 [.,h,w,32] written by
      * vsrb_im2col3x3_c3.  When given (and the launch is large enough) the ring-walk kernel multiplies the whole

@@ -84,3 +84,51 @@ def test_conv_plan_selection(lib):
         # stacked, N <= 256; a block's weights either stream (<= 128 KiB) or half of them stays resident per CTA of a pair
         assert info[0] == 1 and info[3] <= 256 and info[7] <= 200
     assert plan(7, [64], 32)[4] == 32 and plan(7, [32], 64)[4] == 32      # CTA-pair plans keep 64-byte K rows for 7x7
+
+
+# Split-bf16 stores move 16 channels (two 16-byte vectors) at channel c0 and at c0 + out_c/2, and the 16-channel EPI_CLEAN
+# store is two 16-byte vectors: vsrb_conv2d_fwd refuses every channel stride or alignment those stores cannot honour before
+# it touches the device.  Only refused configurations are called here, with placeholder addresses that are never read;
+# the accepted boundaries run on real tensors on the GPU: the EPI_CLEAN split shadow (out_c = 32) in
+# test_gpu_image_epilogues.py, EPI_NHWC split outputs and residuals (out_c = 32, 64, 128) in test_gpu_parity.py.
+E_ARG = -1
+FAKE = 1 << 20                                          # non-null, 16-byte aligned placeholder address
+
+
+def conv_args(epilogue, cout, out_c, split, out=FAKE, res_c=0):
+    from vsrlab_b200 import _lib
+    g = _lib.ConvGeom()
+    g.kh = g.kw = 3
+    g.n_seg = 1
+    g.seg_c[0] = 64
+    g.cout, g.groups, g.dtype = cout, 1, _lib.BF16
+    a = _lib.ConvArgs()
+    a.geom = g
+    a.inp[0], a.in_c[0] = FAKE, 64
+    a.batch, a.h, a.w, a.imgs_per_group = 1, 8, 8, 1
+    a.packed, a.epilogue, a.out, a.out_c, a.split = FAKE, epilogue, out, out_c, split
+    a.f32_io = FAKE
+    if res_c:
+        a.residual, a.res_c = FAKE, res_c
+    return a
+
+
+REFUSED = [
+    # (epilogue, cout, out_c, split, out offset in bytes, res_c, message fragment)
+    *[("clean", 3, oc, 1, 0, 0, b"out_c must be 32") for oc in (3, 8, 16, 17, 24, 31, 33, 48, 64)],
+    ("clean", 3, 32, 1, 2, 0, b"16-byte aligned"),
+    ("clean", 3, 32, 1, 8, 0, b"16-byte aligned"),
+    ("clean", 3, 16, 0, 2, 0, b"16-byte aligned"),
+    ("clean", 3, 16, 0, 8, 0, b"16-byte aligned"),
+    *[("nhwc", 16, oc, 1, 0, 0, b"multiples of 16") for oc in (40, 56, 72)],
+    ("nhwc", 16, 32, 1, 0, 40, b"multiples of 16"),
+    ("nhwc", 16, 64, 1, 0, 72, b"multiples of 16"),
+]
+
+
+@pytest.mark.parametrize("epi,cout,out_c,split,off,res_c,msg", REFUSED)
+def test_conv_refuses_unstorable_split_and_clean_layouts(lib, epi, cout, out_c, split, off, res_c, msg):
+    from vsrlab_b200 import _lib
+    a = conv_args({"clean": _lib.EPI_CLEAN, "nhwc": _lib.EPI_NHWC}[epi], cout, out_c, split, FAKE + off, res_c)
+    assert lib.vsrb_conv2d_fwd(C.byref(a), None) == E_ARG
+    assert msg in lib.vsrb_last_error()

@@ -444,10 +444,19 @@ int vsrb_conv2d_fwd(const vsrb_conv_args* a, void* stream) {
                            "EPI_NHWC: out_c %d too small", a->out_c);
             VSRB_CHECK_ARG(!a->residual || (!p.pixshuf && (a->split ? a->res_c / 2 : a->res_c) >= p.cout_pad), "bad residual");
             VSRB_CHECK_ARG(a->out_c % 8 == 0 && (!a->residual || a->res_c % 8 == 0), "channel strides must be %% 8");
+            // split stores and loads move 16 channels (two 16-byte vectors) at channel c0 and at c0 + out_c/2
+            VSRB_CHECK_ARG(!a->split || (a->out_c % 16 == 0 && (!a->residual || a->res_c % 16 == 0)),
+                           "EPI_NHWC split: out_c %d and res_c %d must be multiples of 16 (the lo half starts at C/2)", a->out_c,
+                           a->res_c);
             break;
         case VSRB_EPI_CLEAN:
-            VSRB_CHECK_ARG(p.cout == 3 && a->f32_io && a->out && a->out_c >= 3 && a->out_c <= (a->split ? 32 : 16) && !p.pixshuf,
-                           "EPI_CLEAN needs cout==3, f32_io, out with 3..16 channels");
+            VSRB_CHECK_ARG(p.cout == 3 && a->f32_io && a->out && !p.pixshuf, "EPI_CLEAN needs cout==3, f32_io, out");
+            // the split store writes the frame as [hi 16 | lo 16]: exactly 32 channels per pixel
+            if (a->split) VSRB_CHECK_ARG(a->out_c == 32, "EPI_CLEAN split: out_c must be 32 ([hi 16 | lo 16]), got %d", a->out_c);
+            else VSRB_CHECK_ARG(a->out_c >= 3 && a->out_c <= 16, "EPI_CLEAN needs out with 3..16 channels, got %d", a->out_c);
+            // 16-channel and split stores are 16-byte vectors
+            VSRB_CHECK_ARG((a->out_c != 16 && !a->split) || (reinterpret_cast<uintptr_t>(a->out) & 15) == 0,
+                           "EPI_CLEAN: out must be 16-byte aligned for a %d-channel store", a->out_c);
             break;
         case VSRB_EPI_FLOW:
             VSRB_CHECK_ARG(p.cout == 2 && a->f32_io && a->f32_in && !p.pixshuf, "EPI_FLOW needs cout==2, f32_io, f32_in");
