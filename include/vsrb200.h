@@ -177,10 +177,14 @@ int    vsrb_conv_plan_info(const vsrb_conv_geom* g, int32_t info[8]);
 
 /* ---- training (backward of the path; reference: autograd through the same modules) -------
  * input gradient of a conv: vsrb_conv2d_fwd on the output gradient with weights packed with
- * geom.transpose = 1.  Weight/bias gradient: dw [groups][cout][cin_total][kh][kw] and db
- * [groups][cout] (or NULL) are fp32, ACCUMULATED into (zero them first); `g` is the forward
- * geometry, in[]/in_c[] the forward inputs, dz the gradient wrt the conv output before the
- * activation, NHWC with dz_c channels per pixel.                                          */
+ * geom.transpose = 1.  Weight/bias gradient: dw [cout][cin_total][kh][kw] and db [cout] (or
+ * NULL) are fp32, ACCUMULATED into (zero them first); `g` is the forward geometry (groups = 1,
+ * imgs_per_group = batch), in[]/in_c[] the forward inputs, dz the gradient wrt the conv output
+ * before the activation, NHWC with dz_c >= cout channels per pixel.  in[] and dz 16-byte
+ * aligned, in_c[] and dz_c multiples of 8.  Kernels: bf16 3x3 segments of a multiple of 64
+ * channels (cout > 16) and bf16 odd square filters up to 7x7 on the tensor cores; fp32 data
+ * and bf16 non-square filters of width 1, 3 or 7 on the FFMA kernel.  Anything else is
+ * refused with VSRB_E_ARG before any work is enqueued.                                    */
 int vsrb_conv2d_wgrad(const vsrb_conv_geom* g, const void* const* in, const int32_t* in_c, const void* dz,
                       int32_t dz_c, int32_t batch, int32_t h, int32_t w, int32_t imgs_per_group,
                       int32_t cin_total, float* dw, float* db, void* stream);

@@ -132,3 +132,47 @@ def test_conv_refuses_unstorable_split_and_clean_layouts(lib, epi, cout, out_c, 
     a = conv_args({"clean": _lib.EPI_CLEAN, "nhwc": _lib.EPI_NHWC}[epi], cout, out_c, split, FAKE + off, res_c)
     assert lib.vsrb_conv2d_fwd(C.byref(a), None) == E_ARG
     assert msg in lib.vsrb_last_error()
+
+
+# vsrb_conv2d_wgrad refuses, before it touches the device, every call its kernels cannot honour: grouped weights, tensors
+# the 16-byte vector loads cannot read, channel strides that are not a multiple of 8, a dz with fewer channels than cout,
+# element types other than bf16 and fp32, and filters no kernel takes.  Placeholder addresses as above: only refused
+# calls are made.
+def wgrad_call(lib, kh=3, kw=3, segs=(64,), cout=64, dtype="bf16", groups=1, ipg=2, in_off=(0, 0), in_c=None, dz_off=0, dz_c=64):
+    from vsrlab_b200 import _lib
+    g = _lib.ConvGeom()
+    g.kh, g.kw, g.n_seg = kh, kw, len(segs)
+    off = 0
+    for i, c in enumerate(segs):
+        g.seg_off[i], g.seg_c[i] = off, c
+        off += c
+    g.cout, g.groups, g.dtype = cout, groups, {"bf16": _lib.BF16, "fp32": _lib.F32, "bf16x2": _lib.BF16X2}[dtype]
+    ins = (C.c_void_p * 2)(*[FAKE + (i + 1) * (1 << 16) + in_off[i] for i in range(2)])
+    cs = (C.c_int32 * 2)(*(in_c or (*segs, 0)[:2]))
+    return lib.vsrb_conv2d_wgrad(C.byref(g), ins, cs, C.c_void_p(FAKE + dz_off), dz_c, 2, 8, 8, ipg, off,
+                                 C.c_void_p(FAKE + (1 << 18)), None, None)
+
+
+WGRAD_REFUSED = {
+    "groups2": (dict(groups=2, ipg=1), b"grouped"),
+    "imgs_per_group": (dict(ipg=1), b"grouped"),
+    "in_unaligned": (dict(in_off=(2, 0)), b"16-byte aligned"),
+    "in1_unaligned": (dict(segs=(64, 64), in_off=(0, 8)), b"16-byte aligned"),
+    "dz_unaligned": (dict(dz_off=4), b"16-byte aligned"),
+    "in_c": (dict(segs=(60,), in_c=(60, 0)), b"multiple of 8"),
+    "dz_c": (dict(cout=60, dz_c=60), b"multiple of 8"),
+    "dz_c_below_cout": (dict(dz_c=56), b">= cout"),
+    "bf16_3x5": (dict(kw=5), b"no kernel for a 3x5"),
+    "bf16_1x5": (dict(kh=1, kw=5), b"no kernel for a 1x5"),
+    "fp32_5x5": (dict(kh=5, kw=5, dtype="fp32"), b"no kernel for a 5x5"),
+    "even_4x4": (dict(kh=4, kw=4), b"odd sizes"),
+    "9x9": (dict(kh=9, kw=9), b"odd sizes"),
+    "split_bf16": (dict(dtype="bf16x2"), b"bf16 or fp32"),
+}
+
+
+@pytest.mark.parametrize("case", list(WGRAD_REFUSED))
+def test_wgrad_refuses_before_launch(lib, case):
+    kw, msg = WGRAD_REFUSED[case]
+    assert wgrad_call(lib, **kw) == E_ARG
+    assert msg in lib.vsrb_last_error(), lib.vsrb_last_error()

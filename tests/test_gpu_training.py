@@ -100,9 +100,8 @@ TAPS_CASES = [
 
 @pytest.mark.parametrize("case", TAPS_CASES, ids=lambda c: "k%d_%d(%d)->%d_b%d_%dx%d" % c)
 def test_wgrad_taps_kernel(dev, case):
-    """csrc/wgrad_taps.cu (tap-stacking tcgen05 weight gradient) against fp64 torch on the same bf16 operands, and against the
-    mma.sync kernel it replaces (VSRB_WGRAD_MMA=1).  Padding channels of the activation tensors hold NaN: they must not leak."""
-    import os
+    """csrc/wgrad_taps.cu (tap-stacking tcgen05 weight gradient) against fp64 torch on the same bf16 operands.  Padding
+    channels of the activation tensors hold NaN: they must not leak."""
     from vsrlab_b200 import _lib as L
     from vsrlab_b200 import ops
     from vsrlab_b200._lib import BF16
@@ -122,26 +121,17 @@ def test_wgrad_taps_kernel(dev, case):
     geom.kh = geom.kw = K
     geom.n_seg, geom.cout, geom.pixshuf, geom.groups, geom.dtype, geom.transpose = 1, cout, 0, 1, BF16, 0
     geom.seg_off[0], geom.seg_c[0] = 0, cin
-    outs = {}
-    for mode in ("taps", "mma") if K != 5 else ("taps",):       # (the mma.sync kernel has no 5x5 instance)
-        if mode == "mma":
-            os.environ["VSRB_WGRAD_MMA"] = "1"
-        try:
-            dw = torch.zeros(cout, cin, K, K, dtype=torch.float32, device=dev)
-            db = torch.zeros(cout, dtype=torch.float32, device=dev)
-            ops.conv2d_wgrad(geom, [xp], [xc], zp, zc, B, h, w, cin, dw, db)
-            ops.conv2d_wgrad(geom, [xp], [xc], zp, zc, B, h, w, cin, dw, None)          # accumulates
-            torch.cuda.synchronize()
-        finally:
-            os.environ.pop("VSRB_WGRAD_MMA", None)
-        outs[mode] = dw.cpu() / 2
-        assert torch.isfinite(dw).all()
-        assert rel(db.cpu(), dz.sum((0, 2, 3))) < 1e-3
+    dw = torch.zeros(cout, cin, K, K, dtype=torch.float32, device=dev)
+    db = torch.zeros(cout, dtype=torch.float32, device=dev)
+    ops.conv2d_wgrad(geom, [xp], [xc], zp, zc, B, h, w, cin, dw, db)
+    ops.conv2d_wgrad(geom, [xp], [xc], zp, zc, B, h, w, cin, dw, None)          # accumulates
+    torch.cuda.synchronize()
+    got = dw.cpu() / 2
+    assert torch.isfinite(dw).all()
+    assert rel(db.cpu(), dz.sum((0, 2, 3))) < 1e-3
     scale = wr.grad.abs().max().item()
-    assert (outs["taps"].double() - wr.grad).abs().max().item() < 2e-3 * scale + 1e-4, (outs["taps"].double() - wr.grad).abs().max().item()
-    assert rel(outs["taps"], wr.grad.float()) < 1e-3
-    if "mma" in outs:
-        assert rel(outs["taps"], outs["mma"]) < 1e-3
+    assert (got.double() - wr.grad).abs().max().item() < 2e-3 * scale + 1e-4, (got.double() - wr.grad).abs().max().item()
+    assert rel(got, wr.grad.float()) < 1e-3
 
 
 @pytest.mark.parametrize("border,dtype", [(False, torch.bfloat16), (True, torch.float32)])
@@ -204,47 +194,63 @@ def test_realbasicvsr_training_step_gradients(dev, train_flow):
     assert rel(torch.cat(got), torch.cat(want)) < 0.1
 
 
-@pytest.mark.parametrize("case", [
-    # (segs, cout, k, h, w): shapes of the mma.sync weight-gradient kernel (7x7, 1x1, narrow segments, ragged widths)
-    ([(0, 8)], 32, 7, 13, 37),
-    ([(0, 32)], 64, 7, 9, 40),
-    ([(0, 64)], 32, 7, 12, 33),
-    ([(0, 16)], 2, 7, 6, 10),
-    ([(0, 64), (64, 64)], 64, 1, 10, 35),
-    ([(0, 3)], 64, 3, 11, 31),
-    ([(0, 64)], 3, 3, 11, 31),
-], ids=lambda c: f"k{c[2]}_{c[0]}_{c[1]}")
-def test_wgrad_mma_matches_ffma_and_fp32(dev, case, monkeypatch):
-    """dW / db of the warp-MMA kernel against the FFMA kernel on the same bf16 data (only the summation order differs)
-    and against fp32 autograd."""
+WGRAD_DISPATCH_CASES = [
+    # (dtype, segs, cout, (kh, kw), h, w)
+    # bf16 odd square filters: the tap-stacking kernel (7x7, 1x1, narrow segments, thin outputs, ragged widths)
+    ("bf16", [(0, 8)], 32, (7, 7), 13, 37),
+    ("bf16", [(0, 32)], 64, (7, 7), 9, 40),
+    ("bf16", [(0, 64)], 32, (7, 7), 12, 33),
+    ("bf16", [(0, 16)], 2, (7, 7), 6, 10),
+    ("bf16", [(0, 64), (64, 64)], 64, (1, 1), 10, 35),
+    ("bf16", [(0, 3)], 64, (3, 3), 11, 31),
+    ("bf16", [(0, 64)], 3, (3, 3), 11, 31),
+    # the FFMA kernel: bf16 non-square filters, fp32 data
+    ("bf16", [(0, 24)], 40, (1, 3), 11, 37),
+    ("bf16", [(0, 64)], 32, (3, 1), 9, 35),
+    ("bf16", [(0, 16)], 64, (1, 7), 10, 33),
+    ("bf16", [(0, 3), (3, 64)], 72, (3, 7), 7, 29),
+    ("fp32", [(0, 64), (64, 20)], 64, (1, 1), 10, 35),
+    ("fp32", [(0, 3)], 64, (3, 3), 11, 31),
+    ("fp32", [(0, 32)], 16, (7, 7), 9, 40),
+]
+
+
+@pytest.mark.parametrize("case", WGRAD_DISPATCH_CASES, ids=lambda c: f"{c[0]}_k{c[3][0]}x{c[3][1]}_{c[1]}_{c[2]}")
+def test_wgrad_dispatch_matches_fp64(dev, case):
+    """dW / db of the segments the 3x3 tensor-core kernel does not take - the tap-stacking kernel (bf16 odd square filters)
+    and the FFMA kernel (bf16 non-square filters, fp32 data) - against float64 conv2d_weight on the same operands.  Padding
+    channels of the activation and dz tensors hold NaN: they must not leak."""
+    from torch.nn.grad import conv2d_weight
     from vsrlab_b200 import autograd as AG, ops
-    segs, cout, k, h, w = case
+    from vsrlab_b200._lib import F32
+    dtype, segs, cout, (kh, kw), h, w = case
+    tdt = torch.bfloat16 if dtype == "bf16" else torch.float32
     g = torch.Generator().manual_seed(5)
     cin = sum(c for _, c in segs)
     B = 3
-    x = bf16r(torch.randn(B, cin, h, w, generator=g))
-    dz = bf16r(torch.randn(B, cout, h, w, generator=g))
-    cv = torch.nn.Conv2d(cin, cout, k, 1, k // 2)
-    geom = AG._wgrad_geom(cv, tuple(segs))
-    ins = [AG.to_cl16(x[:, off:off + c].to(dev)) for off, c in segs]
-    dzd = AG.to_cl16(dz.to(dev))
-    res = []
-    for ffma in ("", "1"):
-        if ffma:
-            monkeypatch.setenv("VSRB_WGRAD_FFMA", "1")
-        else:
-            monkeypatch.delenv("VSRB_WGRAD_FFMA", raising=False)
-        dw = torch.zeros(cout, cin, k, k, device=dev)
-        db = torch.zeros(cout, device=dev)
-        ops.conv2d_wgrad(geom, ins, [t.shape[1] for t in ins], dzd, dzd.shape[1], B, h, w, cin, dw, db)
-        torch.cuda.synchronize()
-        res.append((dw.cpu(), db.cpu()))
-    wr = torch.zeros(cout, cin, k, k, requires_grad=True)
-    (F.conv2d(x, wr, None, padding=k // 2) * dz).sum().backward()
-    scale = wr.grad.abs().max().item()
-    assert (res[0][0] - res[1][0]).abs().max().item() <= 1e-4 * scale
-    assert (res[0][0] - wr.grad).abs().max().item() <= 1e-4 * scale
-    assert (res[0][1] - dz.sum((0, 2, 3))).abs().max().item() <= 1e-3 * dz.sum((0, 2, 3)).abs().max().item()
+    x = torch.randn(B, cin, h, w, generator=g).to(tdt).float()
+    dz = torch.randn(B, cout, h, w, generator=g).to(tdt).float()
+    geom = AG._wgrad_geom(torch.nn.Conv2d(cin, cout, (kh, kw), 1, (kh // 2, kw // 2)), tuple(segs))
+    if dtype == "fp32":
+        geom.dtype = F32
+
+    def nhwc_nan(t):
+        c = t.shape[1]
+        c_alloc = (c + 15) // 16 * 16 + (16 if c % 16 == 0 else 0)
+        out = torch.full((B, c_alloc, h, w), float("nan"), dtype=tdt, device=dev).contiguous(memory_format=torch.channels_last)
+        out[:, :c] = t.to(dev)
+        return out
+    ins = [nhwc_nan(x[:, off:off + c]) for off, c in segs]
+    dzd = nhwc_nan(dz)
+    dw = torch.zeros(cout, cin, kh, kw, device=dev)
+    db = torch.zeros(cout, device=dev)
+    ops.conv2d_wgrad(geom, ins, [t.shape[1] for t in ins], dzd, dzd.shape[1], B, h, w, cin, dw, db)
+    torch.cuda.synchronize()
+    ref = conv2d_weight(x.double(), (cout, cin, kh, kw), dz.double(), padding=(kh // 2, kw // 2))
+    ref_b = dz.double().sum((0, 2, 3))
+    assert torch.isfinite(dw).all() and torch.isfinite(db).all()
+    assert (dw.cpu().double() - ref).abs().max().item() <= 1e-4 * ref.abs().max().item()
+    assert (db.cpu().double() - ref_b).abs().max().item() <= 1e-3 * ref_b.abs().max().item()
 
 
 def test_batched_wgrad_equals_per_use(dev):

@@ -1,6 +1,6 @@
 """Weight-gradient kernels on the shapes of the cfg4 training step: time per launch (CUDA events, L2 flushed between
-launches) of the tap-stacking tcgen05 kernel (csrc/wgrad_taps.cu) against the mma.sync kernel it replaces, with the
-VSRB_WG_DEBUG decomposition (1 = no final atomics, 2 = no MMAs, 4 = no loads).
+launches) of the kernel the library's dispatch picks (csrc/wgrad_taps.cu or csrc/wgrad_tc.cu), with the VSRB_WG_DEBUG
+decomposition (1 = no final atomics, 2 = no MMAs, 4 = no loads).
 
     python tools/wgrad_bench.py [--images 224]
 """
@@ -19,10 +19,13 @@ from vsrlab_b200._lib import BF16  # noqa: E402
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--images", type=int, default=224)
-    ap.add_argument("--modes", default="taps,mma,taps:1,taps:2,taps:3,taps:4", help="taps | mma | all (= every segment on the tap kernel), each optionally :<VSRB_WG_DEBUG bits>")
+    ap.add_argument("--modes", default="default,default:1,default:2,default:3,default:4",
+                    help="default (the library's dispatch), optionally :<VSRB_WG_DEBUG bits>")
     ap.add_argument("--sides", default="64,32,16")
     ap.add_argument("--shapes", default="", help="K,cin,x_channels,cout;... instead of the cfg4 list")
     a = ap.parse_args()
+    if any(m.partition(":")[0] != "default" for m in a.modes.split(",")):
+        ap.error(f"modes are default[:<VSRB_WG_DEBUG bits>], got {a.modes!r}")
     load()
     dev = torch.device("cuda:0")
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
@@ -44,14 +47,8 @@ def main():
             flops = 2.0 * B * side * side * cin * cout * K * K
             row = []
             for mode in a.modes.split(","):
-                name, _, dbg = mode.partition(":")
-                os.environ.pop("VSRB_WGRAD_MMA", None)
+                dbg = mode.partition(":")[2]
                 os.environ.pop("VSRB_WG_DEBUG", None)
-                os.environ.pop("VSRB_WGRAD_TAPS_ALL", None)
-                if name == "all":
-                    os.environ["VSRB_WGRAD_TAPS_ALL"] = "1"
-                if name == "mma":
-                    os.environ["VSRB_WGRAD_MMA"] = "1"
                 if dbg:
                     os.environ["VSRB_WG_DEBUG"] = dbg
                 ts = []
@@ -67,8 +64,7 @@ def main():
                 us = sorted(ts)[len(ts) // 2]
                 row.append(f"{mode} {us:7.1f} us ({flops / us / 1e6:6.1f} TF/s)")
             print(f"{K}x{K} {cin:3d}->{cout:3d} {B}x{side}x{side}: " + " | ".join(row), flush=True)
-    for k in ("VSRB_WGRAD_MMA", "VSRB_WG_DEBUG", "VSRB_WGRAD_TAPS_ALL"):
-        os.environ.pop(k, None)
+    os.environ.pop("VSRB_WG_DEBUG", None)
 
 
 if __name__ == "__main__":

@@ -2,13 +2,12 @@
 //
 //  * input gradient of a conv  = the forward conv kernel run on the output gradient with the weights packed
 //    transposed + flipped (vsrb_conv_geom.transpose = 1) - no new kernel;
-//  * weight / bias gradient     = conv_wgrad_kernel below: dW[co][ci][ky][kx] = sum_pixels dz[p][co] * x[p + tap][ci]
-//    (reference: autograd's ConvolutionBackward0 of every nn.Conv2d on the path);
+//  * weight / bias gradient     = dW[co][ci][ky][kx] = sum_pixels dz[p][co] * x[p + tap][ci] on the tcgen05 kernels of
+//    wgrad_tc.cu / wgrad_taps.cu, or the FFMA fallback conv_wgrad_kernel below (vsrb_conv2d_wgrad picks one per input
+//    segment; reference: autograd's ConvolutionBackward0 of every nn.Conv2d on the path);
 //  * flow_warp backward         = flow_warp_bwd_kernel: scatter of the output gradient through the four bilinear
 //    taps (grad wrt the warped features) and the derivative of the taps wrt the sample position (grad wrt the
 //    flow, needed when train_flow=True) - reference: GridSampler2DBackward0 behind spynet.py:95-106.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "warp_modes.cuh"
 
@@ -30,47 +29,40 @@ template <> struct Ld8<float> {
 };
 
 // ---------------------------------------------------------------------------------------
-// weight gradient (FFMA fallback for the shapes the tensor-core kernel does not take: 7x7, 1x1, 3-channel
-// segments).  One CTA = one filter ROW ky x one 64(co) x 64(ci) tile x a run of 32-pixel row chunks.  Per chunk it
-// stages dz [32 px][64 co] and ONE extended activation strip [32 + kw - 1 px][64 ci] of image row y + ky - pad, and
-// updates the kw taps of the row from it (kw x 4x4 fp32 accumulators per thread), so dz is read kh times instead
-// of kh*kw times.  Results are added to the OIHW fp32 gradient with atomics.
+// weight gradient (FFMA fallback for the segments neither tcgen05 kernel takes: fp32 data, bf16 non-square filters).
+// One CTA = one filter ROW ky x one 64(co) x 64(ci) tile x a run of 32-pixel row chunks.  Per chunk it stages dz
+// [32 px][64 co] and ONE extended activation strip [32 + kw - 1 px][64 ci] of image row y + ky - pad, and updates the kw
+// taps of the row from it (kw x 4x4 fp32 accumulators per thread), so dz is read kh times instead of kh*kw times.
+// Results are added to the OIHW fp32 gradient with atomics.
 // ---------------------------------------------------------------------------------------
 struct WgradParams {
     const void* in[2];
     int in_c[2], seg_c[2], seg_off[2];
-    int n_seg;
     const void* dz;
     int dz_c;
-    int kh, kw, H, W, imgs_per_group, groups;
+    int kh, kw, H, W;
     int cout, cin_total;
-    int chunks_per_row, units_g, units_per_cta;   // unit = (image of the group, row y, 32-pixel chunk)
+    int chunks_per_row, units, units_per_cta;     // unit = (image, row y, 32-pixel chunk)
     int n_co_blk, n_ci_blk;                       // 64-wide blocks
     int ci_blk_seg[8], ci_blk_c0[8];
     float* dw;
 };
 
-// CO_T x CI_T = the (co, ci) tile of one CTA (16, 32 or 64 each).  A thread owns a 4x4 patch of it; the 256 threads
-// form 256 / (CO_T/4 * CI_T/4) pixel groups that split the 32 pixels of a chunk between them, so narrow layers
-// (SPyNet's 8->32, 32->16, 16->2 ...) do not pay for a full 64x64 tile.
-template <typename T, int KW, int CO_T, int CI_T>
+// A thread owns a 4x4 (co, ci) patch of the 64 x 64 tile; the 256 threads are one pixel group walking the 32 pixels of a
+// chunk.
+template <typename T, int KW>
 __global__ void __launch_bounds__(256) conv_wgrad_kernel(WgradParams P) {
-    constexpr int TY = CO_T / 4, TX = CI_T / 4, TPG = TY * TX, PG = 256 / TPG;
-    __shared__ __align__(16) float zs[32][CO_T];
-    __shared__ __align__(16) float xs[32 + KW - 1][CI_T];
+    __shared__ __align__(16) float zs[32][64];
+    __shared__ __align__(16) float xs[32 + KW - 1][64];
     const int tid = threadIdx.x;
-    const int pg = tid / TPG, rr = tid % TPG;
-    const int tx = rr % TX, ty = rr / TX;               // 4 ci per tx, 4 co per ty
+    const int tx = tid % 16, ty = tid / 16;             // 4 ci per tx, 4 co per ty
     const int ky = blockIdx.y;
-    int z = blockIdx.z;
-    const int cib = z % P.n_ci_blk; z /= P.n_ci_blk;
-    const int cob = z % P.n_co_blk;
-    const int g = z / P.n_co_blk;
+    const int cib = blockIdx.z % P.n_ci_blk, cob = blockIdx.z / P.n_ci_blk;
     const int s = P.ci_blk_seg[cib], c0 = P.ci_blk_c0[cib];
-    const int co0 = cob * CO_T;
+    const int co0 = cob * 64;
     const int hw = P.H * P.W;
     const int u_begin = blockIdx.x * P.units_per_cta;
-    const int u_end = min(u_begin + P.units_per_cta, P.units_g);
+    const int u_end = min(u_begin + P.units_per_cta, P.units);
     const T* zin = reinterpret_cast<const T*>(P.dz);
     const T* xin = reinterpret_cast<const T*>(P.in[s]);
     const int dy = ky - P.kh / 2, pad = KW / 2;
@@ -87,12 +79,12 @@ __global__ void __launch_bounds__(256) conv_wgrad_kernel(WgradParams P) {
         const int xc = u % P.chunks_per_row;
         const int rowi = u / P.chunks_per_row;
         const int y = rowi % P.H;
-        const long long img = (long long)g * P.imgs_per_group + rowi / P.H;
+        const long long img = rowi / P.H;
         const int x0 = xc * 32;
         const int yy = y + dy;
         __syncthreads();
-        for (int i = tid; i < 32 * (CO_T / 8); i += 256) {          // dz chunk [32 px][CO_T]
-            const int lp = i / (CO_T / 8), lc = (i % (CO_T / 8)) * 8;
+        for (int i = tid; i < 32 * 8; i += 256) {           // dz chunk [32 px][64 co]
+            const int lp = i / 8, lc = (i % 8) * 8;
             float zv[8];
 #pragma unroll
             for (int e = 0; e < 8; ++e) zv[e] = 0.f;
@@ -105,8 +97,8 @@ __global__ void __launch_bounds__(256) conv_wgrad_kernel(WgradParams P) {
             *reinterpret_cast<float4*>(&zs[lp][lc]) = make_float4(zv[0], zv[1], zv[2], zv[3]);
             *reinterpret_cast<float4*>(&zs[lp][lc + 4]) = make_float4(zv[4], zv[5], zv[6], zv[7]);
         }
-        for (int i = tid; i < (32 + KW - 1) * (CI_T / 8); i += 256) {   // extended strip: image columns x0 - pad + e
-            const int ep = i / (CI_T / 8), lc = (i % (CI_T / 8)) * 8;
+        for (int i = tid; i < (32 + KW - 1) * 8; i += 256) {   // extended strip: image columns x0 - pad + e
+            const int ep = i / 8, lc = (i % 8) * 8;
             float xv[8];
 #pragma unroll
             for (int e = 0; e < 8; ++e) xv[e] = 0.f;
@@ -122,7 +114,7 @@ __global__ void __launch_bounds__(256) conv_wgrad_kernel(WgradParams P) {
         }
         __syncthreads();
 #pragma unroll 2
-        for (int q = pg; q < 32; q += PG) {
+        for (int q = 0; q < 32; ++q) {
             const float4 a = *reinterpret_cast<const float4*>(&zs[q][ty * 4]);
             const float av[4] = {a.x, a.y, a.z, a.w};
 #pragma unroll
@@ -147,179 +139,9 @@ __global__ void __launch_bounds__(256) conv_wgrad_kernel(WgradParams P) {
             for (int j = 0; j < 4; ++j) {
                 const int ci = c0 + tx * 4 + j;
                 if (ci < P.seg_c[s])
-                    atomicAdd(P.dw + (((size_t)g * P.cout + co) * P.cin_total + P.seg_off[s] + ci) * taps + ky * KW + k, acc[k][i][j]);
+                    atomicAdd(P.dw + ((size_t)co * P.cin_total + P.seg_off[s] + ci) * taps + ky * KW + k, acc[k][i][j]);
             }
         }
-}
-
-// ---------------------------------------------------------------------------------------
-// bf16 weight gradient on the warp-level tensor-core path (mma.sync m16n8k16) for the shapes wgrad_tc_kernel does not
-// take (SPyNet's 7x7 layers, 1x1, 3-channel segments).  Same decomposition as conv_wgrad_kernel - one filter row ky and
-// one CO_T x CI_T tile per CTA, 32-pixel row chunks - but the chunk is staged as bf16 and each filter column kx is the
-// GEMM  D_kx[co][ci] += sum_q dz[q][co] * x[q + kx][ci]  (K = 32 pixels = two k16 steps).  Both operands sit pixel-major
-// in shared memory, i.e. transposed for the MMA, and are fetched with ldmatrix.trans; the kx shift is just a row offset
-// of the B fetch, so dz fragments are loaded once per k-step and reused by all kw columns.  (tcgen05 needs the pixel
-// shift in whole swizzle atoms - wgrad_tc.cu pays three halo copies for kw = 3; seven would not fit.)
-// Rows are padded by 16 bytes so the eight 16-byte rows of an ldmatrix land in different banks.
-// ---------------------------------------------------------------------------------------
-__device__ __forceinline__ void ldsm_x4_t(uint32_t addr, uint32_t (&r)[4]) {
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
-                 : "r"(addr));
-}
-__device__ __forceinline__ void mma_bf16_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-                 : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-// keeps the first `valid` (0..8) bf16 of a 16-byte vector, zeroes the rest
-__device__ __forceinline__ uint4 keep_bf16(uint4 u, int valid) {
-    uint32_t w[4] = {u.x, u.y, u.z, u.w};
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const int left = valid - 2 * i;
-        w[i] = left >= 2 ? w[i] : (left == 1 ? (w[i] & 0xFFFFu) : 0u);
-    }
-    return make_uint4(w[0], w[1], w[2], w[3]);
-}
-
-static constexpr int kMmaPx = 64;      // pixels of a chunk: four k16 steps amortise the per-chunk address math and barriers
-
-template <int KW, int CO_T, int CI_T>
-__global__ void __launch_bounds__(256) conv_wgrad_mma_kernel(WgradParams P) {
-    constexpr int PX = kMmaPx, NKS = PX / 16;
-    constexpr int ZP = CO_T * 2 + 16, XP = CI_T * 2 + 16;             // padded row pitch in bytes
-    constexpr int WT = (CO_T / 16) * (CI_T / 16);                     // 16 x 16 warp tiles of the CTA tile
-    constexpr int TPW = WT >= 8 ? WT / 8 : 1;                         // tiles per warp
-    constexpr int KS = WT >= 8 ? 1 : (8 / WT > NKS ? NKS : 8 / WT);   // warps sharing a tile split the k16 steps
-    __shared__ __align__(16) uint8_t zs[PX * ZP];
-    __shared__ __align__(16) uint8_t xs[(PX + KW - 1) * XP];
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int ky = blockIdx.y;
-    int z = blockIdx.z;
-    const int cib = z % P.n_ci_blk; z /= P.n_ci_blk;
-    const int cob = z % P.n_co_blk;
-    const int g = z / P.n_co_blk;
-    const int s = P.ci_blk_seg[cib], c0 = P.ci_blk_c0[cib];
-    const int co0 = cob * CO_T;
-    const int hw = P.H * P.W;
-    const int u_begin = blockIdx.x * P.units_per_cta;
-    const int u_end = min(u_begin + P.units_per_cta, P.units_g);
-    const __nv_bfloat16* zin = reinterpret_cast<const __nv_bfloat16*>(P.dz);
-    const __nv_bfloat16* xin = reinterpret_cast<const __nv_bfloat16*>(P.in[s]);
-    const int dy = ky - P.kh / 2, pad = KW / 2;
-
-    // this warp's tiles and k-steps
-    const int t_first = WT >= 8 ? warp * TPW : warp % WT;
-    const int ks_own = WT >= 8 ? -1 : warp / WT;                       // -1: all k16 steps; else steps ks_own, ks_own + KS, ...
-    const bool active = WT >= 8 || ks_own < KS;
-    float acc[TPW][KW][2][4];
-#pragma unroll
-    for (int t = 0; t < TPW; ++t)
-#pragma unroll
-        for (int k = 0; k < KW; ++k)
-#pragma unroll
-            for (int n = 0; n < 2; ++n)
-#pragma unroll
-                for (int i = 0; i < 4; ++i) acc[t][k][n][i] = 0.f;
-    const uint32_t zs0 = (uint32_t)__cvta_generic_to_shared(zs), xs0 = (uint32_t)__cvta_generic_to_shared(xs);
-    const int lj = lane >> 3, lr = lane & 7;                            // ldmatrix: matrix index and row of this lane's address
-
-    // Register double buffering: the next chunk's 16-byte global loads are issued before the current chunk's MMAs and only
-    // written to shared memory after them, so the global-memory latency hides behind the tensor-core work.
-    constexpr int ZI = PX * (CO_T / 8), XI = (PX + KW - 1) * (CI_T / 8);   // 16-byte items per chunk
-    constexpr int ZJ = (ZI + 255) / 256, XJ = (XI + 255) / 256;
-    uint4 zr[ZJ], xr[XJ];
-    auto fetch = [&](int u) {
-        const int xc = u % P.chunks_per_row;
-        const int rowi = u / P.chunks_per_row;
-        const int y = rowi % P.H;
-        const long long img = (long long)g * P.imgs_per_group + rowi / P.H;
-        const int x0 = xc * PX;
-        const int yy = y + dy;
-#pragma unroll
-        for (int j = 0; j < ZJ; ++j) {                              // dz chunk [PX px][CO_T] bf16
-            const int i = tid + j * 256;
-            zr[j] = make_uint4(0u, 0u, 0u, 0u);
-            if (i < ZI) {
-                const int lp = i / (CO_T / 8), lc = (i % (CO_T / 8)) * 8;
-                if (x0 + lp < P.W && co0 + lc < P.dz_c) {
-                    zr[j] = __ldg(reinterpret_cast<const uint4*>(zin + (img * hw + (long long)y * P.W + x0 + lp) * P.dz_c + co0 + lc));
-                    zr[j] = keep_bf16(zr[j], P.cout - (co0 + lc));
-                }
-            }
-        }
-#pragma unroll
-        for (int j = 0; j < XJ; ++j) {                              // extended strip: image columns x0 - pad + e
-            const int i = tid + j * 256;
-            xr[j] = make_uint4(0u, 0u, 0u, 0u);
-            if (i < XI) {
-                const int ep = i / (CI_T / 8), lc = (i % (CI_T / 8)) * 8;
-                const int xx = x0 - pad + ep;
-                if (yy >= 0 && yy < P.H && xx >= 0 && xx < P.W && c0 + lc < P.in_c[s]) {
-                    xr[j] = __ldg(reinterpret_cast<const uint4*>(xin + (img * hw + (long long)yy * P.W + xx) * P.in_c[s] + c0 + lc));
-                    xr[j] = keep_bf16(xr[j], P.seg_c[s] - (c0 + lc));
-                }
-            }
-        }
-    };
-    if (u_begin < u_end) fetch(u_begin);
-    for (int u = u_begin; u < u_end; ++u) {
-        __syncthreads();                                            // the previous chunk's fragments have been read
-#pragma unroll
-        for (int j = 0; j < ZJ; ++j) {
-            const int i = tid + j * 256;
-            if (i < ZI) *reinterpret_cast<uint4*>(zs + (i / (CO_T / 8)) * ZP + (i % (CO_T / 8)) * 16) = zr[j];
-        }
-#pragma unroll
-        for (int j = 0; j < XJ; ++j) {
-            const int i = tid + j * 256;
-            if (i < XI) *reinterpret_cast<uint4*>(xs + (i / (CI_T / 8)) * XP + (i % (CI_T / 8)) * 16) = xr[j];
-        }
-        __syncthreads();
-        if (u + 1 < u_end) fetch(u + 1);
-        if (active) {
-#pragma unroll
-            for (int ks = 0; ks < NKS; ++ks) {
-                if (ks_own >= 0 && (ks % KS) != ks_own) continue;
-                const int q0 = ks * 16;
-#pragma unroll
-                for (int t = 0; t < TPW; ++t) {
-                    const int tile = t_first + t;
-                    const int co_off = (tile / (CI_T / 16)) * 16, ci_off = (tile % (CI_T / 16)) * 16;
-                    uint32_t a[4];
-                    ldsm_x4_t(zs0 + (uint32_t)((q0 + (lj >> 1) * 8 + lr) * ZP + (co_off + (lj & 1) * 8) * 2), a);
-#pragma unroll
-                    for (int k = 0; k < KW; ++k) {
-                        uint32_t b[4];
-                        ldsm_x4_t(xs0 + (uint32_t)((q0 + k + (lj & 1) * 8 + lr) * XP + (ci_off + (lj >> 1) * 8) * 2), b);
-                        mma_bf16_16816(acc[t][k][0], a, b[0], b[1]);
-                        mma_bf16_16816(acc[t][k][1], a, b[2], b[3]);
-                    }
-                }
-            }
-        }
-    }
-    if (!active) return;
-    const int taps = P.kh * KW;
-    const int gq = lane >> 2, tq = lane & 3;
-#pragma unroll
-    for (int t = 0; t < TPW; ++t) {
-        const int tile = t_first + t;
-        const int co_off = (tile / (CI_T / 16)) * 16, ci_off = (tile % (CI_T / 16)) * 16;
-#pragma unroll
-        for (int k = 0; k < KW; ++k)
-#pragma unroll
-            for (int n = 0; n < 2; ++n)
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const int co = co0 + co_off + gq + (i >> 1) * 8;
-                    const int ci = c0 + ci_off + n * 8 + tq * 2 + (i & 1);
-                    if (co < P.cout && ci < P.seg_c[s])
-                        atomicAdd(P.dw + (((size_t)g * P.cout + co) * P.cin_total + P.seg_off[s] + ci) * taps + ky * KW + k,
-                                  acc[t][k][n][i]);
-                }
-    }
 }
 
 // ---------------------------------------------------------------------------------------
@@ -618,15 +440,38 @@ static void launch_warp_ex_bwd(const T* x, const float2* flow, const T* dout, fl
     else launch_warp_ex_bwd_t<T, VSRB_INTERP_BILINEAR>(x, flow, dout, dx, dflow, n, h, w, c, pad, align, s);
 }
 
-int launch_wgrad_tc(const void* x, int x_c, int c0, int ci_off, const void* dz, int dz_c, int batch, int h, int w, int cout,
-                    int cin_total, float* dw, cudaStream_t stream, float* db = nullptr);
 int launch_bias_grad(const void* dz, int dz_c, long long pixels, int cout, int dtype, float* db, cudaStream_t s);
-int launch_bias_grad_multi(const void* const* dzs, int n_chunks, int dz_c, long long pixels, int cout, int dtype, float* db,
-                           cudaStream_t s);
 int launch_wgrad_tc_multi(const void* const* xs, int x_c, int c0, int ci_off, const void* const* dzs, int dz_c, int n_chunks,
-                          int batch, int h, int w, int cout, int cin_total, float* dw, cudaStream_t stream, float* db = nullptr);
+                          int batch, int h, int w, int cout, int cin_total, float* dw, cudaStream_t stream, float* db);
 int launch_wgrad_taps(const void* x, int x_c, int x_c0, int ci_n, int ci_off, const void* dz, int dz_c, int z_c0, int co_n, int K,
                       int batch, int h, int w, int cin_total, float* dw, cudaStream_t stream);
+
+// The kernel that computes the weight gradient of input segment s.  3x3 layers whose segment has a multiple of 64 channels
+// (the resblock, upsampling and HR convs: > 85 % of the FLOPs) run on wgrad_tc_kernel - except thin outputs: the 64 -> 3
+// image convs would zero-fill 61 of its 64 dz columns.  Every other bf16 segment of an odd square filter up to 7x7
+// (SPyNet's 7x7 stacks, 3-channel image segments, 1x1, thin outputs) runs on the tap-stacking kernel of wgrad_taps.cu,
+// and the rest (fp32 data, non-square filters) on the FFMA kernel conv_wgrad_kernel.
+enum WgradPath { kWgradTc, kWgradTaps, kWgradFfma };
+static WgradPath wgrad_path(const vsrb_conv_geom* g, int s) {
+    if (g->dtype != VSRB_BF16) return kWgradFfma;
+    if (g->kh == 3 && g->kw == 3 && g->seg_c[s] % 64 == 0 && g->cout > 16) return kWgradTc;
+    if (g->kh == g->kw && (g->kw & 1) && g->kw <= 7) return kWgradTaps;
+    return kWgradFfma;
+}
+
+// Every 64-channel block of input segment s on wgrad_tc_kernel, summed over n_chunks (x, dz) pairs.  The bias gradient
+// rides on the first launch if *db is set (the kernel's idle epilogue warps add up the dz tiles it streams anyway); *db is
+// then cleared.
+static int wgrad_tc_segment(const vsrb_conv_geom* g, int s, const void* const* xs, int x_c, const void* const* dzs, int dz_c,
+                            int n_chunks, int batch, int h, int w, int cin_total, float* dw, float** db, cudaStream_t st) {
+    for (int c0 = 0; c0 < g->seg_c[s]; c0 += 64) {
+        int rc = launch_wgrad_tc_multi(xs, x_c, c0, g->seg_off[s] + c0, dzs, dz_c, n_chunks, batch, h, w, g->cout, cin_total, dw, st,
+                                       *db);
+        if (rc != VSRB_OK) return rc;
+        *db = nullptr;
+    }
+    return VSRB_OK;
+}
 
 }  // namespace vsrb
 
@@ -644,27 +489,15 @@ int vsrb_conv2d_wgrad_multi(const vsrb_conv_geom* g, int32_t n_chunks, const voi
     for (int s = 0; s < g->n_seg; ++s)
         VSRB_CHECK_ARG(g->seg_c[s] % 64 == 0 && in_c[s] % 8 == 0 && in_c[s] >= g->seg_c[s] && g->seg_off[s] + g->seg_c[s] <= cin_total,
                        "wgrad_multi: segment %d must have a multiple of 64 channels", s);
-    cudaStream_t st = (cudaStream_t)stream;
-    // the bias gradient rides along with the first input-channel block of every group of chunks (the kernel's idle epilogue
-    // warps add up the dz tiles it streams anyway); VSRB_WGRAD_SEPARATE_BIAS=1 keeps the separate reduction kernel
-    const bool fuse_bias = db && !getenv("VSRB_WGRAD_SEPARATE_BIAS");
     for (int k0 = 0; k0 < n_chunks; k0 += 16) {
         const int nk = n_chunks - k0 < 16 ? n_chunks - k0 : 16;
-        bool first = true;
+        float* bias = db;                                   // once per group of chunks
         for (int s = 0; s < g->n_seg; ++s) {
             const void* xs[16];
             for (int k = 0; k < nk; ++k) xs[k] = in[(size_t)(k0 + k) * g->n_seg + s];
-            for (int c0 = 0; c0 < g->seg_c[s]; c0 += 64) {
-                int rc = launch_wgrad_tc_multi(xs, in_c[s], c0, g->seg_off[s] + c0, dz + k0, dz_c, nk, batch, h, w, g->cout, cin_total, dw, st,
-                                               (fuse_bias && first) ? db : nullptr);
-                if (rc != VSRB_OK) return rc;
-                first = false;
-            }
+            int rc = wgrad_tc_segment(g, s, xs, in_c[s], dz + k0, dz_c, nk, batch, h, w, cin_total, dw, &bias, (cudaStream_t)stream);
+            if (rc != VSRB_OK) return rc;
         }
-    }
-    if (db && !fuse_bias) {
-        int rc = launch_bias_grad_multi(dz, n_chunks, dz_c, (long long)batch * h * w, g->cout, g->dtype, db, st);
-        if (rc != VSRB_OK) return rc;
     }
     return VSRB_OK;
 }
@@ -675,127 +508,75 @@ int vsrb_conv2d_wgrad(const vsrb_conv_geom* g, const void* const* in, const int3
     VSRB_CHECK_ARG(g && in && in_c && dz && dw, "wgrad: null argument");
     VSRB_CHECK_ARG(g->n_seg == 1 || g->n_seg == 2, "wgrad: n_seg must be 1 or 2");
     VSRB_CHECK_ARG(!g->pixshuf && !g->transpose, "wgrad: pass the plain forward geometry (un-shuffle the gradient first)");
-    VSRB_CHECK_ARG(imgs_per_group >= 1 && imgs_per_group * g->groups == batch, "wgrad: batch/groups mismatch");
-    VSRB_CHECK_ARG((long long)imgs_per_group * h * w < (1LL << 31), "wgrad: too many pixels per group");
-    const int vec = g->dtype == VSRB_BF16 ? 8 : 8;
-    VSRB_CHECK_ARG(dz_c % vec == 0, "wgrad: dz channel stride must be a multiple of 8");
+    VSRB_CHECK_ARG(g->groups == 1 && imgs_per_group == batch, "wgrad: grouped weight gradients are not supported (groups %d, "
+                   "imgs_per_group %d, batch %d): call once per group", g->groups, imgs_per_group, batch);
+    VSRB_CHECK_ARG(batch >= 1 && h >= 1 && w >= 1 && (long long)batch * h * w < (1LL << 31), "wgrad: 1 .. 2^31 - 1 pixels");
+    VSRB_CHECK_ARG(g->dtype == VSRB_BF16 || g->dtype == VSRB_F32, "wgrad: dtype must be bf16 or fp32");
+    VSRB_CHECK_ARG(g->kh >= 1 && g->kh <= 7 && (g->kh & 1) && g->kw >= 1 && g->kw <= 7 && (g->kw & 1),
+                   "wgrad: kernel %dx%d unsupported (odd sizes 1..7)", g->kh, g->kw);
+    VSRB_CHECK_ARG(dz_c % 8 == 0 && dz_c >= g->cout, "wgrad: dz channel stride %d must be a multiple of 8 and >= cout %d", dz_c,
+                   g->cout);
+    VSRB_CHECK_ARG((reinterpret_cast<uintptr_t>(dz) & 15) == 0, "wgrad: dz must be 16-byte aligned");
     WgradParams P;
     memset(&P, 0, sizeof(P));
-    P.n_seg = g->n_seg;
-    P.n_ci_blk = 0;
-    // 3x3 layers whose segment has a multiple of 64 channels (the resblock, upsampling and HR convs: > 85 % of
-    // the FLOPs; a cout below 64 is zero-filled by the TMA box) run on the tensor cores; everything else on the
-    // FFMA kernel
-    const bool tc_ok = g->dtype == VSRB_BF16 && g->kh == 3 && g->kw == 3 && g->groups == 1 && dz_c >= g->cout &&
-                       (reinterpret_cast<uintptr_t>(dz) & 15) == 0 && !getenv("VSRB_WGRAD_SIMT");
-    // ... except that every other bf16 segment of an odd square filter up to 7x7 (SPyNet's 7x7 stacks, 3-channel image
-    // segments, 1x1) takes the tap-stacking tcgen05 kernel of wgrad_taps.cu; VSRB_WGRAD_MMA=1 keeps the mma.sync kernel
-    const bool taps_ok = g->dtype == VSRB_BF16 && g->kh == g->kw && (g->kw & 1) && g->kw <= 7 && g->groups == 1 && dz_c % 8 == 0 &&
-                         (reinterpret_cast<uintptr_t>(dz) & 15) == 0 && !getenv("VSRB_WGRAD_SIMT") && !getenv("VSRB_WGRAD_FFMA") &&
-                         !getenv("VSRB_WGRAD_MMA");
-    bool on_tc[4] = {false, false, false, false};
-    bool db_done = false;
-    // (co, ci) tile of the mma.sync kernel: as narrow as its segments allow (the FFMA kernels keep 64 x 64)
-    int co_t = 64, ci_t = 64, cmax = 0;
     for (int s = 0; s < g->n_seg; ++s) {
-        // (a thin output - the 64 -> 3 image convs - would zero-fill 61 of wgrad_tc's 64 dz columns: the tap kernel takes dz as
-        // its narrow operand instead; VSRB_WGRAD_TAPS_ALL=1 sends every segment there, for A/B measurements)
-        on_tc[s] = tc_ok && g->seg_c[s] % 64 == 0 && (reinterpret_cast<uintptr_t>(in[s]) & 15) == 0 &&
-                   !(taps_ok && (g->cout <= 16 || getenv("VSRB_WGRAD_TAPS_ALL")));
-        if (!on_tc[s] && g->seg_c[s] > cmax) cmax = g->seg_c[s];
-    }
-    if (g->dtype == VSRB_BF16 && !getenv("VSRB_WGRAD_FFMA")) {
-        co_t = g->cout <= 16 ? 16 : (g->cout <= 32 ? 32 : 64);
-        ci_t = cmax <= 16 ? 16 : (cmax <= 32 ? 32 : 64);
-    }
-    for (int s = 0; s < g->n_seg; ++s) {
-        VSRB_CHECK_ARG(in[s] && in_c[s] % 8 == 0 && in_c[s] >= g->seg_c[s], "wgrad: bad input segment %d", s);
+        VSRB_CHECK_ARG(in[s] && (reinterpret_cast<uintptr_t>(in[s]) & 15) == 0, "wgrad: input segment %d must be 16-byte aligned", s);
+        VSRB_CHECK_ARG(in_c[s] % 8 == 0 && in_c[s] >= g->seg_c[s],
+                       "wgrad: input segment %d: channel stride %d must be a multiple of 8 and >= its %d channels", s, in_c[s], g->seg_c[s]);
         VSRB_CHECK_ARG(g->seg_off[s] + g->seg_c[s] <= cin_total, "wgrad: segment %d exceeds cin_total", s);
         P.in[s] = in[s]; P.in_c[s] = in_c[s]; P.seg_c[s] = g->seg_c[s]; P.seg_off[s] = g->seg_off[s];
-        if (on_tc[s]) {
-            for (int c0 = 0; c0 < g->seg_c[s]; c0 += 64) {
-                const bool ride = db && !db_done && !getenv("VSRB_WGRAD_SEPARATE_BIAS");      // bias gradient from the same pass over dz
-                int rc = launch_wgrad_tc(in[s], in_c[s], c0, g->seg_off[s] + c0, dz, dz_c, batch, h, w, g->cout, cin_total, dw,
-                                         (cudaStream_t)stream, ride ? db : nullptr);
-                if (rc != VSRB_OK) return rc;
-                db_done = db_done || ride;
-            }
-            continue;
-        }
-        if (taps_ok && (reinterpret_cast<uintptr_t>(in[s]) & 15) == 0) {
-            for (int c0 = 0; c0 < g->seg_c[s]; c0 += 64)
-                for (int n0 = 0; n0 < g->cout; n0 += 64) {
-                    const int ci_n = g->seg_c[s] - c0 < 64 ? g->seg_c[s] - c0 : 64, co_n = g->cout - n0 < 64 ? g->cout - n0 : 64;
-                    int rc = launch_wgrad_taps(in[s], in_c[s], c0, ci_n, g->seg_off[s] + c0, dz, dz_c, n0, co_n, g->kw, batch, h, w, cin_total,
-                                               dw, (cudaStream_t)stream);
-                    if (rc != VSRB_OK) return rc;
-                }
-            continue;
-        }
-        for (int c0 = 0; c0 < g->seg_c[s]; c0 += ci_t) {
-            VSRB_CHECK_ARG(P.n_ci_blk < 8, "wgrad: too many input-channel blocks");
+        if (wgrad_path(g, s) != kWgradFfma) continue;
+        VSRB_CHECK_ARG(g->kw == 1 || g->kw == 3 || g->kw == 7, "wgrad: no kernel for a %dx%d %s filter (the FFMA fallback takes "
+                       "widths 1, 3 and 7)", g->kh, g->kw, g->dtype == VSRB_BF16 ? "bf16" : "fp32");
+        for (int c0 = 0; c0 < g->seg_c[s]; c0 += 64) {
+            VSRB_CHECK_ARG(P.n_ci_blk < 8, "wgrad: more than 512 input channels on the FFMA fallback");
             P.ci_blk_seg[P.n_ci_blk] = s;
             P.ci_blk_c0[P.n_ci_blk] = c0;
             ++P.n_ci_blk;
         }
     }
-    if (db && !db_done) {
-        int rc = launch_bias_grad(dz, dz_c, (long long)batch * h * w, g->cout * g->groups == g->cout ? g->cout : g->cout, g->dtype, db,
-                                  (cudaStream_t)stream);
+    cudaStream_t st = (cudaStream_t)stream;
+    float* bias = db;
+    for (int s = 0; s < g->n_seg; ++s) {
+        const WgradPath path = wgrad_path(g, s);
+        if (path == kWgradTc) {
+            int rc = wgrad_tc_segment(g, s, &in[s], in_c[s], &dz, dz_c, 1, batch, h, w, cin_total, dw, &bias, st);
+            if (rc != VSRB_OK) return rc;
+        } else if (path == kWgradTaps) {
+            for (int c0 = 0; c0 < g->seg_c[s]; c0 += 64)
+                for (int n0 = 0; n0 < g->cout; n0 += 64) {
+                    const int ci_n = g->seg_c[s] - c0 < 64 ? g->seg_c[s] - c0 : 64, co_n = g->cout - n0 < 64 ? g->cout - n0 : 64;
+                    int rc = launch_wgrad_taps(in[s], in_c[s], c0, ci_n, g->seg_off[s] + c0, dz, dz_c, n0, co_n, g->kw, batch, h, w, cin_total,
+                                               dw, st);
+                    if (rc != VSRB_OK) return rc;
+                }
+        }
+    }
+    if (bias) {
+        int rc = launch_bias_grad(dz, dz_c, (long long)batch * h * w, g->cout, g->dtype, bias, st);
         if (rc != VSRB_OK) return rc;
     }
     if (P.n_ci_blk == 0) return VSRB_OK;
+    // every FFMA segment in one launch
     P.dz = dz; P.dz_c = dz_c;
-    P.kh = g->kh; P.kw = g->kw; P.H = h; P.W = w; P.imgs_per_group = imgs_per_group; P.groups = g->groups;
+    P.kh = g->kh; P.kw = g->kw; P.H = h; P.W = w;
     P.cout = g->cout; P.cin_total = cin_total;
-    P.n_co_blk = ceil_div(g->cout, co_t);
+    P.n_co_blk = ceil_div(g->cout, 64);
     P.dw = dw;
-    const bool mma_path = g->dtype == VSRB_BF16 && !getenv("VSRB_WGRAD_FFMA");
-    P.chunks_per_row = ceil_div(w, mma_path ? kMmaPx : 32);
-    const long long units_g = (long long)imgs_per_group * h * P.chunks_per_row;
-    VSRB_CHECK_ARG(units_g < (1LL << 31), "wgrad: too many pixels per group");
-    P.units_g = (int)units_g;
+    P.chunks_per_row = ceil_div(w, 32);
+    P.units = batch * h * P.chunks_per_row;
     // ~6 waves of the 148 SMs, at least 16 chunks (512 pixels) per CTA to amortise the final atomics
-    const long long other = (long long)g->kh * P.n_co_blk * P.n_ci_blk * g->groups;
-    long long ctas = (148LL * 6 + other - 1) / other;
-    long long per = (units_g + ctas - 1) / ctas;
+    const int other = g->kh * P.n_co_blk * P.n_ci_blk;
+    const int ctas = (148 * 6 + other - 1) / other;
+    int per = (P.units + ctas - 1) / ctas;
     if (per < 16) per = 16;
-    P.units_per_cta = (int)per;
-    dim3 grid((unsigned)((units_g + per - 1) / per), g->kh, P.n_co_blk * P.n_ci_blk * g->groups);
-    cudaStream_t st = (cudaStream_t)stream;
-#define VSRB_WG_KW(KERN, CO, CI)                                                       \
-    do {                                                                                \
-        if (g->kw == 1) KERN(1, CO, CI)<<<grid, 256, 0, st>>>(P);                       \
-        else if (g->kw == 3) KERN(3, CO, CI)<<<grid, 256, 0, st>>>(P);                  \
-        else if (g->kw == 7) KERN(7, CO, CI)<<<grid, 256, 0, st>>>(P);                  \
-        else {                                                                          \
-            set_error("wgrad: kernel width %d unsupported", g->kw);                     \
-            return VSRB_E_ARG;                                                          \
-        }                                                                               \
-    } while (0)
-#define VSRB_WG_CI(KERN, CO)                               \
-    do {                                                    \
-        if (ci_t == 16) VSRB_WG_KW(KERN, CO, 16);           \
-        else if (ci_t == 32) VSRB_WG_KW(KERN, CO, 32);      \
-        else VSRB_WG_KW(KERN, CO, 64);                      \
-    } while (0)
-#define VSRB_K_MMA(KW, CO, CI) conv_wgrad_mma_kernel<KW, CO, CI>
-#define VSRB_K_F32(KW, CO, CI) conv_wgrad_kernel<float, KW, CO, CI>
-#define VSRB_K_FFMA16(KW, CO, CI) conv_wgrad_kernel<__nv_bfloat16, KW, CO, CI>
-    if (g->dtype == VSRB_BF16 && !getenv("VSRB_WGRAD_FFMA")) {
-        if (co_t == 16) VSRB_WG_CI(VSRB_K_MMA, 16);
-        else if (co_t == 32) VSRB_WG_CI(VSRB_K_MMA, 32);
-        else VSRB_WG_CI(VSRB_K_MMA, 64);
-    } else if (g->dtype == VSRB_BF16) {                    // cross-check path: the FFMA kernel on bf16 data, 64 x 64 tiles
-        VSRB_WG_KW(VSRB_K_FFMA16, 64, 64);
-    } else {
-        VSRB_WG_KW(VSRB_K_F32, 64, 64);
-    }
-#undef VSRB_K_FFMA16
-#undef VSRB_K_F32
-#undef VSRB_K_MMA
-#undef VSRB_WG_CI
-#undef VSRB_WG_KW
+    P.units_per_cta = per;
+    const dim3 grid((unsigned)ceil_div(P.units, per), g->kh, P.n_co_blk * P.n_ci_blk);
+    using Kern = void (*)(WgradParams);
+    const Kern kern = g->dtype == VSRB_BF16
+        ? (g->kw == 1 ? conv_wgrad_kernel<__nv_bfloat16, 1> : g->kw == 3 ? conv_wgrad_kernel<__nv_bfloat16, 3> : conv_wgrad_kernel<__nv_bfloat16, 7>)
+        : (g->kw == 1 ? conv_wgrad_kernel<float, 1> : g->kw == 3 ? conv_wgrad_kernel<float, 3> : conv_wgrad_kernel<float, 7>);
+    kern<<<grid, 256, 0, st>>>(P);
     VSRB_LAUNCH_CHECK();
     return VSRB_OK;
 }

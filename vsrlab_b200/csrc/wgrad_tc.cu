@@ -244,13 +244,9 @@ __device__ __forceinline__ void bias_ld8(const float* p, float (&v)[8]) {
 // db[c] += sum over pixels of dz[p][c].  HBM-bound (reads dz once): every thread owns 8 consecutive channels (one 16-byte
 // load per pixel for bf16) and a strided set of pixels; the pixel lanes of a CTA are reduced in shared memory, then one
 // atomic per channel and CTA.  blockDim = 256 = G channel groups (G = 8 for 64 channels) x 256/G pixel lanes.
-struct BiasChunks {
-    const void* dz[16];            // up to 16 tensors of `pixels` pixels each (the chunks of vsrb_conv2d_wgrad_multi)
-    int n;
-};
-
 template <typename T>
-__global__ void __launch_bounds__(256) bias_grad_kernel(const BiasChunks ch, int dz_c, long long pixels, int cout, int G, float* __restrict__ db) {
+__global__ void __launch_bounds__(256) bias_grad_kernel(const T* __restrict__ dz, int dz_c, long long pixels, int cout, int G,
+                                                        float* __restrict__ db) {
     __shared__ float red[256][9];                                  // [thread][8 channels] (+1: no bank conflicts)
     const int grp = threadIdx.x % G, lane = threadIdx.x / G, lanes = 256 / G;
     const int c0 = (blockIdx.y * G + grp) * 8;
@@ -258,14 +254,11 @@ __global__ void __launch_bounds__(256) bias_grad_kernel(const BiasChunks ch, int
 #pragma unroll
     for (int i = 0; i < 8; ++i) s[i] = 0.f;
     if (c0 < dz_c) {
-        for (int k = 0; k < ch.n; ++k) {
-            const T* dz = reinterpret_cast<const T*>(ch.dz[k]);
-            for (long long p = (long long)blockIdx.x * lanes + lane; p < pixels; p += (long long)gridDim.x * lanes) {
-                float v[8];
-                bias_ld8(dz + p * dz_c + c0, v);
+        for (long long p = (long long)blockIdx.x * lanes + lane; p < pixels; p += (long long)gridDim.x * lanes) {
+            float v[8];
+            bias_ld8(dz + p * dz_c + c0, v);
 #pragma unroll
-                for (int i = 0; i < 8; ++i) s[i] += v[i];
-            }
+            for (int i = 0; i < 8; ++i) s[i] += v[i];
         }
     }
 #pragma unroll
@@ -284,27 +277,19 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-int launch_bias_grad_multi(const void* const* dzs, int n_chunks, int dz_c, long long pixels, int cout, int dtype, float* db,
-                           cudaStream_t s) {
+int launch_bias_grad(const void* dz, int dz_c, long long pixels, int cout, int dtype, float* db, cudaStream_t s) {
     const int groups = ceil_div(cout, 8);
     int G = 1;
     while (G < groups && G < 32) G *= 2;                            // channel groups per CTA: power of two <= 32
-    long long want = (pixels + 256 / G * 8 - 1) / (256 / G * 8);   // >= 8 pixels of a chunk per thread
+    long long want = (pixels + 256 / G * 8 - 1) / (256 / G * 8);   // >= 8 pixels per thread
     int gx = (int)(want < 1 ? 1 : (want > 148 * 4 ? 148 * 4 : want));
     dim3 grid(gx, ceil_div(groups, G));
-    for (int k0 = 0; k0 < n_chunks; k0 += 16) {
-        BiasChunks ch;
-        ch.n = n_chunks - k0 < 16 ? n_chunks - k0 : 16;
-        for (int k = 0; k < 16; ++k) ch.dz[k] = k < ch.n ? dzs[k0 + k] : nullptr;
-        if (dtype == VSRB_BF16) bias_grad_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(ch, dz_c, pixels, cout, G, db);
-        else bias_grad_kernel<float><<<grid, 256, 0, s>>>(ch, dz_c, pixels, cout, G, db);
-        VSRB_LAUNCH_CHECK();
-    }
+    if (dtype == VSRB_BF16)
+        bias_grad_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(reinterpret_cast<const __nv_bfloat16*>(dz), dz_c, pixels, cout, G, db);
+    else
+        bias_grad_kernel<float><<<grid, 256, 0, s>>>(reinterpret_cast<const float*>(dz), dz_c, pixels, cout, G, db);
+    VSRB_LAUNCH_CHECK();
     return VSRB_OK;
-}
-
-int launch_bias_grad(const void* dz, int dz_c, long long pixels, int cout, int dtype, float* db, cudaStream_t s) {
-    return launch_bias_grad_multi(&dz, 1, dz_c, pixels, cout, dtype, db, s);
 }
 
 // one 64-input-channel block (x channels [c0, c0+64), OIHW offset ci_off) against all 64-wide output blocks, summed over
@@ -374,23 +359,14 @@ int launch_wgrad_tc_multi(const void* const* xs, int x_c, int c0, int ci_off, co
     int ctas = sms / n_blocks;
     if (ctas > P.total_tiles / 32) ctas = P.total_tiles / 32;
     if (ctas < 1) ctas = 1;
-    {
-        const char* e = getenv("VSRB_WG_DEBUG");
-        P.debug = e ? atoi(e) : 0;
-        const char* c = getenv("VSRB_WG_CTAS");
-        if (c && atoi(c) > 0 && atoi(c) < ctas) ctas = atoi(c);
-    }
+    const char* dbg = getenv("VSRB_WG_DEBUG");
+    P.debug = dbg ? atoi(dbg) : 0;
     // blockIdx.y = 64-wide output block: all blocks of a wide layer (64 -> 256) share ONE launch.  (A launch per block on
     // sms / n_blocks CTAs each ran them one after the other - same stream - on a quarter of the GPU: 560 -> 230 us.)
     P.n0 = 0;
     wgrad_tc_kernel<<<dim3(ctas, n_blocks), kWgThreads, kWgSmem, stream>>>(P);
     VSRB_LAUNCH_CHECK();
     return VSRB_OK;
-}
-
-int launch_wgrad_tc(const void* x, int x_c, int c0, int ci_off, const void* dz, int dz_c, int batch, int h, int w, int cout,
-                    int cin_total, float* dw, cudaStream_t stream, float* db) {
-    return launch_wgrad_tc_multi(&x, x_c, c0, ci_off, &dz, dz_c, 1, batch, h, w, cout, cin_total, dw, stream, db);
 }
 
 }  // namespace vsrb
