@@ -28,7 +28,7 @@ pytestmark = pytest.mark.gpu
 
 # the kernel selection switches of the conv launcher (VSRB_TC_NO_STACK is read at pack and at launch time)
 SWITCHES = ("VSRB_RING_MIN_ROWS", "VSRB_TC_NO_RING", "VSRB_TC_NO_PAIR", "VSRB_TC_NO_STACK", "VSRB_RING_DEBUG",
-            "VSRB_TC_DIRECT_STORE", "VSRB_TC_DEBUG")
+            "VSRB_TC_DEBUG")
 TOL = 2e-5
 WORST = {}                                         # (epilogue, variant) -> worst error / bound, printed at the end
 

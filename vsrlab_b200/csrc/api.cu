@@ -1,8 +1,10 @@
-// C-ABI plumbing: errors, device info, conv geometry, weight packing, conv dispatch.
+// C-ABI plumbing: errors, device info, conv geometry, weight packing, conv dispatch; the per-device set-up and tensor
+// maps of the tcgen05 launchers.
 #include <stdarg.h>
 #include <stdlib.h>
 
 #include <atomic>
+#include <mutex>
 
 #include "common.cuh"
 
@@ -24,6 +26,69 @@ int* debug_flag() {
     int* p = nullptr;
     cudaGetSymbolAddress(reinterpret_cast<void**>(&p), g_debug_flag);
     return p;
+}
+
+int env_int(const char* name) {
+    const char* e = getenv(name);
+    return e ? atoi(e) : 0;
+}
+
+static std::mutex g_init_mutex;            // one-time per-process / per-device initialisation (callers may be threads)
+static int g_sm_count[kMaxDevices] = {0};
+
+int device_setup(int* dev, int* sms, bool (&done)[kMaxDevices], const std::function<int(int dev)>& setup) {
+    VSRB_CUDA(cudaGetDevice(dev));
+    VSRB_CHECK_ARG(*dev >= 0 && *dev < kMaxDevices, "device ordinal %d out of range", *dev);
+    std::lock_guard<std::mutex> lock(g_init_mutex);
+    if (!g_sm_count[*dev]) VSRB_CUDA(cudaDeviceGetAttribute(&g_sm_count[*dev], cudaDevAttrMultiProcessorCount, *dev));
+    if (!done[*dev]) {
+        const int rc = setup(*dev);
+        if (rc != VSRB_OK) return rc;
+        done[*dev] = true;
+    }
+    *sms = g_sm_count[*dev];
+    return VSRB_OK;
+}
+
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+int encode_map(CUtensorMap* map, const char* what, const void* base, int rank, const cuuint64_t* dims,
+               const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapSwizzle swz) {
+    static const EncodeTiledFn encode = [] {      // looked up once per process; a failed lookup stays failed
+        void* p = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
+                        q == cudaDriverEntryPointSuccess;
+        return ok ? reinterpret_cast<EncodeTiledFn>(p) : nullptr;
+    }();
+    if (!encode) {
+        set_error("cuTensorMapEncodeTiled not available from the driver");
+        return VSRB_E_NODEVICE;
+    }
+    const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+    const CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, const_cast<void*>(base), dims, strides, box, estr,
+                              CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r == CUDA_SUCCESS) return VSRB_OK;
+    char msg[400];
+    int n = snprintf(msg, sizeof(msg), "cuTensorMapEncodeTiled (%.40s) failed with %d: dims", what, (int)r);
+    for (int i = 0; i < rank; ++i) n += snprintf(msg + n, sizeof(msg) - n, " %llu", (unsigned long long)dims[i]);
+    n += snprintf(msg + n, sizeof(msg) - n, ", byte strides");
+    for (int i = 0; i + 1 < rank; ++i) n += snprintf(msg + n, sizeof(msg) - n, " %llu", (unsigned long long)strides[i]);
+    n += snprintf(msg + n, sizeof(msg) - n, ", box");
+    for (int i = 0; i < rank; ++i) n += snprintf(msg + n, sizeof(msg) - n, " %u", (unsigned)box[i]);
+    set_error("%s", msg);
+    return VSRB_E_CUDA;
+}
+
+int encode_nhwc(CUtensorMap* map, const char* what, const void* base, int c, int w, int h, int n, int box_c, int box_w,
+                int box_h) {
+    const cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)n};
+    const cuuint64_t strides[3] = {(cuuint64_t)c * 2, (cuuint64_t)w * c * 2, (cuuint64_t)h * w * c * 2};
+    const cuuint32_t box[4] = {(cuuint32_t)box_c, (cuuint32_t)box_w, (cuuint32_t)box_h, 1};
+    return encode_map(map, what, base, 4, dims, strides, box, swizzle_for(box_c));
 }
 
 // ---------------------------------------------------------------------------------------

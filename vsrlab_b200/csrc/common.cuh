@@ -8,6 +8,8 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <functional>
+
 #include "../../include/vsrb200.h"
 
 namespace vsrb {
@@ -50,6 +52,60 @@ int* debug_flag();   // device flag raised by kernels on a pipeline time-out
 
 static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 static inline size_t round_up(size_t a, size_t b) { return (a + b - 1) / b * b; }
+
+// ---------------------------------------------------------------------------------------
+// host plumbing of the tcgen05 launchers
+// ---------------------------------------------------------------------------------------
+int env_int(const char* name);   // integer debug switch from the environment, 0 when unset
+
+constexpr int kMaxDevices = 64;
+// The current device and its SM count (read once per device).  `setup` is the caller's one-time set-up for that device
+// (function attributes, constant tables); it runs under the library's initialisation lock until it returns VSRB_OK,
+// which the caller's `done` records.
+int device_setup(int* dev, int* sms, bool (&done)[kMaxDevices], const std::function<int(int dev)>& setup);
+
+// Swizzle of a K-major shared-memory tile whose rows hold `channels` bf16 (64: 128 B, 32: 64 B, 16: 32 B)
+static inline CUtensorMapSwizzle swizzle_for(int channels) {
+    return channels == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : (channels == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
+}
+// A bf16 tensor map of rank 4 or 5 (unit element strides, no interleave, 128-byte L2 promotion, zero fill out of bounds).
+// `strides` are the byte strides of dims 1..rank-1.  On failure the error names the map (`what`), its extents and strides.
+int encode_map(CUtensorMap* map, const char* what, const void* base, int rank, const cuuint64_t* dims,
+               const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapSwizzle swz);
+// The dense NHWC map: dims {c, w, h, n}, box {box_c, box_w, box_h, 1}, swizzle_for(box_c)
+int encode_nhwc(CUtensorMap* map, const char* what, const void* base, int c, int w, int h, int n, int box_c, int box_w,
+                int box_h);
+
+// cudaLaunchKernelEx with programmatic stream serialization (`pdl`) and clusters of `cluster_x` CTAs along x
+template <typename Params>
+int launch_ex(void (*kernel)(Params), const Params& args, dim3 grid, dim3 block, int smem, cudaStream_t stream, bool pdl,
+              int cluster_x) {
+    cudaLaunchAttribute attr[2];
+    int na = 0;
+    if (pdl) {
+        attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        attr[na].val.programmaticStreamSerializationAllowed = 1;
+        ++na;
+    }
+    if (cluster_x > 1) {
+        attr[na].id = cudaLaunchAttributeClusterDimension;
+        attr[na].val.clusterDim.x = cluster_x;
+        attr[na].val.clusterDim.y = 1;
+        attr[na].val.clusterDim.z = 1;
+        ++na;
+    }
+    cudaLaunchConfig_t cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cfg.attrs = attr;
+    cfg.numAttrs = na;
+    VSRB_CUDA(cudaLaunchKernelEx(&cfg, kernel, args));
+    VSRB_LAUNCH_CHECK();
+    return VSRB_OK;
+}
 
 // ---------------------------------------------------------------------------------------
 // conv geometry shared by packer and launchers

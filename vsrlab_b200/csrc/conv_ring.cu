@@ -31,8 +31,6 @@
 // as an equal number of ranges per strip (no crossings).  The launcher picks whichever needs fewer steps.
 #include <stdlib.h>
 
-#include <mutex>
-
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
@@ -476,14 +474,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) conv_ring_kernel(const __grid
 // ---------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn get_encode();        // conv_tc.cu
-
-static std::mutex g_ring_mutex;
-static bool g_ring_ready[64] = {false};
-static int g_ring_sms[64] = {0};
+static bool g_ring_ready[kMaxDevices] = {false};
 
 // Does this launch take the ring kernel?  (geometry: make_plan's p.ring; arguments: plain bf16 NHWC in / out)
 bool ring_eligible(const vsrb_conv_args* a, const ConvPlan& p) {
@@ -520,22 +511,12 @@ static int ring_steps(uint32_t rows_g, int H, int cols, int rpc, int n_ranges) {
 }
 
 int launch_conv_ring(const vsrb_conv_args* a, const ConvPlan& p, cudaStream_t stream) {
-    EncodeTiledFn encode = get_encode();
-    if (!encode) {
-        set_error("cuTensorMapEncodeTiled not available from the driver");
-        return VSRB_E_NODEVICE;
-    }
-    int dev = 0;
-    VSRB_CUDA(cudaGetDevice(&dev));
-    VSRB_CHECK_ARG(dev >= 0 && dev < 64, "device ordinal %d out of range", dev);
-    {
-        std::lock_guard<std::mutex> lock(g_ring_mutex);
-        if (!g_ring_ready[dev]) {
-            VSRB_CUDA(cudaDeviceGetAttribute(&g_ring_sms[dev], cudaDevAttrMultiProcessorCount, dev));
-            VSRB_CUDA(cudaFuncSetAttribute(conv_ring_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kRingSmem));
-            g_ring_ready[dev] = true;
-        }
-    }
+    int dev = 0, sms = 0;
+    int rc = device_setup(&dev, &sms, g_ring_ready, [](int) {
+        VSRB_CUDA(cudaFuncSetAttribute(conv_ring_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kRingSmem));
+        return VSRB_OK;
+    });
+    if (rc != VSRB_OK) return rc;
     RingParams P;
     memset(&P, 0, sizeof(P));
     EpiParams e;
@@ -552,66 +533,37 @@ int launch_conv_ring(const vsrb_conv_args* a, const ConvPlan& p, cudaStream_t st
     P.rows_g = (uint32_t)P.cols * (uint32_t)P.H;
     P.act_k = e.act_k;
     P.dbg = debug_flag();
-    {
-        const char* dbg_env = getenv("VSRB_RING_DEBUG");
-        P.debug = dbg_env ? atoi(dbg_env) : 0;
-    }
-    cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+    P.debug = env_int("VSRB_RING_DEBUG");
     if (P.has_main) {
         const int ms = p.ring_main_seg;
-        cuuint64_t dims[4] = {(cuuint64_t)a->in_c[ms], (cuuint64_t)a->w, (cuuint64_t)a->h, (cuuint64_t)a->batch};
-        cuuint64_t strides[3] = {(cuuint64_t)a->in_c[ms] * 2, (cuuint64_t)a->w * a->in_c[ms] * 2, (cuuint64_t)a->h * a->w * a->in_c[ms] * 2};
-        cuuint32_t box[4] = {64, 32, 1, 1};
-        CUresult r = encode(&P.in_map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(a->in[ms]), dims, strides, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            set_error("cuTensorMapEncodeTiled (ring input) failed with %d", (int)r);
-            return VSRB_E_CUDA;
-        }
+        rc = encode_nhwc(&P.in_map, "ring input", a->in[ms], a->in_c[ms], a->w, a->h, a->batch, 64, 32, 1);
+        if (rc != VSRB_OK) return rc;
     }
     for (int gi = 0; gi < (P.has_patch ? p.groups : 0); ++gi) {
         // both strides 0 = dense [groups][imgs_per_group]; with an explicit image stride the group stride is taken literally
         // (0 is then a real value: both propagation directions read the same frame at the middle time step)
         const long long istr = a->patch_img_stride ? a->patch_img_stride : (long long)a->h * a->w * 32;
         const long long gstr = (a->patch_img_stride || a->patch_group_stride) ? a->patch_group_stride : istr * a->imgs_per_group;
-        char* base = reinterpret_cast<char*>(const_cast<void*>(a->patch)) + (long long)gi * gstr * 2;
+        const char* base = reinterpret_cast<const char*>(a->patch) + (long long)gi * gstr * 2;
         cuuint64_t dims[4] = {32, (cuuint64_t)a->w, (cuuint64_t)a->h, (cuuint64_t)a->imgs_per_group};
         cuuint64_t strides[3] = {64, (cuuint64_t)a->w * 64, (cuuint64_t)istr * 2};
         cuuint32_t box[4] = {32, 32, 1, 1};
-        CUresult r = encode(&P.patch_map[gi], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                            CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            set_error("cuTensorMapEncodeTiled (ring patches) failed with %d", (int)r);
-            return VSRB_E_CUDA;
-        }
+        rc = encode_map(&P.patch_map[gi], "ring patches", base, 4, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_64B);
+        if (rc != VSRB_OK) return rc;
     }
     if (P.has_res) {
-        cuuint64_t dims[4] = {(cuuint64_t)a->res_c, (cuuint64_t)a->w, (cuuint64_t)a->h, (cuuint64_t)a->batch};
-        cuuint64_t strides[3] = {(cuuint64_t)a->res_c * 2, (cuuint64_t)a->w * a->res_c * 2, (cuuint64_t)a->h * a->w * a->res_c * 2};
-        cuuint32_t box[4] = {64, 32, 1, 1};
-        CUresult r = encode(&P.res_map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(a->residual), dims, strides, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            set_error("cuTensorMapEncodeTiled (ring residual) failed with %d", (int)r);
-            return VSRB_E_CUDA;
-        }
+        rc = encode_nhwc(&P.res_map, "ring residual", a->residual, a->res_c, a->w, a->h, a->batch, 64, 32, 1);
+        if (rc != VSRB_OK) return rc;
     }
     {
         cuuint64_t dims[5] = {(cuuint64_t)a->out_c, (cuuint64_t)a->w, (cuuint64_t)a->h, (cuuint64_t)a->imgs_per_group, (cuuint64_t)p.groups};
         cuuint64_t strides[4] = {(cuuint64_t)a->out_c * 2, (cuuint64_t)a->w * a->out_c * 2, (cuuint64_t)e.out_img_stride * 2,
                                  (cuuint64_t)e.out_group_stride * 2};
         cuuint32_t box[5] = {64, (cuuint32_t)kRingUW, 1, 1, 1};
-        CUresult r = encode(&P.out_map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, a->out, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            set_error("cuTensorMapEncodeTiled (ring output) failed with %d (c=%d w=%d h=%d imgs=%d groups=%d)", (int)r, a->out_c, a->w,
-                      a->h, a->imgs_per_group, p.groups);
-            return VSRB_E_CUDA;
-        }
+        rc = encode_map(&P.out_map, "ring output", a->out, 5, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B);
+        if (rc != VSRB_OK) return rc;
     }
-    int ctas_x = (g_ring_sms[dev] / p.groups) & ~1;
+    int ctas_x = (sms / p.groups) & ~1;
     if (ctas_x < 2) ctas_x = 2;
     {   // never more ranges than rows: empty walks are legal but pointless
         long long want = ((long long)P.rows_g + 3) / 4;
@@ -627,29 +579,8 @@ int launch_conv_ring(const vsrb_conv_args* a, const ConvPlan& p, cudaStream_t st
             ring_steps(P.rows_g, P.H, P.cols, rpc, n_ranges) < ring_steps(P.rows_g, P.H, P.cols, 0, n_ranges))
             P.rpc = rpc;
     }
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(ctas_x, p.groups);
-    cfg.blockDim = dim3(kRingThreads);
-    cfg.dynamicSmemBytes = kRingCtrl + 1024 + VSRB_RING_W_BYTES + P.num_slots * P.slot_bytes + kRingStageBytes;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[2];
-    int na = 0;
-    if (a->flags & VSRB_CONV_PDL) {
-        attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[na].val.programmaticStreamSerializationAllowed = 1;
-        ++na;
-    }
-    attr[na].id = cudaLaunchAttributeClusterDimension;
-    attr[na].val.clusterDim.x = 2;
-    attr[na].val.clusterDim.y = 1;
-    attr[na].val.clusterDim.z = 1;
-    ++na;
-    cfg.attrs = attr;
-    cfg.numAttrs = na;
-    VSRB_CUDA(cudaLaunchKernelEx(&cfg, conv_ring_kernel, P));
-    VSRB_LAUNCH_CHECK();
-    return VSRB_OK;
+    const int smem = kRingCtrl + 1024 + VSRB_RING_W_BYTES + P.num_slots * P.slot_bytes + kRingStageBytes;
+    return launch_ex(conv_ring_kernel, P, dim3(ctas_x, p.groups), dim3(kRingThreads), smem, stream, a->flags & VSRB_CONV_PDL, 2);
 }
 
 }  // namespace vsrb

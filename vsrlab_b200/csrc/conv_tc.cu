@@ -27,8 +27,6 @@
 // basicvsr.py:75-82; realbasicvsr.py:28-29; spynet.py:16-21 (see include/vsrb200.h).
 #include <stdlib.h>
 
-#include <mutex>
-
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
@@ -771,73 +769,34 @@ __global__ void fill_identity_kernel() {
 // ---------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+// conv_tc_kernel<staged, kw, pair> by [staged][pair][kw: 0, 3, 7] (kw 0: classic layout, 3 / 7: stacked)
+static void (*const kConvTcKernels[2][2][3])(TcParams) = {
+    {{conv_tc_kernel<false, 0>, conv_tc_kernel<false, 3>, conv_tc_kernel<false, 7>},
+     {conv_tc_kernel<false, 0, true>, conv_tc_kernel<false, 3, true>, conv_tc_kernel<false, 7, true>}},
+    {{conv_tc_kernel<true, 0>, conv_tc_kernel<true, 3>, conv_tc_kernel<true, 7>},
+     {conv_tc_kernel<true, 0, true>, conv_tc_kernel<true, 3, true>, conv_tc_kernel<true, 7, true>}}};
 
-static std::mutex g_init_mutex;            // one-time per-process / per-device initialisation (callers may be threads)
-
-EncodeTiledFn get_encode() {
-    static EncodeTiledFn fn = nullptr;
-    static bool tried = false;
-    std::lock_guard<std::mutex> lock(g_init_mutex);
-    if (!tried) {
-        tried = true;
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeTiledFn>(p);
-    }
-    return fn;
-}
-
-static int g_sm_count[64] = {0};
-static bool g_dev_ready[64] = {false};
-static const uint8_t* g_ident_ptr[64] = {nullptr};
-
-static CUtensorMapSwizzle swizzle_for(int channels) {
-    return channels == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : (channels == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-}
+static bool g_dev_ready[kMaxDevices] = {false};
+static const uint8_t* g_ident_ptr[kMaxDevices] = {nullptr};
 
 int launch_conv_tc(const vsrb_conv_args* a, const ConvPlan& p, cudaStream_t stream) {
-    EncodeTiledFn encode = get_encode();
-    if (!encode) {
-        set_error("cuTensorMapEncodeTiled not available from the driver");
-        return VSRB_E_NODEVICE;
-    }
-    int dev = 0;
-    VSRB_CUDA(cudaGetDevice(&dev));
-    VSRB_CHECK_ARG(dev >= 0 && dev < 64, "device ordinal %d out of range", dev);
-    std::unique_lock<std::mutex> init_lock(g_init_mutex);
-    if (!g_dev_ready[dev]) {
-        VSRB_CUDA(cudaDeviceGetAttribute(&g_sm_count[dev], cudaDevAttrMultiProcessorCount, dev));
-        VSRB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<true, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        VSRB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<false, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        VSRB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<true, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        VSRB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<false, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        VSRB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<true, 7>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        VSRB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<false, 7>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        VSRB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<true, 3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        VSRB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<true, 7, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        VSRB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<false, 3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        VSRB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<false, 7, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        VSRB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<true, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
-        VSRB_CUDA(cudaFuncSetAttribute(conv_tc_kernel<false, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
+    int dev = 0, sms = 0;
+    int rc = device_setup(&dev, &sms, g_dev_ready, [&](int d) {
+        for (auto& by_pair : kConvTcKernels)
+            for (auto& by_kw : by_pair)
+                for (auto kern : by_kw) VSRB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax));
         void* ip = nullptr;
         VSRB_CUDA(cudaGetSymbolAddress(&ip, g_identity));
-        g_ident_ptr[dev] = reinterpret_cast<const uint8_t*>(ip);
+        g_ident_ptr[d] = reinterpret_cast<const uint8_t*>(ip);
         // one-time: finish before any other stream of this process can launch a conv that reads it
         fill_identity_kernel<<<16, 256, 0, stream>>>();
         VSRB_LAUNCH_CHECK();
-        {
-            cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-            cudaStreamIsCapturing(stream, &cap);
-            if (cap == cudaStreamCaptureStatusNone) VSRB_CUDA(cudaStreamSynchronize(stream));
-        }
-        g_dev_ready[dev] = true;
-    }
-    init_lock.unlock();
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        cudaStreamIsCapturing(stream, &cap);
+        if (cap == cudaStreamCaptureStatusNone) VSRB_CUDA(cudaStreamSynchronize(stream));
+        return VSRB_OK;
+    });
+    if (rc != VSRB_OK) return rc;
     TcParams P;
     memset(&P, 0, sizeof(P));
     P.n_seg = p.n_seg; P.kh = p.kh; P.kw = p.kw; P.H = a->h; P.W = a->w;
@@ -847,10 +806,7 @@ int launch_conv_tc(const vsrb_conv_args* a, const ConvPlan& p, cudaStream_t stre
     P.w = reinterpret_cast<const uint8_t*>(a->packed) + p.bias_bytes;
     P.ident = g_ident_ptr[dev];
     P.dbg = debug_flag();
-    {
-        const char* e = getenv("VSRB_TC_DEBUG");
-        P.debug = e ? atoi(e) : 0;
-    }
+    P.debug = env_int("VSRB_TC_DEBUG");
     fill_epi(a, p, &P.epi);
 
     P.TW = p.stacked ? 32 : (a->w <= 8 ? 8 : 16);
@@ -860,13 +816,13 @@ int launch_conv_tc(const vsrb_conv_args* a, const ConvPlan& p, cudaStream_t stre
     P.ns = p.ns;
     P.res_xoff = p.stacked ? p.kw / 2 : 0;
     const int units = p.groups * p.n_blocks;
-    const int ctas_budget = (a->max_ctas > 0 ? a->max_ctas : g_sm_count[dev]);
+    const int ctas_budget = (a->max_ctas > 0 ? a->max_ctas : sms);
 
     // EPI_NHWC tiles leave through two swizzled staging buffers and TMA stores (full-line, asynchronous
-    // writes); needs positive 16-byte-multiple strides.  VSRB_TC_DIRECT_STORE=1 forces per-thread stores.
+    // writes); needs positive 16-byte-multiple strides.
     const long long oimg = P.epi.out_img_stride, ogrp = P.epi.out_group_stride;
     bool staged = a->epilogue == VSRB_EPI_NHWC && oimg > 0 && ogrp > 0 && oimg % 8 == 0 && ogrp % 8 == 0 && !a->split &&
-                  (reinterpret_cast<uintptr_t>(a->out) & 15) == 0 && !getenv("VSRB_TC_DIRECT_STORE");
+                  (reinterpret_cast<uintptr_t>(a->out) & 15) == 0;
     P.n_store = (p.n_tile % 64 == 0) ? 64 : ((p.n_tile % 32 == 0) ? 32 : 16);   // store block must divide n_tile
     if (p.pixshuf && p.cout / 4 < P.n_store) P.n_store = p.cout / 4;
     if (P.n_store != 16 && P.n_store != 32 && P.n_store != 64) staged = false;
@@ -932,7 +888,6 @@ int launch_conv_tc(const vsrb_conv_args* a, const ConvPlan& p, cudaStream_t stre
     P.acc_cols = P.MT * p.ns;
     P.tiles_x = ceil_div(a->w, P.UW);
     P.tiles_per_img = P.tiles_x * ceil_div(a->h, P.rows_sub * P.MT);
-    cuuint32_t estr[5] = {1, 1, 1, 1, 1};
     {
         uint32_t woff = 0;
         for (int s = 0; s < p.n_seg; ++s) {
@@ -948,32 +903,14 @@ int launch_conv_tc(const vsrb_conv_args* a, const ConvPlan& p, cudaStream_t stre
         P.op_wseg[s] = a->n_in ? a->in_wseg[s] : s;
         P.op_c0[s] = a->n_in ? a->in_c0[s] : 0;
         const SegPlan& sp = p.seg[P.op_wseg[s]];
-        cuuint64_t dims[4] = {(cuuint64_t)a->in_c[s], (cuuint64_t)a->w, (cuuint64_t)a->h, (cuuint64_t)a->batch};
-        cuuint64_t strides[3] = {(cuuint64_t)a->in_c[s] * 2, (cuuint64_t)a->w * a->in_c[s] * 2,
-                                 (cuuint64_t)a->h * a->w * a->in_c[s] * 2};
-        cuuint32_t box[4] = {(cuuint32_t)sp.ck, (cuuint32_t)P.TW, (cuuint32_t)P.box_rows, 1};
         VSRB_CHECK_ARG(a->in_c[s] % 8 == 0, "segment %d: channel stride %d must be a multiple of 8", s, a->in_c[s]);
         VSRB_CHECK_ARG((reinterpret_cast<uintptr_t>(a->in[s]) & 15) == 0, "segment %d: pointer not 16-byte aligned", s);
-        CUresult r = encode(&P.tmap[s], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(a->in[s]), dims, strides, box,
-                            estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(sp.ck), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            set_error("cuTensorMapEncodeTiled failed with %d (seg %d, c=%d w=%d h=%d b=%d box=%d,%d,%d)", (int)r, s,
-                      a->in_c[s], a->w, a->h, a->batch, sp.ck, P.TW, P.box_rows);
-            return VSRB_E_CUDA;
-        }
+        rc = encode_nhwc(&P.tmap[s], "input", a->in[s], a->in_c[s], a->w, a->h, a->batch, sp.ck, P.TW, P.box_rows);
+        if (rc != VSRB_OK) return rc;
     }
     if (P.res_mma) {
-        cuuint64_t dims[4] = {(cuuint64_t)a->res_c, (cuuint64_t)a->w, (cuuint64_t)a->h, (cuuint64_t)a->batch};
-        cuuint64_t strides[3] = {(cuuint64_t)a->res_c * 2, (cuuint64_t)a->w * a->res_c * 2, (cuuint64_t)a->h * a->w * a->res_c * 2};
-        cuuint32_t box[4] = {64, (cuuint32_t)P.TW, (cuuint32_t)(P.rows_sub * P.MT), 1};
-        CUresult r = encode(&P.rmap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(a->residual), dims, strides, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            set_error("cuTensorMapEncodeTiled (residual) failed with %d", (int)r);
-            return VSRB_E_CUDA;
-        }
+        rc = encode_nhwc(&P.rmap, "residual", a->residual, a->res_c, a->w, a->h, a->batch, 64, P.TW, P.rows_sub * P.MT);
+        if (rc != VSRB_OK) return rc;
     }
     if (staged) {
         const int nq = p.pixshuf ? 4 : 1, sx = p.pixshuf ? 2 : 1;
@@ -985,14 +922,8 @@ int launch_conv_tc(const vsrb_conv_args* a, const ConvPlan& p, cudaStream_t stre
             cuuint64_t strides[4] = {(cuuint64_t)sx * a->out_c * 2, (cuuint64_t)sx * OW * a->out_c * 2, (cuuint64_t)oimg * 2,
                                      (cuuint64_t)ogrp * 2};
             cuuint32_t box[5] = {(cuuint32_t)P.n_store, (cuuint32_t)P.UW, (cuuint32_t)(p.stacked ? 1 : 32 / P.TW), 1, 1};
-            CUresult r = encode(&P.smap[q], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, obase, dims, strides, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(P.n_store), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r != CUDA_SUCCESS) {
-                set_error("cuTensorMapEncodeTiled (store) failed with %d (c=%d w=%d h=%d imgs=%d groups=%d, strides %lld %lld)",
-                          (int)r, a->out_c, a->w, a->h, a->imgs_per_group, p.groups, oimg, ogrp);
-                return VSRB_E_CUDA;
-            }
+            rc = encode_map(&P.smap[q], "store", obase, 5, dims, strides, box, swizzle_for(P.n_store));
+            if (rc != VSRB_OK) return rc;
         }
     }
     const int tiles_g = a->imgs_per_group * P.tiles_per_img;
@@ -1006,41 +937,10 @@ int launch_conv_tc(const vsrb_conv_args* a, const ConvPlan& p, cudaStream_t stre
         if (ctas_x > want) ctas_x = want;
     }
     const int smem = kCtrlBytes + 1024 + (int)P.wres_bytes + ident_total + P.num_slots * P.slot_bytes + (staged ? stg_total : 0);
-    dim3 grid(ctas_x, units);
-    const int kkw = p.stacked ? p.kw : 0;
     P.pdl = (a->flags & VSRB_CONV_PDL) ? 1 : 0;
-    void (*kern)(TcParams) = nullptr;
-    if (pair && staged)
-        kern = kkw == 3 ? conv_tc_kernel<true, 3, true> : (kkw == 7 ? conv_tc_kernel<true, 7, true> : conv_tc_kernel<true, 0, true>);
-    else if (pair)
-        kern = kkw == 3 ? conv_tc_kernel<false, 3, true> : (kkw == 7 ? conv_tc_kernel<false, 7, true> : conv_tc_kernel<false, 0, true>);
-    else if (staged) kern = kkw == 3 ? conv_tc_kernel<true, 3> : (kkw == 7 ? conv_tc_kernel<true, 7> : conv_tc_kernel<true, 0>);
-    else kern = kkw == 3 ? conv_tc_kernel<false, 3> : (kkw == 7 ? conv_tc_kernel<false, 7> : conv_tc_kernel<false, 0>);
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = grid;
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[2];
-    int na = 0;
-    if (P.pdl) {
-        attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[na].val.programmaticStreamSerializationAllowed = 1;
-        ++na;
-    }
-    if (pair) {
-        attr[na].id = cudaLaunchAttributeClusterDimension;
-        attr[na].val.clusterDim.x = 2;
-        attr[na].val.clusterDim.y = 1;
-        attr[na].val.clusterDim.z = 1;
-        ++na;
-    }
-    cfg.attrs = attr;
-    cfg.numAttrs = na;
-    VSRB_CUDA(cudaLaunchKernelEx(&cfg, kern, P));
-    VSRB_LAUNCH_CHECK();
-    return VSRB_OK;
+    const int kkw = p.stacked ? p.kw : 0;
+    return launch_ex(kConvTcKernels[staged][pair][kkw == 3 ? 1 : (kkw == 7 ? 2 : 0)], P, dim3(ctas_x, units), dim3(kThreads), smem,
+                     stream, P.pdl, pair ? 2 : 1);
 }
 
 }  // namespace vsrb

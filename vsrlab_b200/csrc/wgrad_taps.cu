@@ -19,10 +19,6 @@
 // U rows it needs.  One box of S (R rows, 16 + K-1 pixels) and one of U (R + nj-1 rows, 16 pixels) per 16 x R pixel tile,
 // mbarrier ring.  Epilogue: per 16 U channels the accumulators go through shared memory in OIHW order, then leave as runs
 // of nj*K consecutive floats with coalesced atomics.
-#include <stdlib.h>
-
-#include <mutex>
-
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
@@ -210,42 +206,21 @@ __global__ void __launch_bounds__(kTpThreads, 1) wgrad_taps_kernel(const __grid_
     }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 static int pow2_block(int c) { return c <= 16 ? 16 : (c <= 32 ? 32 : 64); }
 
 // One (input-channel block, output-channel block) pair: x channels [x_c0, x_c0 + ci_n), dz channels [z_c0, z_c0 + co_n),
 // ci_n, co_n <= 64.  `ci_off` = OIHW position of x channel x_c0.
 int launch_wgrad_taps(const void* x, int x_c, int x_c0, int ci_n, int ci_off, const void* dz, int dz_c, int z_c0, int co_n, int K,
                       int batch, int h, int w, int cin_total, float* dw, cudaStream_t stream) {
-    static EncodeTiledFn encode = nullptr;
-    static bool attr[64] = {false};
-    static int sm_count[64] = {0};
-    static std::mutex init_mutex;
-    int dev = 0;
-    VSRB_CUDA(cudaGetDevice(&dev));
-    VSRB_CHECK_ARG(dev >= 0 && dev < 64, "device ordinal %d out of range", dev);
+    static bool ready[kMaxDevices] = {false};
     VSRB_CHECK_ARG(K >= 1 && K <= 7 && (K & 1) && ci_n >= 1 && ci_n <= 64 && co_n >= 1 && co_n <= 64, "wgrad_taps: bad block");
     constexpr int kSmemMax = 200 * 1024;
-    {
-        std::lock_guard<std::mutex> lock(init_mutex);
-        if (!encode) {
-            void* p = nullptr;
-            cudaDriverEntryPointQueryResult q;
-            if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
-                set_error("cuTensorMapEncodeTiled not available from the driver");
-                return VSRB_E_NODEVICE;
-            }
-            encode = reinterpret_cast<EncodeTiledFn>(p);
-        }
-        if (!attr[dev]) {
-            VSRB_CUDA(cudaFuncSetAttribute(wgrad_taps_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax + 2048));
-            VSRB_CUDA(cudaDeviceGetAttribute(&sm_count[dev], cudaDevAttrMultiProcessorCount, dev));
-            attr[dev] = true;
-        }
-    }
+    int dev = 0, sms = 0;
+    int rc = device_setup(&dev, &sms, ready, [](int) {
+        VSRB_CUDA(cudaFuncSetAttribute(wgrad_taps_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemMax + 2048));
+        return VSRB_OK;
+    });
+    if (rc != VSRB_OK) return rc;
     WgTapsParams P;
     memset(&P, 0, sizeof(P));
     const int bx = pow2_block(ci_n), bz = pow2_block(co_n);
@@ -291,32 +266,15 @@ int launch_wgrad_taps(const void* x, int x_c, int x_c0, int ci_n, int ci_off, co
     P.dbg = debug_flag();
     VSRB_CHECK_ARG(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dz)) & 15) == 0 && x_c % 8 == 0 && dz_c % 8 == 0,
                    "wgrad_taps: tensors must be 16-byte aligned with channel strides that are multiples of 8");
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    auto swz = [](int c) { return c == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : (c == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B); };
-    {
-        cuuint64_t dims[4] = {(cuuint64_t)s_c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)batch};
-        cuuint64_t strides[3] = {(cuuint64_t)s_c * 2, (cuuint64_t)w * s_c * 2, (cuuint64_t)h * w * s_c * 2};
-        cuuint32_t box[4] = {(cuuint32_t)P.cs, (cuuint32_t)box_w, (cuuint32_t)P.rows, 1};
-        CUresult r = encode(&P.smap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(s_ptr), dims, strides, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, swz(P.cs), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) { set_error("wgrad_taps: tensor map (S) failed with %d", (int)r); return VSRB_E_CUDA; }
-    }
-    {
-        cuuint64_t dims[4] = {(cuuint64_t)u_c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)batch};
-        cuuint64_t strides[3] = {(cuuint64_t)u_c * 2, (cuuint64_t)w * u_c * 2, (cuuint64_t)h * w * u_c * 2};
-        cuuint32_t box[4] = {(cuuint32_t)P.cu, (cuuint32_t)kTpTW, (cuuint32_t)u_rows, 1};
-        CUresult r = encode(&P.umap, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(u_ptr), dims, strides, box, estr,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, swz(P.cu), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) { set_error("wgrad_taps: tensor map (U) failed with %d", (int)r); return VSRB_E_CUDA; }
-    }
+    rc = encode_nhwc(&P.smap, "wgrad_taps S", s_ptr, s_c, w, h, batch, P.cs, box_w, P.rows);
+    if (rc != VSRB_OK) return rc;
+    rc = encode_nhwc(&P.umap, "wgrad_taps U", u_ptr, u_c, w, h, batch, P.cu, kTpTW, u_rows);
+    if (rc != VSRB_OK) return rc;
     // every CTA ends with K*K*cs*cu/passes atomics: small problems use fewer CTAs (>= 8 tiles each)
-    int ctas = sm_count[dev] / passes;
+    int ctas = sms / passes;
     if (ctas > P.total_tiles / 8) ctas = P.total_tiles / 8;
     if (ctas < 1) ctas = 1;
-    {
-        const char* e = getenv("VSRB_WG_DEBUG");
-        P.debug = e ? atoi(e) : 0;
-    }
+    P.debug = env_int("VSRB_WG_DEBUG");
     const int smem = 1024 + 1024 + P.stages * P.stage_bytes;
     wgrad_taps_kernel<<<dim3(ctas, passes), kTpThreads, smem, stream>>>(P);
     VSRB_LAUNCH_CHECK();

@@ -19,10 +19,6 @@
 //                persistent CTA; K advances 16 pixels (2048 bytes) per MMA.
 // Every pixel tile is read once; at the end each CTA adds its partial dW into the fp32 OIHW gradient with atomics.
 // Replaces the wgrad half of autograd's ConvolutionBackward0 for the hot 64->64 / 64->256 3x3 layers.
-#include <stdlib.h>
-
-#include <mutex>
-
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
@@ -273,10 +269,6 @@ __global__ void __launch_bounds__(256) bias_grad_kernel(const T* __restrict__ dz
     }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
 int launch_bias_grad(const void* dz, int dz_c, long long pixels, int cout, int dtype, float* db, cudaStream_t s) {
     const int groups = ceil_div(cout, 8);
     int G = 1;
@@ -296,32 +288,14 @@ int launch_bias_grad(const void* dz, int dz_c, long long pixels, int cout, int d
 // `n_chunks` (x, dz) pairs of `batch` images each
 int launch_wgrad_tc_multi(const void* const* xs, int x_c, int c0, int ci_off, const void* const* dzs, int dz_c, int n_chunks,
                           int batch, int h, int w, int cout, int cin_total, float* dw, cudaStream_t stream, float* db) {
-    static EncodeTiledFn encode = nullptr;
-    static bool attr[64] = {false};                  // function attributes are per device
-    static int sm_count[64] = {0};
-    static std::mutex init_mutex;
-    int dev = 0;
-    VSRB_CUDA(cudaGetDevice(&dev));
-    VSRB_CHECK_ARG(dev >= 0 && dev < 64, "device ordinal %d out of range", dev);
+    static bool ready[kMaxDevices] = {false};
     VSRB_CHECK_ARG(n_chunks >= 1 && n_chunks <= kWgMaxChunks, "wgrad: 1..%d chunks per launch", kWgMaxChunks);
-    {
-        std::lock_guard<std::mutex> lock(init_mutex);
-        if (!encode) {
-            void* p = nullptr;
-            cudaDriverEntryPointQueryResult q;
-            if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
-                set_error("cuTensorMapEncodeTiled not available from the driver");
-                return VSRB_E_NODEVICE;
-            }
-            encode = reinterpret_cast<EncodeTiledFn>(p);
-        }
-        if (!attr[dev]) {
-            VSRB_CUDA(cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem));
-            VSRB_CUDA(cudaDeviceGetAttribute(&sm_count[dev], cudaDevAttrMultiProcessorCount, dev));
-            attr[dev] = true;
-        }
-    }
-    const int sms = sm_count[dev];
+    int dev = 0, sms = 0;
+    int rc = device_setup(&dev, &sms, ready, [](int) {
+        VSRB_CUDA(cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem));
+        return VSRB_OK;
+    });
+    if (rc != VSRB_OK) return rc;
     WgTcParams P;
     memset(&P, 0, sizeof(P));
     P.H = h; P.W = w; P.batch = batch;
@@ -331,36 +305,20 @@ int launch_wgrad_tc_multi(const void* const* xs, int x_c, int c0, int ci_off, co
     P.total_tiles = P.tiles_per_chunk * n_chunks;
     P.c0 = c0; P.cout = cout; P.cin_total = cin_total; P.ci_off = ci_off; P.dw = dw; P.db = db;
     P.dbg = debug_flag();
-    cuuint32_t estr[4] = {1, 1, 1, 1};
     for (int k = 0; k < n_chunks; ++k) {
         VSRB_CHECK_ARG(xs[k] && dzs[k] && ((reinterpret_cast<uintptr_t>(xs[k]) | reinterpret_cast<uintptr_t>(dzs[k])) & 15) == 0,
                        "wgrad: chunk %d: null or unaligned tensor", k);
-        {
-            cuuint64_t dims[4] = {(cuuint64_t)x_c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)batch};
-            cuuint64_t strides[3] = {(cuuint64_t)x_c * 2, (cuuint64_t)w * x_c * 2, (cuuint64_t)h * w * x_c * 2};
-            cuuint32_t box[4] = {64, kWgXW, kWgRows + 2, 1};
-            CUresult r = encode(&P.xmap[k], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(xs[k]), dims, strides, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r != CUDA_SUCCESS) { set_error("wgrad: tensor map (x) failed with %d", (int)r); return VSRB_E_CUDA; }
-        }
-        {
-            cuuint64_t dims[4] = {(cuuint64_t)dz_c, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)batch};
-            cuuint64_t strides[3] = {(cuuint64_t)dz_c * 2, (cuuint64_t)w * dz_c * 2, (cuuint64_t)h * w * dz_c * 2};
-            cuuint32_t box[4] = {64, kWgTW, kWgRows, 1};
-            CUresult r = encode(&P.zmap[k], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(dzs[k]), dims, strides, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r != CUDA_SUCCESS) { set_error("wgrad: tensor map (dz) failed with %d", (int)r); return VSRB_E_CUDA; }
-        }
+        rc = encode_nhwc(&P.xmap[k], "wgrad x", xs[k], x_c, w, h, batch, 64, kWgXW, kWgRows + 2);
+        if (rc != VSRB_OK) return rc;
+        rc = encode_nhwc(&P.zmap[k], "wgrad dz", dzs[k], dz_c, w, h, batch, 64, kWgTW, kWgRows);
+        if (rc != VSRB_OK) return rc;
     }
     const int n_blocks = ceil_div(cout, 64);
     // every CTA ends with 9*64*64 atomics, so small problems use fewer CTAs (>= 32 pixel tiles each)
     int ctas = sms / n_blocks;
     if (ctas > P.total_tiles / 32) ctas = P.total_tiles / 32;
     if (ctas < 1) ctas = 1;
-    const char* dbg = getenv("VSRB_WG_DEBUG");
-    P.debug = dbg ? atoi(dbg) : 0;
+    P.debug = env_int("VSRB_WG_DEBUG");
     // blockIdx.y = 64-wide output block: all blocks of a wide layer (64 -> 256) share ONE launch.  (A launch per block on
     // sms / n_blocks CTAs each ran them one after the other - same stream - on a quarter of the GPU: 560 -> 230 us.)
     P.n0 = 0;
