@@ -201,6 +201,34 @@ int vsrb_flow_warp_bwd(const void* x, const float* flow, const void* dout, float
                        int32_t n, int32_t h, int32_t w, int32_t c, int32_t dtype, int32_t padding_mode,
                        void* stream);
 
+/* ---- deterministic gradients (torch.use_deterministic_algorithms) ----------------------
+ * The same gradients with a fixed order of every floating-point addition: two calls on the same inputs, on a GPU with the
+ * same SM count, give bit-identical results.  The library allocates nothing: the caller passes a device workspace of at
+ * least the bytes its *_workspace_bytes query returns (16-byte aligned; 0 from a query = refused arguments, see
+ * vsrb_last_error).  Nothing synchronises the host, so the calls can be captured in CUDA graphs.  Arguments, including a
+ * workspace that is too small, are refused with VSRB_E_ARG before any work is enqueued.
+ * vsrb_conv2d_wgrad(_multi)_det: the contract of vsrb_conv2d_wgrad(_multi) (dw, db accumulated); every CTA stores its
+ * partial block to its own workspace slot and one kernel adds the slots in slot order.  Refused: the geometries of the
+ * FFMA fallback (fp32 data, non-square filters).  The query takes the forward geometry, the chunk count (1 = the plan of
+ * vsrb_conv2d_wgrad_det) and whether db is computed.                                                                  */
+size_t vsrb_conv2d_wgrad_det_workspace_bytes(const vsrb_conv_geom* g, int32_t n_chunks, int32_t batch, int32_t h, int32_t w,
+                                             int32_t with_bias);
+int vsrb_conv2d_wgrad_det(const vsrb_conv_geom* g, const void* const* in, const int32_t* in_c, const void* dz,
+                          int32_t dz_c, int32_t batch, int32_t h, int32_t w, int32_t imgs_per_group,
+                          int32_t cin_total, float* dw, float* db, void* workspace, size_t workspace_bytes, void* stream);
+int vsrb_conv2d_wgrad_multi_det(const vsrb_conv_geom* g, int32_t n_chunks, const void* const* in, const int32_t* in_c,
+                                const void* const* dz, int32_t dz_c, int32_t batch, int32_t h, int32_t w,
+                                int32_t cin_total, float* dw, float* db, void* workspace, size_t workspace_bytes,
+                                void* stream);
+/* vsrb_flow_warp_bwd with dx OVERWRITTEN (fp32 [n,h,w,c], or NULL): the taps' contributions are summed as 64-bit
+ * fixed-point integers scaled from max|dout|; a non-finite dout makes all of dx NaN.  dflow (or NULL) is the output of
+ * vsrb_flow_warp_bwd itself (single writer per pixel); it needs c / (8 bf16 | 4 fp32) to be a power of two <= 32.
+ * padding_mode zeros or border.  The workspace is needed for dx only.                                                 */
+size_t vsrb_flow_warp_bwd_det_workspace_bytes(int32_t n, int32_t h, int32_t w, int32_t c);
+int vsrb_flow_warp_bwd_det(const void* x, const float* flow, const void* dout, float* dx, float* dflow,
+                           int32_t n, int32_t h, int32_t w, int32_t c, int32_t dtype, int32_t padding_mode,
+                           void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- backward warp: replaces flow_warp = meshgrid + normalise + F.grid_sample ---------
  * reference: spynet.py:95-106; callers basicvsr.py:54,69.
  * x,out: NHWC [n,h,w,c] of `dtype`, c % 8 == 0; flow fp32 [n,h,w,2].                    */
@@ -283,6 +311,22 @@ int vsrb_psnr_sums(const float* x, const float* y, int32_t images, int64_t per_i
  * borders, k1 0.01, k2 0.03, value range 1 = piqa.SSIM defaults); the map has channels*(h-10)*(w-10) entries      */
 int vsrb_ssim_sums(const float* x, const float* y, int32_t images, int32_t channels, int32_t h, int32_t w,
                    int32_t clamp_x, double* sums, void* stream);
+/* the same four with each block's sum stored to a workspace slot and the slots added in block order (deterministic
+ * sums, see "deterministic gradients" above); the queries take the shape arguments of their entry point           */
+size_t vsrb_charbonnier_det_workspace_bytes(int64_t n);
+size_t vsrb_charbonnier_resized_det_workspace_bytes(int32_t planes, int32_t h, int32_t w);
+size_t vsrb_psnr_sums_det_workspace_bytes(int32_t images, int64_t per_image);
+size_t vsrb_ssim_sums_det_workspace_bytes(int32_t images, int32_t channels, int32_t h, int32_t w);
+int vsrb_charbonnier_det(const float* x, const float* y, int64_t n, float eps, double* sum, float* grad,
+                         const float* grad_scale_dev, float grad_scale, void* workspace, size_t workspace_bytes,
+                         void* stream);
+int vsrb_charbonnier_resized_det(const float* lq, const float* hr, int32_t planes, int32_t h, int32_t w, int32_t H,
+                                 int32_t W, float eps, double* sum, float* grad, const float* grad_scale_dev,
+                                 float grad_scale, void* workspace, size_t workspace_bytes, void* stream);
+int vsrb_psnr_sums_det(const float* x, const float* y, int32_t images, int64_t per_image, double* sums,
+                       void* workspace, size_t workspace_bytes, void* stream);
+int vsrb_ssim_sums_det(const float* x, const float* y, int32_t images, int32_t channels, int32_t h, int32_t w,
+                       int32_t clamp_x, double* sums, void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -4,6 +4,7 @@ launched with torchrun.  Prints one JSON line (rank 0)."""
 import argparse
 import json
 import os
+import subprocess
 import sys
 import time
 from pathlib import Path
@@ -32,7 +33,12 @@ def main():
                          "single GPU) and time its replay: what the step costs once the host is out of the loop")
     ap.add_argument("--host-profile", action="store_true", help="cProfile one step on the host (stderr)")
     ap.add_argument("--kernel-profile", action="store_true", help="torch.profiler (CUPTI) table of every kernel of one step (stderr)")
+    ap.add_argument("--deterministic", action="store_true",
+                    help="also time the step under torch.use_deterministic_algorithms(True), alternating with the default mode "
+                         "in rounds of --steps steps (single GPU)")
     a = ap.parse_args()
+    if a.deterministic:
+        os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")     # torch's condition for deterministic cuBLAS products
     import torch.distributed as dist
     from vsrlab.vsr.models.RealBasicVSR.realbasicvsr import RealBasicVSR
     from vsrlab_b200 import ops
@@ -150,6 +156,35 @@ def main():
         d[0] += ev0.elapsed_time(ev1)
         d[1] += work
         d[2] += 1
+    det_ms = None
+    if a.deterministic and world == 1:
+        # both modes warmed up (each captures its own training graphs), then alternating rounds: the median per mode
+        def timed(mode, n):
+            torch.use_deterministic_algorithms(mode)
+            ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            ev0.record()
+            for _ in range(n):
+                step()
+            ev1.record()
+            torch.cuda.synchronize()
+            return ev0.elapsed_time(ev1) / n
+        for mode in (False, True):
+            timed(mode, a.warmup + 4)
+        rounds = {False: [], True: []}
+        for _ in range(5):
+            for mode in (False, True):
+                rounds[mode].append(timed(mode, a.steps))
+        torch.use_deterministic_algorithms(False)
+        med = {m: sorted(v)[len(v) // 2] for m, v in rounds.items()}
+        try:
+            power = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", str(local)],
+                                   capture_output=True, text=True, timeout=30).stdout.strip()
+        except (OSError, subprocess.SubprocessError):
+            power = "unknown"
+        det_ms = {"gpu": torch.cuda.get_device_name(dev), "power_limit": power, "ms_default": round(med[False], 3),
+                  "ms_deterministic": round(med[True], 3), "rounds_ms": {"default": [round(v, 3) for v in rounds[False]],
+                                                                         "deterministic": [round(v, 3) for v in rounds[True]]},
+                  "cost": f"{100.0 * (med[True] / med[False] - 1.0):+.1f} %"}
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -165,6 +200,7 @@ def main():
             "workload": f"cfg4 training step: batch {a.batch}/GPU x {a.frames} frames 64x64, {a.blocks}/{a.blocks} blocks, train_flow={a.train_flow}",
             "n_gpus": world, "ms_per_step": t.item(), "ms_per_step_cuda_graph": ms_graph, "clips_per_sec": world * a.batch / (t.item() * 1e-3),
             "loss_first": float(losses[0]), "loss_last": float(losses[-1]), "replicas_identical": same,
+            **({"deterministic": det_ms} if det_ms is not None else {}),
             "kernels_ms": {k: {"ms": round(v[0], 2), "launches": v[2], "tflops_or_gbs": round(v[1] / max(v[0], 1e-9) / 1e9, 1)}
                            for k, v in fam.items()},
         }), flush=True)

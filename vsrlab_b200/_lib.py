@@ -106,6 +106,27 @@ SYMBOLS = {
                                                                                        C.c_float, C.c_void_p]),
     "vsrb_psnr_sums": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p]),
     "vsrb_ssim_sums": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int32] * 5 + [C.c_void_p, C.c_void_p]),
+    # deterministic variants: the arguments above + (workspace, workspace_bytes) before the stream
+    "vsrb_conv2d_wgrad_det_workspace_bytes": (C.c_size_t, [C.POINTER(ConvGeom)] + [C.c_int32] * 5),
+    "vsrb_conv2d_wgrad_det": (C.c_int, [C.POINTER(ConvGeom), C.POINTER(C.c_void_p), C.POINTER(C.c_int32), C.c_void_p, C.c_int32,
+                                        C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_size_t, C.c_void_p]),
+    "vsrb_conv2d_wgrad_multi_det": (C.c_int, [C.POINTER(ConvGeom), C.c_int32, C.POINTER(C.c_void_p), C.POINTER(C.c_int32),
+                                              C.POINTER(C.c_void_p), C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
+                                              C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "vsrb_flow_warp_bwd_det_workspace_bytes": (C.c_size_t, [C.c_int32] * 4),
+    "vsrb_flow_warp_bwd_det": (C.c_int, [C.c_void_p] * 5 + [C.c_int32] * 6 + [C.c_void_p, C.c_size_t, C.c_void_p]),
+    "vsrb_charbonnier_det_workspace_bytes": (C.c_size_t, [C.c_int64]),
+    "vsrb_charbonnier_resized_det_workspace_bytes": (C.c_size_t, [C.c_int32] * 3),
+    "vsrb_psnr_sums_det_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int64]),
+    "vsrb_ssim_sums_det_workspace_bytes": (C.c_size_t, [C.c_int32] * 4),
+    "vsrb_charbonnier_det": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float,
+                                       C.c_void_p, C.c_size_t, C.c_void_p]),
+    "vsrb_charbonnier_resized_det": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int32] * 5 + [C.c_float, C.c_void_p, C.c_void_p,
+                                                                                           C.c_void_p, C.c_float, C.c_void_p,
+                                                                                           C.c_size_t, C.c_void_p]),
+    "vsrb_psnr_sums_det": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "vsrb_ssim_sums_det": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int32] * 5 + [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
 }
 
 _lib = None

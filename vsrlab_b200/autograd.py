@@ -250,7 +250,10 @@ class SrTailFn(torch.autograd.Function):
                 dx = F.pad(dx[:, :conv.in_channels], (0, 0, 0, 0, 0, xc - conv.in_channels))
         dlq = None
         if ctx.needs_input_grad[6]:
-            dlq = torch.ops.aten.upsample_bilinear2d_backward(dsr, [hh, ww], list(ctx.lq_shape), False, None, None)
+            if ops.deterministic():
+                dlq = _resize_bilinear_backward(dsr, ctx.lq_shape[-2:], False)
+            else:
+                dlq = torch.ops.aten.upsample_bilinear2d_backward(dsr, [hh, ww], list(ctx.lq_shape), False, None, None)
         return dw, (db if (conv.bias is not None and ctx.needs_input_grad[1]) else None), None, None, None, dx, dlq
 
 
@@ -460,42 +463,77 @@ def cleaner(cl, x: torch.Tensor) -> torch.Tensor:
     return x
 
 
-_up2_mats: dict = {}
+_resize_mats: dict = {}
+
+
+def _resize_matrix(size: int, out: int, align_corners: bool, device) -> torch.Tensor:
+    """[out, size] fp32: the weights of F.interpolate's bilinear resize (no antialias) along one axis."""
+    key = (size, out, bool(align_corners), str(device))
+    m = _resize_mats.get(key)
+    if m is None:
+        o = torch.arange(out, dtype=torch.float64)
+        if align_corners:
+            pos = o * ((size - 1) / (out - 1) if out > 1 else 0.0)
+        else:
+            pos = ((o + 0.5) * (size / out) - 0.5).clamp_(min=0.0)
+        i0 = pos.floor().clamp_(0, size - 1).long()
+        i1 = (i0 + 1).clamp_(max=size - 1)
+        f = (pos - i0.double()).float()
+        m = torch.zeros(out, size)
+        m[torch.arange(out), i0] += 1.0 - f
+        m[torch.arange(out), i1] += f
+        m = m.to(device)
+        _resize_mats[key] = m
+    return m
+
+
+def _resize_bilinear(x: torch.Tensor, size, align_corners: bool) -> torch.Tensor:
+    """F.interpolate(x, size, mode="bilinear", align_corners) as matrix products A_h @ x @ A_w^T (fp32), differentiable as
+    is.  An axis that keeps its size is not multiplied, so a same-size resize is an exact identity.  torch's bilinear
+    kernel parallelises over the output pixels only and loops over n * c inside each thread (0.08 - 0.2 ms per level on the
+    224 x 2 flow maps of SPyNet's x2 upsampling), and its backward has no deterministic CUDA implementation."""
+    n, c, h, w = x.shape
+    oh, ow = size
+    with torch.autocast("cuda", enabled=False):                           # flows stay fp32 (autocast would run the products in half)
+        y = x.float().reshape(n * c, h, w)
+        if oh != h:
+            y = torch.matmul(_resize_matrix(h, oh, align_corners, x.device), y)          # rows
+        if ow != w:
+            y = torch.matmul(y, _resize_matrix(w, ow, align_corners, x.device).t())      # columns
+        return y.view(n, c, oh, ow)
+
+
+def _resize_bilinear_backward(g: torch.Tensor, size, align_corners: bool) -> torch.Tensor:
+    """The gradient of _resize_bilinear wrt its [n, c, *size] input: A_h^T @ g @ A_w."""
+    n, c, oh, ow = g.shape
+    h, w = size
+    y = g.float().reshape(n * c, oh, ow)
+    if oh != h:
+        y = torch.matmul(_resize_matrix(h, oh, align_corners, g.device).t(), y)
+    if ow != w:
+        y = torch.matmul(y, _resize_matrix(w, ow, align_corners, g.device))
+    return y.reshape(n, c, h, w)
+
+
+def _bilinear(x: torch.Tensor, size, align_corners: bool = False) -> torch.Tensor:
+    """F.interpolate(x, size, mode="bilinear"); under torch.use_deterministic_algorithms the matrix products of
+    _resize_bilinear, whose backward is deterministic."""
+    if ops.deterministic():
+        return _resize_bilinear(x, size, align_corners)
+    return F.interpolate(x, size=size, mode="bilinear", align_corners=align_corners)
 
 
 def _upsample2_aligned(x: torch.Tensor) -> torch.Tensor:
-    """F.interpolate(x, scale_factor=2, mode="bilinear", align_corners=True) (spynet.py:64-66) as two small matrix
-    products, A_h @ x @ A_w^T.  torch's kernel parallelises over the output pixels only and loops over n * c inside each
-    thread: on the 224 x 2 flow maps of a pyramid level it took 0.08 - 0.2 ms per level (0.95 ms per step with its
-    backward); differentiable as is."""
-    n, c, h, w = x.shape
-
-    def mat(size):
-        key = (size, str(x.device))
-        m = _up2_mats.get(key)
-        if m is None:
-            out = 2 * size
-            pos = torch.arange(out, dtype=torch.float64) * ((size - 1) / (out - 1) if out > 1 else 0.0)
-            i0 = pos.floor().clamp_(0, size - 1).long()
-            i1 = (i0 + 1).clamp_(max=size - 1)
-            f = (pos - i0.double()).float()
-            m = torch.zeros(out, size)
-            m[torch.arange(out), i0] += 1.0 - f
-            m[torch.arange(out), i1] += f
-            m = m.to(x.device)
-            _up2_mats[key] = m
-        return m
-    with torch.autocast("cuda", enabled=False):                           # flows stay fp32 (autocast would run the products in half)
-        y = torch.matmul(mat(h), x.float().reshape(n * c, h, w))          # rows
-        return torch.matmul(y, mat(w).t()).view(n, c, 2 * h, 2 * w)       # columns
+    """F.interpolate(x, scale_factor=2, mode="bilinear", align_corners=True) (spynet.py:64-66)."""
+    return _resize_bilinear(x, (2 * x.shape[2], 2 * x.shape[3]), True)
 
 
 def spynet(sp, ref: torch.Tensor, supp: torch.Tensor) -> torch.Tensor:
     """Spynet.forward with gradients (spynet.py:38-93); resampling glue in torch fp32, convs + warps native."""
     h, w = ref.shape[-2:]
     hp, wp = (h + 31) // 32 * 32, (w + 31) // 32 * 32
-    ref = F.interpolate(ref, size=(hp, wp), mode="bilinear", align_corners=False)
-    supp = F.interpolate(supp, size=(hp, wp), mode="bilinear", align_corners=False)
+    ref = _bilinear(ref, (hp, wp))
+    supp = _bilinear(supp, (hp, wp))
     refs, supps = [(ref - sp.mean) / sp.std], [(supp - sp.mean) / sp.std]
     for _ in range(5):
         refs.append(F.avg_pool2d(refs[-1], 2, 2))
@@ -512,7 +550,7 @@ def spynet(sp, ref: torch.Tensor, supp: torch.Tensor) -> torch.Tensor:
             cv = mods[j].conv[0]
             x = conv(cv, [x], [(0, cv.in_channels)], "relu")
         flow = flow_up + x[:, :2].float()
-    flow = F.interpolate(flow, size=(h, w), mode="bilinear", align_corners=False)
+    flow = _bilinear(flow, (h, w))
     # per-axis rescale without a host-built tensor (keeps the step capturable in a CUDA graph)
     return torch.cat([flow[:, :1] * (float(w) / float(wp)), flow[:, 1:] * (float(h) / float(hp))], 1)
 
@@ -633,7 +671,11 @@ def basicvsr(bv, lrs: torch.Tensor) -> torch.Tensor:
         sr = sr_tail(last, x, lrs.reshape(n * t, c, h, w))                   # conv + bilinear skip in one kernel
     else:
         x = conv(last, [x], [(0, last.in_channels)], "none")[:, :c].float()
-        sr = x + F.interpolate(lrs.reshape(n * t, c, h, w), scale_factor=scale, mode="bilinear", align_corners=False)
+        lq = lrs.reshape(n * t, c, h, w)
+        if ops.deterministic():
+            sr = x + _resize_bilinear(lq, (h * scale, w * scale), False)
+        else:
+            sr = x + F.interpolate(lq, scale_factor=scale, mode="bilinear", align_corners=False)
     return sr.view(n, t, c, h * scale, w * scale)
 
 

@@ -64,6 +64,21 @@ constexpr int kMaxDevices = 64;
 // which the caller's `done` records.
 int device_setup(int* dev, int* sms, bool (&done)[kMaxDevices], const std::function<int(int dev)>& setup);
 
+// Deterministic weight / bias gradients (the *_det entry points of train.cu): the launchers store every CTA's partial block
+// in a slot of the caller's workspace `ws` and sum the slots in slot order (launch_slot_reduce) instead of adding with
+// atomics.  With `plan` set they launch nothing and only raise `need` (floats) to what they would use.
+struct WgradDet {
+    float* ws;
+    size_t need;
+    bool plan;
+};
+int launch_slot_reduce(const float* parts, int slots, int rows, int row_len, long long dst_stride, float* dst, cudaStream_t s);
+// a launcher about to use `floats` of the workspace: true = planning only, launch nothing
+static inline bool det_take(WgradDet* det, size_t floats) {
+    if (floats > det->need) det->need = floats;
+    return det->plan;
+}
+
 // Swizzle of a K-major shared-memory tile whose rows hold `channels` bf16 (64: 128 B, 32: 64 B, 16: 32 B)
 static inline CUtensorMapSwizzle swizzle_for(int channels) {
     return channels == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : (channels == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);

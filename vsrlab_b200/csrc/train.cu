@@ -8,6 +8,9 @@
 //  * flow_warp backward         = flow_warp_bwd_kernel: scatter of the output gradient through the four bilinear
 //    taps (grad wrt the warped features) and the derivative of the taps wrt the sample position (grad wrt the
 //    flow, needed when train_flow=True) - reference: GridSampler2DBackward0 behind spynet.py:95-106.
+#include <algorithm>
+#include <vector>
+
 #include "common.cuh"
 #include "warp_modes.cuh"
 
@@ -440,11 +443,11 @@ static void launch_warp_ex_bwd(const T* x, const float2* flow, const T* dout, fl
     else launch_warp_ex_bwd_t<T, VSRB_INTERP_BILINEAR>(x, flow, dout, dx, dflow, n, h, w, c, pad, align, s);
 }
 
-int launch_bias_grad(const void* dz, int dz_c, long long pixels, int cout, int dtype, float* db, cudaStream_t s);
+int launch_bias_grad(const void* dz, int dz_c, long long pixels, int cout, int dtype, float* db, cudaStream_t s, WgradDet* det);
 int launch_wgrad_tc_multi(const void* const* xs, int x_c, int c0, int ci_off, const void* const* dzs, int dz_c, int n_chunks,
-                          int batch, int h, int w, int cout, int cin_total, float* dw, cudaStream_t stream, float* db);
+                          int batch, int h, int w, int cout, int cin_total, float* dw, cudaStream_t stream, float* db, WgradDet* det);
 int launch_wgrad_taps(const void* x, int x_c, int x_c0, int ci_n, int ci_off, const void* dz, int dz_c, int z_c0, int co_n, int K,
-                      int batch, int h, int w, int cin_total, float* dw, cudaStream_t stream);
+                      int batch, int h, int w, int cin_total, float* dw, cudaStream_t stream, WgradDet* det);
 
 // The kernel that computes the weight gradient of input segment s.  3x3 layers whose segment has a multiple of 64 channels
 // (the resblock, upsampling and HR convs: > 85 % of the FLOPs) run on wgrad_tc_kernel - except thin outputs: the 64 -> 3
@@ -463,14 +466,158 @@ static WgradPath wgrad_path(const vsrb_conv_geom* g, int s) {
 // rides on the first launch if *db is set (the kernel's idle epilogue warps add up the dz tiles it streams anyway); *db is
 // then cleared.
 static int wgrad_tc_segment(const vsrb_conv_geom* g, int s, const void* const* xs, int x_c, const void* const* dzs, int dz_c,
-                            int n_chunks, int batch, int h, int w, int cin_total, float* dw, float** db, cudaStream_t st) {
+                            int n_chunks, int batch, int h, int w, int cin_total, float* dw, float** db, cudaStream_t st,
+                            WgradDet* det) {
     for (int c0 = 0; c0 < g->seg_c[s]; c0 += 64) {
         int rc = launch_wgrad_tc_multi(xs, x_c, c0, g->seg_off[s] + c0, dzs, dz_c, n_chunks, batch, h, w, g->cout, cin_total, dw, st,
-                                       *db);
+                                       *db, det);
         if (rc != VSRB_OK) return rc;
         *db = nullptr;
     }
     return VSRB_OK;
+}
+
+// ---------------------------------------------------------------------------------------
+// Deterministic dx of flow_warp_bwd (vsrb_flow_warp_bwd_det).  The output gradient is scattered through the four bilinear
+// taps as 64-bit fixed-point integers: integer addition is associative, so the order in which the atomics land does not
+// change the sum.  The scale is a power of two derived from max|dout|, itself found with an atomicMax of the bit patterns
+// (order-independent), such that no target can overflow: a target receives at most h*w contributions (one per source
+// pixel of its image: a pixel's four taps are distinct) of at most max|dout| each.  The quantum is then at most
+// max|dout| * h*w * 2^-60, far below fp32 rounding of any entry that is not ~2^-30 times smaller than max|dout|.
+// ---------------------------------------------------------------------------------------
+template <typename T>
+__global__ void __launch_bounds__(256) abs_max_kernel(const T* __restrict__ v, long long n, unsigned* __restrict__ out) {
+    unsigned m = 0;
+    for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n; i += (long long)gridDim.x * 256)
+        m = max(m, __float_as_uint(fabsf((float)v[i])));           // non-negative floats order like their bit patterns
+#pragma unroll
+    for (int o = 16; o >= 1; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
+    if ((threadIdx.x & 31) == 0) atomicMax(out, m);
+}
+
+// 2^(62 - e - e_hw) with max|dout| < 2^e and h*w < 2^e_hw
+__device__ __forceinline__ double fixed_scale(unsigned amax_bits, int hw) {
+    int e;
+    frexpf(__uint_as_float(amax_bits), &e);
+    const int e_hw = 32 - __clz(hw);
+    return ldexp(1.0, 62 - e - e_hw);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(256) flow_warp_bwd_dx_fixed_kernel(const float2* __restrict__ flow, const T* __restrict__ dout,
+                                                                     unsigned long long* __restrict__ acc, const unsigned* __restrict__ amax,
+                                                                     int n, int h, int w, int tpp, int border) {
+    constexpr int VEC = 16 / sizeof(T);
+    const unsigned mbits = *amax;
+    if (mbits >= 0x7f800000u) return;                               // inf / NaN in dout: the conversion reports it
+    const double scale = fixed_scale(mbits, h * w);
+    const int C = tpp * VEC;
+    const int hw = h * w;
+    const long long total = (long long)n * hw * tpp;
+    for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < total; i += (long long)gridDim.x * 256) {
+        const int part = (int)(i % tpp);
+        const long long pix = i / tpp;
+        const int img = (int)(pix / hw), r = (int)(pix - (long long)img * hw);
+        const int yy = r / w, xx = r - yy * w;
+        const float2 f = __ldg(flow + pix);
+        float ix, iy;                                               // the forward's / flow_warp_bwd_kernel's fp32 arithmetic
+        sample_pos_b((float)xx + f.x, (float)yy + f.y, w, h, ix, iy);
+        if (border) {
+            ix = fminf(fmaxf(ix, 0.f), (float)(w - 1));
+            iy = fminf(fmaxf(iy, 0.f), (float)(h - 1));
+        }
+        float fx = floorf(ix), fy = floorf(iy);
+        const float wx1 = ix - fx, wy1 = iy - fy, wx0 = 1.f - wx1, wy0 = 1.f - wy1;
+        fx = fminf(fmaxf(fx, -2.f), (float)w);
+        fy = fminf(fmaxf(fy, -2.f), (float)h);
+        const int x0 = (int)fx, y0 = (int)fy;
+        float go[VEC];
+        ld_vec<T>(dout + pix * C + part * VEC, go);
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const int xi = x0 + (k & 1), yi = y0 + (k >> 1);
+            if (xi < 0 || xi >= w || yi < 0 || yi >= h) continue;
+            const double wgt = (double)(((k & 1) ? wx1 : wx0) * ((k >> 1) ? wy1 : wy0)) * scale;
+            unsigned long long* dst = acc + ((long long)img * hw + (long long)yi * w + xi) * C + part * VEC;
+#pragma unroll
+            for (int j = 0; j < VEC; ++j)
+                if (go[j] != 0.f) atomicAdd(dst + j, (unsigned long long)__double2ll_rn((double)go[j] * wgt));
+        }
+    }
+}
+
+// dx = acc / scale, one store per element (targets nothing reached get 0); a non-finite max|dout| gives NaN everywhere
+__global__ void __launch_bounds__(256) fixed_to_float_kernel(const long long* __restrict__ acc, const unsigned* __restrict__ amax,
+                                                             long long n, int hw, float* __restrict__ dx) {
+    const unsigned mbits = *amax;
+    const bool finite = mbits < 0x7f800000u;
+    const double inv = finite ? 1.0 / fixed_scale(mbits, hw) : 0.0;
+    for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n; i += (long long)gridDim.x * 256)
+        dx[i] = finite ? (float)((double)acc[i] * inv) : __int_as_float(0x7fffffff);
+}
+
+template <typename T>
+static int launch_warp_bwd_dx_det(const float2* flow, const T* dout, float* dx, int n, int h, int w, int c, int border, void* ws,
+                                  cudaStream_t s) {
+    constexpr int VEC = 16 / sizeof(T);
+    const long long elems = (long long)n * h * w * c;
+    unsigned* amax = reinterpret_cast<unsigned*>(ws);
+    long long* acc = reinterpret_cast<long long*>(reinterpret_cast<char*>(ws) + 16);
+    VSRB_CUDA(cudaMemsetAsync(ws, 0, 16 + (size_t)elems * 8, s));
+    auto grid = [](long long items) { long long b = (items + 255) / 256; return (int)(b > 148 * 16 ? 148 * 16 : b); };
+    abs_max_kernel<T><<<grid(elems), 256, 0, s>>>(dout, elems, amax);
+    flow_warp_bwd_dx_fixed_kernel<T><<<grid(elems / VEC), 256, 0, s>>>(flow, dout, reinterpret_cast<unsigned long long*>(acc), amax, n,
+                                                                       h, w, c / VEC, border);
+    fixed_to_float_kernel<<<grid(elems), 256, 0, s>>>(acc, amax, elems, h * w, dx);
+    VSRB_LAUNCH_CHECK();
+    return VSRB_OK;
+}
+
+static size_t warp_bwd_det_bytes(int n, int h, int w, int c) { return 16 + (size_t)n * h * w * c * 8; }
+
+// The launches of vsrb_conv2d_wgrad_multi after its argument checks (det: deterministic mode, see WgradDet)
+static int wgrad_multi_run(const vsrb_conv_geom* g, int n_chunks, const void* const* in, const int32_t* in_c, const void* const* dz,
+                           int dz_c, int batch, int h, int w, int cin_total, float* dw, float* db, cudaStream_t st, WgradDet* det) {
+    for (int k0 = 0; k0 < n_chunks; k0 += 16) {
+        const int nk = n_chunks - k0 < 16 ? n_chunks - k0 : 16;
+        float* bias = db;                                   // once per group of chunks
+        for (int s = 0; s < g->n_seg; ++s) {
+            const void* xs[16];
+            for (int k = 0; k < nk; ++k) xs[k] = in[(size_t)(k0 + k) * g->n_seg + s];
+            int rc = wgrad_tc_segment(g, s, xs, in_c[s], dz + k0, dz_c, nk, batch, h, w, cin_total, dw, &bias, st, det);
+            if (rc != VSRB_OK) return rc;
+        }
+    }
+    return VSRB_OK;
+}
+
+static int check_wgrad_multi(const vsrb_conv_geom* g, int32_t n_chunks, const void* const* in, const int32_t* in_c,
+                             const void* const* dz, int32_t dz_c, int32_t cin_total, float* dw) {
+    VSRB_CHECK_ARG(g && in && in_c && dz && dw && n_chunks >= 1, "wgrad_multi: null argument");
+    VSRB_CHECK_ARG(g->dtype == VSRB_BF16 && g->kh == 3 && g->kw == 3 && g->groups == 1 && !g->pixshuf && !g->transpose &&
+                       g->n_seg >= 1 && g->n_seg <= 2 && dz_c >= g->cout && dz_c % 8 == 0,
+                   "wgrad_multi: bf16 3x3 ungrouped convs only (tensor-core path)");
+    for (int s = 0; s < g->n_seg; ++s)
+        VSRB_CHECK_ARG(g->seg_c[s] % 64 == 0 && in_c[s] % 8 == 0 && in_c[s] >= g->seg_c[s] && g->seg_off[s] + g->seg_c[s] <= cin_total,
+                       "wgrad_multi: segment %d must have a multiple of 64 channels", s);
+    return VSRB_OK;
+}
+
+static int wgrad_impl(const vsrb_conv_geom* g, const void* const* in, const int32_t* in_c, const void* dz, int32_t dz_c,
+                      int32_t batch, int32_t h, int32_t w, int32_t imgs_per_group, int32_t cin_total, float* dw, float* db,
+                      void* stream, WgradDet* det);
+
+// Runs `run` once in planning mode, checks the caller's workspace against what it needs, then runs it for real.
+template <typename Run>
+static int det_run(void* workspace, size_t workspace_bytes, const char* what, Run run) {
+    WgradDet det = {nullptr, 0, true};
+    int rc = run(&det);
+    if (rc != VSRB_OK) return rc;
+    VSRB_CHECK_ARG(det.need * 4 <= workspace_bytes && (det.need == 0 || workspace) && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0,
+                   "%s: the workspace must be 16-byte aligned and hold %zu bytes (got %zu)", what, det.need * 4, workspace_bytes);
+    det.ws = reinterpret_cast<float*>(workspace);
+    det.plan = false;
+    return run(&det);
 }
 
 }  // namespace vsrb
@@ -482,29 +629,64 @@ extern "C" {
 int vsrb_conv2d_wgrad_multi(const vsrb_conv_geom* g, int32_t n_chunks, const void* const* in, const int32_t* in_c,
                             const void* const* dz, int32_t dz_c, int32_t batch, int32_t h, int32_t w, int32_t cin_total,
                             float* dw, float* db, void* stream) {
-    VSRB_CHECK_ARG(g && in && in_c && dz && dw && n_chunks >= 1, "wgrad_multi: null argument");
-    VSRB_CHECK_ARG(g->dtype == VSRB_BF16 && g->kh == 3 && g->kw == 3 && g->groups == 1 && !g->pixshuf && !g->transpose &&
-                       g->n_seg >= 1 && g->n_seg <= 2 && dz_c >= g->cout && dz_c % 8 == 0,
-                   "wgrad_multi: bf16 3x3 ungrouped convs only (tensor-core path)");
-    for (int s = 0; s < g->n_seg; ++s)
-        VSRB_CHECK_ARG(g->seg_c[s] % 64 == 0 && in_c[s] % 8 == 0 && in_c[s] >= g->seg_c[s] && g->seg_off[s] + g->seg_c[s] <= cin_total,
-                       "wgrad_multi: segment %d must have a multiple of 64 channels", s);
-    for (int k0 = 0; k0 < n_chunks; k0 += 16) {
-        const int nk = n_chunks - k0 < 16 ? n_chunks - k0 : 16;
-        float* bias = db;                                   // once per group of chunks
-        for (int s = 0; s < g->n_seg; ++s) {
-            const void* xs[16];
-            for (int k = 0; k < nk; ++k) xs[k] = in[(size_t)(k0 + k) * g->n_seg + s];
-            int rc = wgrad_tc_segment(g, s, xs, in_c[s], dz + k0, dz_c, nk, batch, h, w, cin_total, dw, &bias, (cudaStream_t)stream);
-            if (rc != VSRB_OK) return rc;
-        }
-    }
-    return VSRB_OK;
+    const int rc = check_wgrad_multi(g, n_chunks, in, in_c, dz, dz_c, cin_total, dw);
+    if (rc != VSRB_OK) return rc;
+    return wgrad_multi_run(g, n_chunks, in, in_c, dz, dz_c, batch, h, w, cin_total, dw, db, (cudaStream_t)stream, nullptr);
+}
+
+int vsrb_conv2d_wgrad_multi_det(const vsrb_conv_geom* g, int32_t n_chunks, const void* const* in, const int32_t* in_c,
+                                const void* const* dz, int32_t dz_c, int32_t batch, int32_t h, int32_t w, int32_t cin_total,
+                                float* dw, float* db, void* workspace, size_t workspace_bytes, void* stream) {
+    const int rc = check_wgrad_multi(g, n_chunks, in, in_c, dz, dz_c, cin_total, dw);
+    if (rc != VSRB_OK) return rc;
+    return det_run(workspace, workspace_bytes, "wgrad_multi_det", [&](WgradDet* det) {
+        return wgrad_multi_run(g, n_chunks, in, in_c, dz, dz_c, batch, h, w, cin_total, dw, db, (cudaStream_t)stream, det);
+    });
 }
 
 int vsrb_conv2d_wgrad(const vsrb_conv_geom* g, const void* const* in, const int32_t* in_c, const void* dz, int32_t dz_c,
                       int32_t batch, int32_t h, int32_t w, int32_t imgs_per_group, int32_t cin_total, float* dw, float* db,
                       void* stream) {
+    return wgrad_impl(g, in, in_c, dz, dz_c, batch, h, w, imgs_per_group, cin_total, dw, db, stream, nullptr);
+}
+
+int vsrb_conv2d_wgrad_det(const vsrb_conv_geom* g, const void* const* in, const int32_t* in_c, const void* dz, int32_t dz_c,
+                          int32_t batch, int32_t h, int32_t w, int32_t imgs_per_group, int32_t cin_total, float* dw, float* db,
+                          void* workspace, size_t workspace_bytes, void* stream) {
+    return det_run(workspace, workspace_bytes, "wgrad_det", [&](WgradDet* det) {
+        return wgrad_impl(g, in, in_c, dz, dz_c, batch, h, w, imgs_per_group, cin_total, dw, db, stream, det);
+    });
+}
+
+size_t vsrb_conv2d_wgrad_det_workspace_bytes(const vsrb_conv_geom* g, int32_t n_chunks, int32_t batch, int32_t h, int32_t w,
+                                             int32_t with_bias) {
+    // the planning pass of the entry point on placeholder tensors (16-byte aligned, never dereferenced: nothing is launched)
+    if (!g || n_chunks < 1 || n_chunks > 4096 || g->n_seg < 1 || g->n_seg > 2) {
+        set_error("wgrad_det_workspace_bytes: bad geometry or chunk count");
+        return 0;
+    }
+    const void* fake = reinterpret_cast<const void*>(uintptr_t(1) << 20);
+    std::vector<const void*> ins((size_t)n_chunks * g->n_seg, fake), dzs((size_t)n_chunks, fake);
+    int32_t in_c[2] = {(g->seg_c[0] + 7) / 8 * 8, g->n_seg > 1 ? (g->seg_c[1] + 7) / 8 * 8 : 0};
+    const int cin_total = g->n_seg > 1 ? std::max(g->seg_off[0] + g->seg_c[0], g->seg_off[1] + g->seg_c[1]) : g->seg_off[0] + g->seg_c[0];
+    float* dw = reinterpret_cast<float*>(uintptr_t(1) << 20);
+    float* db = with_bias ? dw : nullptr;
+    const int dz_c = (g->cout + 7) / 8 * 8;
+    WgradDet det = {nullptr, 0, true};
+    const int rc = n_chunks == 1
+        ? wgrad_impl(g, ins.data(), in_c, fake, dz_c, batch, h, w, batch, cin_total, dw, db, nullptr, &det)
+        : (check_wgrad_multi(g, n_chunks, ins.data(), in_c, dzs.data(), dz_c, cin_total, dw) != VSRB_OK
+               ? VSRB_E_ARG
+               : wgrad_multi_run(g, n_chunks, ins.data(), in_c, dzs.data(), dz_c, batch, h, w, cin_total, dw, db, nullptr, &det));
+    return rc == VSRB_OK ? std::max<size_t>(det.need * 4, 16) : 0;
+}
+
+}  // extern "C"
+
+namespace vsrb {
+static int wgrad_impl(const vsrb_conv_geom* g, const void* const* in, const int32_t* in_c, const void* dz, int32_t dz_c,
+                      int32_t batch, int32_t h, int32_t w, int32_t imgs_per_group, int32_t cin_total, float* dw, float* db,
+                      void* stream, WgradDet* det) {
     VSRB_CHECK_ARG(g && in && in_c && dz && dw, "wgrad: null argument");
     VSRB_CHECK_ARG(g->n_seg == 1 || g->n_seg == 2, "wgrad: n_seg must be 1 or 2");
     VSRB_CHECK_ARG(!g->pixshuf && !g->transpose, "wgrad: pass the plain forward geometry (un-shuffle the gradient first)");
@@ -526,6 +708,8 @@ int vsrb_conv2d_wgrad(const vsrb_conv_geom* g, const void* const* in, const int3
         VSRB_CHECK_ARG(g->seg_off[s] + g->seg_c[s] <= cin_total, "wgrad: segment %d exceeds cin_total", s);
         P.in[s] = in[s]; P.in_c[s] = in_c[s]; P.seg_c[s] = g->seg_c[s]; P.seg_off[s] = g->seg_off[s];
         if (wgrad_path(g, s) != kWgradFfma) continue;
+        VSRB_CHECK_ARG(!det, "wgrad_det: no deterministic kernel for a %dx%d %s filter (its FFMA fallback adds with atomics)", g->kh,
+                       g->kw, g->dtype == VSRB_BF16 ? "bf16" : "fp32");
         VSRB_CHECK_ARG(g->kw == 1 || g->kw == 3 || g->kw == 7, "wgrad: no kernel for a %dx%d %s filter (the FFMA fallback takes "
                        "widths 1, 3 and 7)", g->kh, g->kw, g->dtype == VSRB_BF16 ? "bf16" : "fp32");
         for (int c0 = 0; c0 < g->seg_c[s]; c0 += 64) {
@@ -540,20 +724,20 @@ int vsrb_conv2d_wgrad(const vsrb_conv_geom* g, const void* const* in, const int3
     for (int s = 0; s < g->n_seg; ++s) {
         const WgradPath path = wgrad_path(g, s);
         if (path == kWgradTc) {
-            int rc = wgrad_tc_segment(g, s, &in[s], in_c[s], &dz, dz_c, 1, batch, h, w, cin_total, dw, &bias, st);
+            int rc = wgrad_tc_segment(g, s, &in[s], in_c[s], &dz, dz_c, 1, batch, h, w, cin_total, dw, &bias, st, det);
             if (rc != VSRB_OK) return rc;
         } else if (path == kWgradTaps) {
             for (int c0 = 0; c0 < g->seg_c[s]; c0 += 64)
                 for (int n0 = 0; n0 < g->cout; n0 += 64) {
                     const int ci_n = g->seg_c[s] - c0 < 64 ? g->seg_c[s] - c0 : 64, co_n = g->cout - n0 < 64 ? g->cout - n0 : 64;
                     int rc = launch_wgrad_taps(in[s], in_c[s], c0, ci_n, g->seg_off[s] + c0, dz, dz_c, n0, co_n, g->kw, batch, h, w, cin_total,
-                                               dw, st);
+                                               dw, st, det);
                     if (rc != VSRB_OK) return rc;
                 }
         }
     }
     if (bias) {
-        int rc = launch_bias_grad(dz, dz_c, (long long)batch * h * w, g->cout, g->dtype, bias, st);
+        int rc = launch_bias_grad(dz, dz_c, (long long)batch * h * w, g->cout, g->dtype, bias, st, det);
         if (rc != VSRB_OK) return rc;
     }
     if (P.n_ci_blk == 0) return VSRB_OK;
@@ -580,6 +764,9 @@ int vsrb_conv2d_wgrad(const vsrb_conv_geom* g, const void* const* in, const int3
     VSRB_LAUNCH_CHECK();
     return VSRB_OK;
 }
+}  // namespace vsrb
+
+extern "C" {
 
 int vsrb_flow_warp_bwd(const void* x, const float* flow, const void* dout, float* dx, float* dflow, int32_t n, int32_t h,
                        int32_t w, int32_t c, int32_t dtype, int32_t padding_mode, void* stream) {
@@ -598,6 +785,49 @@ int vsrb_flow_warp_bwd(const void* x, const float* flow, const void* dout, float
         rc = launch_warp_bwd<float>(reinterpret_cast<const float*>(x), reinterpret_cast<const float2*>(flow),
                                     reinterpret_cast<const float*>(dout), dx, reinterpret_cast<float2*>(dflow), n, h, w, c,
                                     padding_mode, s);
+    }
+    if (rc != VSRB_OK) return rc;
+    VSRB_LAUNCH_CHECK();
+    return VSRB_OK;
+}
+
+size_t vsrb_flow_warp_bwd_det_workspace_bytes(int32_t n, int32_t h, int32_t w, int32_t c) {
+    if (n < 1 || h < 1 || w < 1 || c < 1 || (long long)n * h * w * c >= (1LL << 40)) {
+        set_error("flow_warp_bwd_det_workspace_bytes: bad shape");
+        return 0;
+    }
+    return warp_bwd_det_bytes(n, h, w, c);
+}
+
+int vsrb_flow_warp_bwd_det(const void* x, const float* flow, const void* dout, float* dx, float* dflow, int32_t n, int32_t h,
+                           int32_t w, int32_t c, int32_t dtype, int32_t padding_mode, void* workspace, size_t workspace_bytes,
+                           void* stream) {
+    VSRB_CHECK_ARG(flow && dout && (dx || dflow) && n >= 1 && h >= 1 && w >= 1 && c >= 1, "flow_warp_bwd_det: bad arguments");
+    VSRB_CHECK_ARG(!dflow || x, "flow_warp_bwd_det: the flow gradient needs the forward input x");
+    VSRB_CHECK_ARG((long long)n * h * w * c < (1LL << 40) && (long long)h * w < (1LL << 30), "flow_warp_bwd_det: tensor too large");
+    VSRB_CHECK_ARG(dtype == VSRB_BF16 || dtype == VSRB_F32, "flow_warp_bwd_det: dtype must be bf16 or fp32 (got %d)", dtype);
+    VSRB_CHECK_ARG(padding_mode == VSRB_PAD_ZEROS || padding_mode == VSRB_PAD_BORDER,
+                   "flow_warp_bwd_det: padding_mode must be zeros (0) or border (1), got %d", padding_mode);
+    const int vec = dtype == VSRB_BF16 ? 8 : 4, tpp = c / vec;
+    VSRB_CHECK_ARG(c % vec == 0, "flow_warp_bwd_det: %s needs c %% %d == 0 (got %d)", dtype == VSRB_BF16 ? "bf16" : "fp32", vec, c);
+    // the flow gradient is single-writer when a pixel's lanes form a power-of-two group inside a warp (see launch_warp_bwd)
+    VSRB_CHECK_ARG(!dflow || (tpp <= 32 && (tpp & (tpp - 1)) == 0),
+                   "flow_warp_bwd_det: the flow gradient needs c / %d to be a power of two <= 32 (got c = %d)", vec, c);
+    VSRB_CHECK_ARG(!dx || (workspace && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0 &&
+                           workspace_bytes >= warp_bwd_det_bytes(n, h, w, c)),
+                   "flow_warp_bwd_det: dx needs a 16-byte aligned workspace of %zu bytes (got %zu)", warp_bwd_det_bytes(n, h, w, c),
+                   workspace_bytes);
+    cudaStream_t s = (cudaStream_t)stream;
+    const float2* fl = reinterpret_cast<const float2*>(flow);
+    int rc = VSRB_OK;
+    if (dtype == VSRB_BF16) {
+        const __nv_bfloat16 *xb = reinterpret_cast<const __nv_bfloat16*>(x), *db = reinterpret_cast<const __nv_bfloat16*>(dout);
+        if (dflow) rc = launch_warp_bwd<__nv_bfloat16>(xb, fl, db, nullptr, reinterpret_cast<float2*>(dflow), n, h, w, c, padding_mode, s);
+        if (rc == VSRB_OK && dx) rc = launch_warp_bwd_dx_det<__nv_bfloat16>(fl, db, dx, n, h, w, c, padding_mode, workspace, s);
+    } else {
+        const float *xf = reinterpret_cast<const float*>(x), *df = reinterpret_cast<const float*>(dout);
+        if (dflow) rc = launch_warp_bwd<float>(xf, fl, df, nullptr, reinterpret_cast<float2*>(dflow), n, h, w, c, padding_mode, s);
+        if (rc == VSRB_OK && dx) rc = launch_warp_bwd_dx_det<float>(fl, df, dx, n, h, w, c, padding_mode, workspace, s);
     }
     if (rc != VSRB_OK) return rc;
     VSRB_LAUNCH_CHECK();

@@ -18,7 +18,7 @@
 // accumulator columns exceed the 512 of TMEM (or K * Cu > 256), blockIdx.y splits the ty range; each pass loads only the
 // U rows it needs.  One box of S (R rows, 16 + K-1 pixels) and one of U (R + nj-1 rows, 16 pixels) per 16 x R pixel tile,
 // mbarrier ring.  Epilogue: per 16 U channels the accumulators go through shared memory in OIHW order, then leave as runs
-// of nj*K consecutive floats with coalesced atomics.
+// of nj*K consecutive floats with coalesced atomics (deterministic mode: stores to the CTA's slot, summed in slot order).
 #include "common.cuh"
 #include "tc_ptx.cuh"
 
@@ -42,6 +42,7 @@ struct WgTapsParams {
     int co_valid, ci_valid;     // channels of the block that exist
     int cin_total;
     float* dw;
+    float* slots;               // deterministic mode: CTA x stores its [co_valid][ci_valid][K*K] block at slots + x * that size
     int* dbg;
     int debug;                  // VSRB_WG_DEBUG: 1 / 2 / 4 = skip the final atomics / the MMAs / the loads
 };
@@ -186,7 +187,17 @@ __global__ void __launch_bounds__(kTpThreads, 1) wgrad_taps_kernel(const __grid_
         }
         tc_fence_before();
         __syncthreads();
-        if (my_tiles > 0 && !(P.debug & 1)) {
+        if (P.slots) {
+            const int co_rel = P.s_is_x ? n0 : 0, ci_rel = P.s_is_x ? 0 : n0;
+            const int co_lim = P.co_valid - co_rel, ci_lim = P.ci_valid - ci_rel;
+            float* slot = P.slots + (size_t)blockIdx.x * P.co_valid * P.ci_valid * KK;
+            for (int i = threadIdx.x; i < A * B * run; i += kTpThreads) {
+                const int ab = i / run, rr = i - ab * run;
+                const int a = ab / B, b = ab - a * B;
+                if (a < co_lim && b < ci_lim)
+                    slot[((size_t)(co_rel + a) * P.ci_valid + ci_rel + b) * KK + r_base + rr] = my_tiles > 0 ? stg[i] : 0.f;
+            }
+        } else if (my_tiles > 0 && !(P.debug & 1)) {
             const int co_base = P.co0 + (P.s_is_x ? n0 : 0), ci_base = P.ci0 + (P.s_is_x ? 0 : n0);
             const int co_lim = P.co_valid - (P.s_is_x ? n0 : 0), ci_lim = P.ci_valid - (P.s_is_x ? 0 : n0);
             const int total = A * B * run;
@@ -211,7 +222,7 @@ static int pow2_block(int c) { return c <= 16 ? 16 : (c <= 32 ? 32 : 64); }
 // One (input-channel block, output-channel block) pair: x channels [x_c0, x_c0 + ci_n), dz channels [z_c0, z_c0 + co_n),
 // ci_n, co_n <= 64.  `ci_off` = OIHW position of x channel x_c0.
 int launch_wgrad_taps(const void* x, int x_c, int x_c0, int ci_n, int ci_off, const void* dz, int dz_c, int z_c0, int co_n, int K,
-                      int batch, int h, int w, int cin_total, float* dw, cudaStream_t stream) {
+                      int batch, int h, int w, int cin_total, float* dw, cudaStream_t stream, WgradDet* det) {
     static bool ready[kMaxDevices] = {false};
     VSRB_CHECK_ARG(K >= 1 && K <= 7 && (K & 1) && ci_n >= 1 && ci_n <= 64 && co_n >= 1 && co_n <= 64, "wgrad_taps: bad block");
     constexpr int kSmemMax = 200 * 1024;
@@ -264,20 +275,28 @@ int launch_wgrad_taps(const void* x, int x_c, int x_c0, int ci_n, int ci_off, co
     P.cin_total = cin_total;
     P.dw = dw;
     P.dbg = debug_flag();
+    // every CTA ends with K*K*cs*cu/passes atomics: small problems use fewer CTAs (>= 8 tiles each)
+    int ctas = sms / passes;
+    if (ctas > P.total_tiles / 8) ctas = P.total_tiles / 8;
+    if (ctas < 1) ctas = 1;
     VSRB_CHECK_ARG(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dz)) & 15) == 0 && x_c % 8 == 0 && dz_c % 8 == 0,
                    "wgrad_taps: tensors must be 16-byte aligned with channel strides that are multiples of 8");
     rc = encode_nhwc(&P.smap, "wgrad_taps S", s_ptr, s_c, w, h, batch, P.cs, box_w, P.rows);
     if (rc != VSRB_OK) return rc;
     rc = encode_nhwc(&P.umap, "wgrad_taps U", u_ptr, u_c, w, h, batch, P.cu, kTpTW, u_rows);
     if (rc != VSRB_OK) return rc;
-    // every CTA ends with K*K*cs*cu/passes atomics: small problems use fewer CTAs (>= 8 tiles each)
-    int ctas = sms / passes;
-    if (ctas > P.total_tiles / 8) ctas = P.total_tiles / 8;
-    if (ctas < 1) ctas = 1;
+    // deterministic mode: the planning pass stops here, after every argument check of the launch
+    if (det) {
+        if (det_take(det, (size_t)ctas * co_n * ci_n * K * K)) return VSRB_OK;
+        P.slots = det->ws;
+    }
     P.debug = env_int("VSRB_WG_DEBUG");
     const int smem = 1024 + 1024 + P.stages * P.stage_bytes;
     wgrad_taps_kernel<<<dim3(ctas, passes), kTpThreads, smem, stream>>>(P);
     VSRB_LAUNCH_CHECK();
+    if (det)
+        return launch_slot_reduce(P.slots, ctas, co_n, ci_n * K * K, (long long)cin_total * K * K,
+                                  dw + ((size_t)z_c0 * cin_total + ci_off) * K * K, stream);
     return VSRB_OK;
 }
 

@@ -17,7 +17,8 @@
 //   B (N side) = the output gradient dz (N = 64 output channels).
 //   D          = five accumulators of 128 x 64 fp32 in TMEM (9 taps = 4 pairs + 1 single), kept for the whole
 //                persistent CTA; K advances 16 pixels (2048 bytes) per MMA.
-// Every pixel tile is read once; at the end each CTA adds its partial dW into the fp32 OIHW gradient with atomics.
+// Every pixel tile is read once; at the end each CTA adds its partial dW into the fp32 OIHW gradient with atomics, or, for
+// deterministic gradients, stores it to its own slot of a workspace that slot_reduce_kernel then sums in slot order.
 // Replaces the wgrad half of autograd's ConvolutionBackward0 for the hot 64->64 / 64->256 3x3 layers.
 #include "common.cuh"
 #include "tc_ptx.cuh"
@@ -47,6 +48,8 @@ struct WgTcParams {
     float* dw;
     float* db;                  // bias gradient (sum of dz over the pixels), or null: the epilogue warps, idle while the tiles stream
                                 // through, add up the dz tiles in shared memory - no second pass over dz
+    float* slots;               // deterministic mode: CTA x stores its [cout][64][9] block at slots + x * cout * 576 (else null)
+    float* bslots;              // ... and its bias sums at bslots + x * cout
     int* dbg;
     int debug;                  // VSRB_WG_DEBUG: 1 / 2 / 4 = skip the final atomics / the MMAs / the loads (timing decomposition only)
 };
@@ -201,7 +204,12 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
     __syncthreads();
     // ---- epilogue part 2 (all warps): the block leaves with coalesced atomics - consecutive lanes add consecutive floats
     // of dw[co][ci_off .. ci_off+63][0..8], 8x fewer L2 sector operations than one scattered atomic per (ci, tap) ----
-    if (my_tiles > 0 && !(P.debug & 1)) {
+    if (P.slots) {
+        const float* stg = reinterpret_cast<const float*>(base_ptr + 1024);
+        float* slot = P.slots + (size_t)blockIdx.x * P.cout * 576;
+        for (int co = 0; co < 64 && n0 + co < P.cout; ++co)
+            for (int i = threadIdx.x; i < 576; i += kWgThreads) slot[(size_t)(n0 + co) * 576 + i] = my_tiles > 0 ? stg[co * 576 + i] : 0.f;
+    } else if (my_tiles > 0 && !(P.debug & 1)) {
         const float* stg = reinterpret_cast<const float*>(base_ptr + 1024);
         for (int co = 0; co < 64 && n0 + co < P.cout; ++co) {
             float* dst = P.dw + ((size_t)(n0 + co) * P.cin_total + P.ci_off) * 9;
@@ -215,7 +223,10 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
             bsum[(warp - 4) * 64 + 2 * lane + 1] = bs1;
         }
         __syncthreads();
-        if (threadIdx.x < 64 && my_tiles > 0 && n0 + (int)threadIdx.x < P.cout && !(P.debug & 1))
+        if (P.bslots && threadIdx.x < 64 && n0 + (int)threadIdx.x < P.cout)
+            P.bslots[(size_t)blockIdx.x * P.cout + n0 + threadIdx.x] =
+                my_tiles > 0 ? bsum[threadIdx.x] + bsum[64 + threadIdx.x] + bsum[128 + threadIdx.x] + bsum[192 + threadIdx.x] : 0.f;
+        else if (threadIdx.x < 64 && my_tiles > 0 && n0 + (int)threadIdx.x < P.cout && !(P.debug & 1))
             atomicAdd(P.db + n0 + threadIdx.x, bsum[threadIdx.x] + bsum[64 + threadIdx.x] + bsum[128 + threadIdx.x] + bsum[192 + threadIdx.x]);
     }
     tc_fence_before();
@@ -239,10 +250,11 @@ __device__ __forceinline__ void bias_ld8(const float* p, float (&v)[8]) {
 
 // db[c] += sum over pixels of dz[p][c].  HBM-bound (reads dz once): every thread owns 8 consecutive channels (one 16-byte
 // load per pixel for bf16) and a strided set of pixels; the pixel lanes of a CTA are reduced in shared memory, then one
-// atomic per channel and CTA.  blockDim = 256 = G channel groups (G = 8 for 64 channels) x 256/G pixel lanes.
+// atomic per channel and CTA (or, deterministic, a store to the CTA's slot: slots + blockIdx.x * cout).
+// blockDim = 256 = G channel groups (G = 8 for 64 channels) x 256/G pixel lanes.
 template <typename T>
 __global__ void __launch_bounds__(256) bias_grad_kernel(const T* __restrict__ dz, int dz_c, long long pixels, int cout, int G,
-                                                        float* __restrict__ db) {
+                                                        float* __restrict__ db, float* __restrict__ slots) {
     __shared__ float red[256][9];                                  // [thread][8 channels] (+1: no bank conflicts)
     const int grp = threadIdx.x % G, lane = threadIdx.x / G, lanes = 256 / G;
     const int c0 = (blockIdx.y * G + grp) * 8;
@@ -265,29 +277,59 @@ __global__ void __launch_bounds__(256) bias_grad_kernel(const T* __restrict__ dz
         float t = 0.f;
         for (int l = 0; l < lanes; ++l) t += red[l * G + g2][ch];
         const int c = (blockIdx.y * G + g2) * 8 + ch;
-        if (c < cout) atomicAdd(db + c, t);
+        if (c < cout) {
+            if (slots) slots[(size_t)blockIdx.x * cout + c] = t;
+            else atomicAdd(db + c, t);
+        }
     }
 }
 
-int launch_bias_grad(const void* dz, int dz_c, long long pixels, int cout, int dtype, float* db, cudaStream_t s) {
+// dst[r * dst_stride + e] += sum over s = 0, 1, ..., slots - 1 of parts[s][r][e]  (parts: `slots` blocks of rows x row_len).
+// One writer per element and a fixed order of the additions: the deterministic end of every weight / bias gradient.
+__global__ void __launch_bounds__(256) slot_reduce_kernel(const float* __restrict__ parts, int slots, int rows, int row_len,
+                                                          long long dst_stride, float* __restrict__ dst) {
+    const long long n = (long long)rows * row_len;
+    for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n; i += (long long)gridDim.x * 256) {
+        float acc = 0.f;
+        for (int s = 0; s < slots; ++s) acc += __ldg(parts + (long long)s * n + i);
+        const long long r = i / row_len;
+        dst[r * dst_stride + (i - r * row_len)] += acc;
+    }
+}
+
+int launch_slot_reduce(const float* parts, int slots, int rows, int row_len, long long dst_stride, float* dst, cudaStream_t s) {
+    const long long n = (long long)rows * row_len;
+    long long b = (n + 255) / 256;
+    if (b > 148 * 8) b = 148 * 8;
+    slot_reduce_kernel<<<(int)b, 256, 0, s>>>(parts, slots, rows, row_len, dst_stride, dst);
+    VSRB_LAUNCH_CHECK();
+    return VSRB_OK;
+}
+
+int launch_bias_grad(const void* dz, int dz_c, long long pixels, int cout, int dtype, float* db, cudaStream_t s, WgradDet* det) {
     const int groups = ceil_div(cout, 8);
     int G = 1;
     while (G < groups && G < 32) G *= 2;                            // channel groups per CTA: power of two <= 32
     long long want = (pixels + 256 / G * 8 - 1) / (256 / G * 8);   // >= 8 pixels per thread
     int gx = (int)(want < 1 ? 1 : (want > 148 * 4 ? 148 * 4 : want));
     dim3 grid(gx, ceil_div(groups, G));
+    float* slots = nullptr;
+    if (det) {
+        if (det_take(det, (size_t)gx * cout)) return VSRB_OK;
+        slots = det->ws;
+    }
     if (dtype == VSRB_BF16)
-        bias_grad_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(reinterpret_cast<const __nv_bfloat16*>(dz), dz_c, pixels, cout, G, db);
+        bias_grad_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(reinterpret_cast<const __nv_bfloat16*>(dz), dz_c, pixels, cout, G, db, slots);
     else
-        bias_grad_kernel<float><<<grid, 256, 0, s>>>(reinterpret_cast<const float*>(dz), dz_c, pixels, cout, G, db);
+        bias_grad_kernel<float><<<grid, 256, 0, s>>>(reinterpret_cast<const float*>(dz), dz_c, pixels, cout, G, db, slots);
     VSRB_LAUNCH_CHECK();
-    return VSRB_OK;
+    return slots ? launch_slot_reduce(slots, gx, 1, cout, 0, db, s) : VSRB_OK;
 }
 
 // one 64-input-channel block (x channels [c0, c0+64), OIHW offset ci_off) against all 64-wide output blocks, summed over
 // `n_chunks` (x, dz) pairs of `batch` images each
 int launch_wgrad_tc_multi(const void* const* xs, int x_c, int c0, int ci_off, const void* const* dzs, int dz_c, int n_chunks,
-                          int batch, int h, int w, int cout, int cin_total, float* dw, cudaStream_t stream, float* db) {
+                          int batch, int h, int w, int cout, int cin_total, float* dw, cudaStream_t stream, float* db, WgradDet* det) {
     static bool ready[kMaxDevices] = {false};
     VSRB_CHECK_ARG(n_chunks >= 1 && n_chunks <= kWgMaxChunks, "wgrad: 1..%d chunks per launch", kWgMaxChunks);
     int dev = 0, sms = 0;
@@ -305,6 +347,11 @@ int launch_wgrad_tc_multi(const void* const* xs, int x_c, int c0, int ci_off, co
     P.total_tiles = P.tiles_per_chunk * n_chunks;
     P.c0 = c0; P.cout = cout; P.cin_total = cin_total; P.ci_off = ci_off; P.dw = dw; P.db = db;
     P.dbg = debug_flag();
+    const int n_blocks = ceil_div(cout, 64);
+    // every CTA ends with 9*64*64 atomics, so small problems use fewer CTAs (>= 32 pixel tiles each)
+    int ctas = sms / n_blocks;
+    if (ctas > P.total_tiles / 32) ctas = P.total_tiles / 32;
+    if (ctas < 1) ctas = 1;
     for (int k = 0; k < n_chunks; ++k) {
         VSRB_CHECK_ARG(xs[k] && dzs[k] && ((reinterpret_cast<uintptr_t>(xs[k]) | reinterpret_cast<uintptr_t>(dzs[k])) & 15) == 0,
                        "wgrad: chunk %d: null or unaligned tensor", k);
@@ -313,17 +360,23 @@ int launch_wgrad_tc_multi(const void* const* xs, int x_c, int c0, int ci_off, co
         rc = encode_nhwc(&P.zmap[k], "wgrad dz", dzs[k], dz_c, w, h, batch, 64, kWgTW, kWgRows);
         if (rc != VSRB_OK) return rc;
     }
-    const int n_blocks = ceil_div(cout, 64);
-    // every CTA ends with 9*64*64 atomics, so small problems use fewer CTAs (>= 32 pixel tiles each)
-    int ctas = sms / n_blocks;
-    if (ctas > P.total_tiles / 32) ctas = P.total_tiles / 32;
-    if (ctas < 1) ctas = 1;
+    // deterministic mode: the planning pass stops here, after every argument check of the launch
+    if (det) {
+        if (det_take(det, (size_t)ctas * cout * (576 + (db ? 1 : 0)))) return VSRB_OK;
+        P.slots = det->ws;
+        P.bslots = db ? det->ws + (size_t)ctas * cout * 576 : nullptr;
+    }
     P.debug = env_int("VSRB_WG_DEBUG");
     // blockIdx.y = 64-wide output block: all blocks of a wide layer (64 -> 256) share ONE launch.  (A launch per block on
     // sms / n_blocks CTAs each ran them one after the other - same stream - on a quarter of the GPU: 560 -> 230 us.)
     P.n0 = 0;
     wgrad_tc_kernel<<<dim3(ctas, n_blocks), kWgThreads, kWgSmem, stream>>>(P);
     VSRB_LAUNCH_CHECK();
+    if (det) {
+        rc = launch_slot_reduce(P.slots, ctas, cout, 576, (long long)cin_total * 9, dw + (size_t)ci_off * 9, stream);
+        if (rc == VSRB_OK && db) rc = launch_slot_reduce(P.bslots, ctas, 1, cout, 0, db, stream);
+        return rc;
+    }
     return VSRB_OK;
 }
 

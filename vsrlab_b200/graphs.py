@@ -167,7 +167,8 @@ def training_forward(model, lr: torch.Tensor):
         return AG.realbasicvsr(model, lr)
     params = list(model.parameters())
     key = (tuple(lr.shape), str(lr.device), model.training, torch.is_autocast_enabled("cuda"),
-           tuple(p.requires_grad for p in params), tuple(p.data_ptr() for p in params))
+           tuple(p.requires_grad for p in params), tuple(p.data_ptr() for p in params),
+           torch.are_deterministic_algorithms_enabled())      # the deterministic kernels are a different graph
     table = _train_entries.get(id(model))
     if table is None or table["model"]() is not model:
         table = {"model": weakref.ref(model), "by_key": {}}
@@ -217,19 +218,28 @@ class GraphedTrainStep:
     def _build(self, example_inputs, warmup):
         self.static_in = [t.clone() for t in example_inputs]
         self.stream = torch.cuda.Stream(device=self.static_in[0].device)
+        self.warmup = warmup
+        self._graphs = {}                                 # torch.are_deterministic_algorithms_enabled() -> (graph, loss)
+        self._capture(update=True)
+
+    def _capture(self, update: bool):
+        """Warm up and capture the step for the current value of the deterministic flag.  `update`: the warm-up steps are
+        real training steps (construction); otherwise they run forward and backward only and discard the gradients, so a
+        capture for the other flag value in the middle of a run changes neither the parameters nor the optimizer state."""
         self.stream.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(self.stream):              # warm-up on the capture stream (also where the grad accumulators live)
-            for _ in range(warmup):
+            for _ in range(self.warmup):
                 self.opt.zero_grad(set_to_none=True)
-                self._body()
+                self._body(update)
         torch.cuda.current_stream().wait_stream(self.stream)
         torch.cuda.synchronize()
         self.opt.zero_grad(set_to_none=True)
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph, stream=self.stream):
             self.static_loss = self._body()
+        self._graphs[torch.are_deterministic_algorithms_enabled()] = (self.graph, self.static_loss)
 
-    def _body(self) -> torch.Tensor:
+    def _body(self, update: bool = True) -> torch.Tensor:
         x = self.static_in[0].clone()                     # the model refines its input in place (reference contract)
         if self.dtype is not None:
             with torch.autocast("cuda", dtype=self.dtype):
@@ -238,6 +248,8 @@ class GraphedTrainStep:
             out = self.model(x)
         loss = self.loss_fn(out, *self.static_in[1:])
         loss.backward()
+        if not update:
+            return loss.detach()
         if self.clip is not None:
             torch.nn.utils.clip_grad_norm_(self.model.parameters(), self.clip)
         self.opt.step()
@@ -246,5 +258,14 @@ class GraphedTrainStep:
     def __call__(self, *inputs: torch.Tensor) -> torch.Tensor:
         for dst, src in zip(self.static_in, inputs):
             dst.copy_(src, non_blocking=True)
+        det = torch.are_deterministic_algorithms_enabled()
+        if det not in self._graphs:                       # the flag changed since the capture: capture the other kernels too
+            global _auto_off
+            _auto_off += 1
+            try:
+                self._capture(update=False)
+            finally:
+                _auto_off -= 1
+        self.graph, self.static_loss = self._graphs[det]
         self.graph.replay()
         return self.static_loss

@@ -21,7 +21,7 @@ from typing import Optional
 import torch
 
 from . import _lib as L
-from .ops import _p, _stream, require_cuda
+from .ops import _p, loss_sums, require_cuda
 
 
 def _f32c(t: torch.Tensor) -> torch.Tensor:
@@ -36,7 +36,7 @@ class _CharbonnierFn(torch.autograd.Function):
         if xc.shape != yc.shape:
             raise L.VsrbError(f"CharbonnierLoss: shapes differ {tuple(xc.shape)} vs {tuple(yc.shape)}")
         acc = torch.zeros(1, dtype=torch.float64, device=x.device)
-        L.check(L.load().vsrb_charbonnier(_p(xc), _p(yc), xc.numel(), eps, _p(acc), None, None, 1.0, _stream()), "vsrb_charbonnier")
+        loss_sums("charbonnier", (xc.numel(),), _p(xc), _p(yc), xc.numel(), eps, _p(acc), None, None, 1.0)
         ctx.save_for_backward(xc, yc)
         ctx.eps, ctx.x_dtype, ctx.y_dtype = eps, x.dtype, y.dtype
         return (acc / xc.numel()).to(torch.float32).squeeze(0)
@@ -47,8 +47,7 @@ class _CharbonnierFn(torch.autograd.Function):
         gx = torch.empty_like(xc)
         acc = torch.zeros(1, dtype=torch.float64, device=xc.device)
         gs = g.detach().to(torch.float32).contiguous()
-        L.check(L.load().vsrb_charbonnier(_p(xc), _p(yc), xc.numel(), ctx.eps, _p(acc), _p(gx), _p(gs), 1.0 / xc.numel(), _stream()),
-                "vsrb_charbonnier")
+        loss_sums("charbonnier", (xc.numel(),), _p(xc), _p(yc), xc.numel(), ctx.eps, _p(acc), _p(gx), _p(gs), 1.0 / xc.numel())
         gy = -gx if ctx.needs_input_grad[1] else None
         return (gx.to(ctx.x_dtype) if ctx.needs_input_grad[0] else None), (gy.to(ctx.y_dtype) if gy is not None else None), None
 
@@ -66,8 +65,7 @@ class _CharbonnierResizedFn(torch.autograd.Function):
         if hc.numel() // (H * W) != planes:
             raise L.VsrbError("charbonnier_resized: lq and hr must have the same leading dimensions")
         acc = torch.zeros(1, dtype=torch.float64, device=lq.device)
-        L.check(L.load().vsrb_charbonnier_resized(_p(lc), _p(hc), planes, h, w, H, W, eps, _p(acc), None, None, 1.0, _stream()),
-                "vsrb_charbonnier_resized")
+        loss_sums("charbonnier_resized", (planes, h, w), _p(lc), _p(hc), planes, h, w, H, W, eps, _p(acc), None, None, 1.0)
         ctx.save_for_backward(lc, hc)
         ctx.eps, ctx.dtype = eps, lq.dtype
         return (acc / lc.numel()).to(torch.float32).squeeze(0)
@@ -81,8 +79,8 @@ class _CharbonnierResizedFn(torch.autograd.Function):
         gl = torch.empty_like(lc)
         acc = torch.zeros(1, dtype=torch.float64, device=lc.device)
         gs = g.detach().to(torch.float32).contiguous()
-        L.check(L.load().vsrb_charbonnier_resized(_p(lc), _p(hc), planes, h, w, H, W, ctx.eps, _p(acc), _p(gl), _p(gs), 1.0 / lc.numel(),
-                                                  _stream()), "vsrb_charbonnier_resized")
+        loss_sums("charbonnier_resized", (planes, h, w), _p(lc), _p(hc), planes, h, w, H, W, ctx.eps, _p(acc), _p(gl), _p(gs),
+                  1.0 / lc.numel())
         return gl.to(ctx.dtype), None, None
 
 
@@ -205,7 +203,7 @@ class PSNR(torch.nn.Module):
         n = xc.shape[0]
         per = xc.numel() // n
         sums = torch.zeros(n, dtype=torch.float64, device=x.device)
-        L.check(L.load().vsrb_psnr_sums(_p(xc), _p(yc), n, per, _p(sums), _stream()), "vsrb_psnr_sums")
+        loss_sums("psnr_sums", (n, per), _p(xc), _p(yc), n, per, _p(sums))
         v = (10.0 * torch.log10(1.0 / (sums / per + self.epsilon))).to(torch.float32)
         return v.mean() if self.reduction == "mean" else (v.sum() if self.reduction == "sum" else v)
 
@@ -225,7 +223,7 @@ class SSIM(torch.nn.Module):
         xc, yc = _f32c(x), _f32c(y)
         n, c, h, w = xc.shape
         sums = torch.zeros(n, dtype=torch.float64, device=x.device)
-        L.check(L.load().vsrb_ssim_sums(_p(xc), _p(yc), n, c, h, w, 1, _p(sums), _stream()), "vsrb_ssim_sums")
+        loss_sums("ssim_sums", (n, c, h, w), _p(xc), _p(yc), n, c, h, w, 1, _p(sums))
         v = (sums / (c * (h - 10) * (w - 10))).to(torch.float32)
         return v.mean() if self.reduction == "mean" else (v.sum() if self.reduction == "sum" else v)
 

@@ -5,6 +5,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import warnings
 from typing import Optional, Sequence, Tuple
 
 import torch
@@ -63,6 +64,33 @@ def _p(t) -> Optional[C.c_void_p]:
     if isinstance(t, int):
         return C.c_void_p(t)
     return C.c_void_p(t.data_ptr())
+
+
+# torch.use_deterministic_algorithms(True), read at call time: the weight / bias gradients, the warp backward and the loss
+# and metric sums then run their *_det entry points (fixed summation order), and ops without one alert as torch's do.
+def deterministic() -> bool:
+    return torch.are_deterministic_algorithms_enabled()
+
+
+_alerted = set()
+
+
+def nondeterministic_alert(op: str) -> None:
+    """torch's behaviour for an op without a deterministic implementation: raise, or warn once under warn_only=True."""
+    msg = (f"{op} does not have a deterministic implementation, but you set 'torch.use_deterministic_algorithms(True)'. "
+           "You can turn off determinism just for this operation, or you can use the 'warn_only=True' option, if that's "
+           "acceptable for your application.")
+    if not torch.is_deterministic_algorithms_warn_only_enabled():
+        raise RuntimeError(msg)
+    if op not in _alerted:
+        _alerted.add(op)
+        warnings.warn(msg, UserWarning, stacklevel=3)
+
+
+def _workspace(nbytes: int, what: str, device) -> torch.Tensor:
+    if nbytes == 0:
+        raise L.VsrbError(f"{what}: {L.load().vsrb_last_error().decode()}")
+    return torch.empty(nbytes, dtype=torch.uint8, device=device)
 
 
 def require_cuda(t: torch.Tensor, what: str) -> None:
@@ -307,6 +335,10 @@ class PackedConvT(PackedConv):
 def conv2d_wgrad(geom: "L.ConvGeom", ins: Sequence[torch.Tensor], in_c: Sequence[int], dz: torch.Tensor, dz_c: int, batch: int,
                  h: int, w: int, cin_total: int, dw: torch.Tensor, db: Optional[torch.Tensor]) -> None:
     """dw (fp32 OIHW) += sum_pixels dz (x) x ;  db += sum_pixels dz.  `geom` = forward geometry without pixshuf."""
+    if deterministic():
+        if geom.dtype == BF16 and geom.kh == geom.kw:
+            return conv2d_wgrad_det(geom, ins, in_c, dz, dz_c, batch, h, w, cin_total, dw, db)
+        nondeterministic_alert(f"vsrlab_b200 conv weight gradient ({geom.kh}x{geom.kw} filter, FFMA kernel)")
     n = len(ins)
     ptrs = (C.c_void_p * 2)(*[t.data_ptr() for t in ins], *([None] * (2 - n)))
     cs = (C.c_int32 * 2)(*in_c, *([0] * (2 - n)))
@@ -321,6 +353,8 @@ def conv2d_wgrad_multi(geom: "L.ConvGeom", chunks: Sequence[Tuple[Sequence[torch
                        dz_c: int, batch: int, h: int, w: int, cin_total: int, dw: torch.Tensor, db: Optional[torch.Tensor]) -> None:
     """dw / db += the gradient summed over `chunks` = [(inputs of one use, its dz), ...] of one shape, without concatenating
     them (tensor-core path: bf16 3x3 convs whose input segments have a multiple of 64 channels)."""
+    if deterministic():
+        return conv2d_wgrad_multi_det(geom, chunks, in_c, dz_c, batch, h, w, cin_total, dw, db)
     n, ns = len(chunks), geom.n_seg
     ptrs = (C.c_void_p * (n * ns))(*[t.data_ptr() for ins, _ in chunks for t in ins])
     dzs = (C.c_void_p * n)(*[dz.data_ptr() for _, dz in chunks])
@@ -333,6 +367,15 @@ def conv2d_wgrad_multi(geom: "L.ConvGeom", chunks: Sequence[Tuple[Sequence[torch
 
 
 def flow_warp_bwd(x, flow, dout, dx, dflow, n: int, h: int, w: int, c: int, dtype: int, padding: int = PAD_ZEROS) -> None:
+    """dx = the gradient wrt x, dflow = the gradient wrt the flow (either may be None).  `dx` must be a ZEROED fp32 buffer:
+    the default kernel adds into it with atomics, the deterministic one (torch.use_deterministic_algorithms) overwrites
+    it, so a buffer that already holds a gradient would be accumulated in one mode and lost in the other.  To sum several
+    warp gradients, add the results."""
+    if deterministic():
+        tpp = c // (8 if dtype == BF16 else 4)
+        if dflow is None or (tpp <= 32 and tpp & (tpp - 1) == 0):
+            return flow_warp_bwd_det(x, flow, dout, dx, dflow, n, h, w, c, dtype, padding)
+        nondeterministic_alert(f"vsrlab_b200 flow_warp backward ({c} channels)")
     with _Timed("flow_warp_bwd", float(n) * h * w * (3 * c * ESIZE[dtype] + 4 * c * 4)):
         L.check(L.load().vsrb_flow_warp_bwd(_p(x), _p(flow), _p(dout), _p(dx), _p(dflow), n, h, w, c, dtype, padding, _stream()),
                 "vsrb_flow_warp_bwd")
@@ -340,6 +383,65 @@ def flow_warp_bwd(x, flow, dout, dx, dflow, n: int, h: int, w: int, c: int, dtyp
 
 def flow_warp_ex_bwd(x, flow, dout, dx, dflow, n: int, h: int, w: int, c: int, dtype: int, interp: int = INTERP_BILINEAR,
                      padding: int = PAD_ZEROS, align_corners: bool = True) -> None:
+    """flow_warp_bwd for every grid_sample mode; the same contract for `dx` (a zeroed buffer that receives the gradient)."""
+    if deterministic():
+        if interp == INTERP_BILINEAR and align_corners and padding in (PAD_ZEROS, PAD_BORDER):
+            return flow_warp_bwd(x, flow, dout, dx, dflow, n, h, w, c, dtype, padding)
+        nondeterministic_alert("vsrlab_b200 flow_warp backward (nearest / bicubic, reflection or align_corners=False; as "
+                               "grid_sampler_2d_backward_cuda)")
     with _Timed("flow_warp_ex_bwd", float(n) * h * w * (3 * c * ESIZE[dtype] + 4 * c * 4)):
         L.check(L.load().vsrb_flow_warp_ex_bwd(_p(x), _p(flow), _p(dout), _p(dx), _p(dflow), n, h, w, c, dtype, interp, padding,
                                                int(bool(align_corners)), _stream()), "vsrb_flow_warp_ex_bwd")
+
+
+# ---- deterministic variants (torch.use_deterministic_algorithms; see deterministic()) ----
+def conv2d_wgrad_det(geom: "L.ConvGeom", ins: Sequence[torch.Tensor], in_c: Sequence[int], dz: torch.Tensor, dz_c: int, batch: int,
+                     h: int, w: int, cin_total: int, dw: torch.Tensor, db: Optional[torch.Tensor]) -> None:
+    """conv2d_wgrad with a fixed summation order (bf16 square filters)."""
+    lib = L.load()
+    n = len(ins)
+    ptrs = (C.c_void_p * 2)(*[t.data_ptr() for t in ins], *([None] * (2 - n)))
+    cs = (C.c_int32 * 2)(*in_c, *([0] * (2 - n)))
+    ws = _workspace(lib.vsrb_conv2d_wgrad_det_workspace_bytes(C.byref(geom), 1, batch, h, w, int(db is not None)), "wgrad_det", dz.device)
+    with _Timed("conv_wgrad_det", 2.0 * batch * h * w * geom.cout * sum(geom.seg_c[i] for i in range(geom.n_seg)) * geom.kh * geom.kw):
+        L.check(lib.vsrb_conv2d_wgrad_det(C.byref(geom), ptrs, cs, _p(dz), dz_c, batch, h, w, batch // geom.groups, cin_total, _p(dw),
+                                          _p(db), _p(ws), ws.numel(), _stream()), "vsrb_conv2d_wgrad_det")
+
+
+def conv2d_wgrad_multi_det(geom: "L.ConvGeom", chunks: Sequence[Tuple[Sequence[torch.Tensor], torch.Tensor]], in_c: Sequence[int],
+                           dz_c: int, batch: int, h: int, w: int, cin_total: int, dw: torch.Tensor, db: Optional[torch.Tensor]) -> None:
+    """conv2d_wgrad_multi with a fixed summation order."""
+    lib = L.load()
+    n, ns = len(chunks), geom.n_seg
+    ptrs = (C.c_void_p * (n * ns))(*[t.data_ptr() for ins, _ in chunks for t in ins])
+    dzs = (C.c_void_p * n)(*[dz.data_ptr() for _, dz in chunks])
+    cs = (C.c_int32 * ns)(*in_c)
+    ws = _workspace(lib.vsrb_conv2d_wgrad_det_workspace_bytes(C.byref(geom), n, batch, h, w, int(db is not None)), "wgrad_multi_det",
+                    dw.device)
+    with _Timed("conv_wgrad_det", 2.0 * n * batch * h * w * geom.cout * sum(geom.seg_c[i] for i in range(ns)) * geom.kh * geom.kw):
+        L.check(lib.vsrb_conv2d_wgrad_multi_det(C.byref(geom), n, ptrs, cs, dzs, dz_c, batch, h, w, cin_total, _p(dw), _p(db), _p(ws),
+                                                ws.numel(), _stream()), "vsrb_conv2d_wgrad_multi_det")
+
+
+def flow_warp_bwd_det(x, flow, dout, dx, dflow, n: int, h: int, w: int, c: int, dtype: int, padding: int = PAD_ZEROS) -> None:
+    """flow_warp_bwd with dx OVERWRITTEN (fixed-point sums) and the default kernel's dflow."""
+    lib = L.load()
+    ws = _workspace(lib.vsrb_flow_warp_bwd_det_workspace_bytes(n, h, w, c), "flow_warp_bwd_det", dout.device) if dx is not None else None
+    with _Timed("flow_warp_bwd_det", float(n) * h * w * (3 * c * ESIZE[dtype] + 4 * c * 4)):
+        L.check(lib.vsrb_flow_warp_bwd_det(_p(x), _p(flow), _p(dout), _p(dx), _p(dflow), n, h, w, c, dtype, padding, _p(ws),
+                                           0 if ws is None else ws.numel(), _stream()), "vsrb_flow_warp_bwd_det")
+
+
+def loss_sums(name: str, query: Sequence, *args) -> None:
+    """vsrb_<name>(*args) of loss.cu (charbonnier, charbonnier_resized, psnr_sums, ssim_sums); `query` = the shape arguments of its
+    workspace query.  Deterministic mode: loss_sums_det."""
+    if deterministic():
+        return loss_sums_det(name, query, *args)
+    L.check(getattr(L.load(), "vsrb_" + name)(*args, _stream()), "vsrb_" + name)
+
+
+def loss_sums_det(name: str, query: Sequence, *args) -> None:
+    lib = L.load()
+    dev = torch.device("cuda", torch.cuda.current_device())
+    ws = _workspace(getattr(lib, f"vsrb_{name}_det_workspace_bytes")(*query), name + "_det", dev)
+    L.check(getattr(lib, f"vsrb_{name}_det")(*args, _p(ws), ws.numel(), _stream()), f"vsrb_{name}_det")
